@@ -1,6 +1,6 @@
 """Benchmarks of the retrieval scoring hot path on B200 (BASELINE.json configs 2-5).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config c5|c4|c3|c2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config c5|c4|c3|c2] [--dump-outputs DIR]
 
 Default (the driver's call): config C5, the headline -- text->video queries/sec at top-100 over a 10M-video
 corpus.  A step is one pass of the hot path over one query batch: 8,192 raw text-query embeddings (two
@@ -72,7 +72,7 @@ METRICS = {
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps of the measured config")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--config", default="c5", choices=sorted(WORKLOADS))
@@ -83,7 +83,15 @@ def parse():
     ap.add_argument("--no-extra-configs", action="store_true", help="C5 only: do not also measure C2-C4")
     ap.add_argument("--no-head-stream", action="store_true",
                     help="C5: keep K1 / sampling / threshold of the next batch on the main stream (A/B switch)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float64), "
+                         "so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200: the reference arm times a sample, not the whole workload")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -408,6 +416,33 @@ def result_digest(scores, idx):
     return h.hexdigest()
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def host_lists(result):
+    """The (scores, idx) lists of a search as the host arrays its caller receives."""
+    s, i = result
+    return {"scores": s.cpu().numpy(), "indices": i.cpu().numpy()}
+
+
+def dump_outputs(path, arrays):
+    """Write ``arrays`` (name -> array, one row per query) as ``path/<name>.npy`` in float64 (row ids < 2**53 are
+    exact).  Above DUMP_LIMIT bytes in all, the same fixed, seeded sample of rows is kept in every array and the
+    sampled row numbers are written as ``rows.npy``."""
+    import numpy as np
+    out = {name: np.asarray(a, dtype=np.float64) for name, a in arrays.items()}
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT:
+        n = len(next(iter(out.values())))
+        keep = (DUMP_LIMIT - 4096 * (len(out) + 1)) // (total // n + 8)
+        rows = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        out = {name: a[rows] for name, a in out.items()}
+        out["rows"] = rows.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def fp64_topk_regenerated(torch, chunks, q_sub, dims, weights, k, eps_norm=False, exclude=None):
     """Exact top-k of ``sum_s w_s cos_s`` in plain torch fp64 (checker only) over corpus rows handed in chunk by chunk
     by ``chunks`` -- a generator of (first global row, fp32 rows [n, sum(dims)]) REGENERATED from the seed, never the
@@ -465,6 +500,7 @@ class Ctx:
             dist.init_process_group("nccl", device_id=self.device)
         _native.require_device()
         self.peak_tf, self.peak_gbs, self.peak_src = peaks()
+        self.outputs = None            # host arrays the last timed step of the latest config returned (--dump-outputs)
 
     def barrier(self):
         if self.world > 1:
@@ -524,7 +560,8 @@ class Ctx:
 def pipelined(search_fn):
     """(step, finish): ``step`` enqueues one deferred search and resolves the PREVIOUS one -- the certificate of a
     step (one int32: how many rows need a re-run) comes back asynchronously, so the host enqueues step i+1 while the
-    GPU still scores step i; ``finish`` resolves what is in flight (called INSIDE the timed region)."""
+    GPU still scores step i; ``finish`` resolves what is in flight (called INSIDE the timed region) and returns the
+    (scores, idx) of the last step."""
     in_flight = []
 
     def step():
@@ -533,8 +570,10 @@ def pipelined(search_fn):
             in_flight.pop(0).result()
 
     def finish():
+        last = None
         while in_flight:
-            in_flight.pop(0).result()
+            last = in_flight.pop(0).result()
+        return last
     return step, finish
 
 
@@ -614,7 +653,9 @@ def bench_c5(ctx, args, steps, warmup):
     sampler = ClockSampler(ctx.local) if rank == 0 else None
     filt_events.clear()
     launches0 = ctx.native.launch_count
-    ms_total = ctx.timed(step_device, steps, finish_device)
+    last = []
+    ms_total = ctx.timed(step_device, steps, lambda: last.append(finish_device()))
+    ctx.outputs = host_lists(last[0])
     launches = ctx.native.launch_count - launches0
     filt_ms = [a.elapsed_time(b) for a, b in filt_events]
     clocks = sampler.stop() if sampler else None
@@ -758,7 +799,9 @@ def bench_c4(ctx, args, steps, warmup):
     finish_device()
     filt_events.clear()
     launches0 = ctx.native.launch_count
-    ms_total = ctx.timed(step_device, steps, finish_device)
+    last = []
+    ms_total = ctx.timed(step_device, steps, lambda: last.append(finish_device()))
+    ctx.outputs = host_lists(last[0])              # before the graph's output buffers are replayed into again
     launches = ctx.native.launch_count - launches0
     filt_ms = [a.elapsed_time(b) for a, b in filt_events]
     ms_eager = None
@@ -904,7 +947,9 @@ def bench_c3(ctx, args, steps, warmup):
     finish_device()
     filt_events.clear()
     launches0 = ctx.native.launch_count
-    ms_total = ctx.timed(step_device, steps, finish_device)
+    last = []
+    ms_total = ctx.timed(step_device, steps, lambda: last.append(finish_device()))
+    ctx.outputs = host_lists(last[0])              # before the graph's output buffers are replayed into again
     launches = ctx.native.launch_count - launches0
     filt_ms = [a.elapsed_time(b) for a, b in filt_events]
     ms_eager = None
@@ -1019,7 +1064,9 @@ def bench_c2(ctx, args, steps, warmup):
         step_device()
     f64_events.clear()
     launches0 = ctx.native.launch_count
-    ms_total = ctx.timed(step_device, steps)
+    last = []
+    ms_total = ctx.timed(lambda: last.append(step_device()), steps)
+    ctx.outputs = {"perf": last[-1]}                     # [v2t, t2v] x (R@1, R@5, R@10, MedR, MeanR, mAP)
     launches = ctx.native.launch_count - launches0
     f64_ms = [a.elapsed_time(b) for a, b in f64_events]
     step_e2e()
@@ -1094,6 +1141,8 @@ def run_b200_arm(args):
     ctx = Ctx()
     warmup = max(args.warmup, 3)
     line = BENCHES[args.config](ctx, args, args.steps, warmup)
+    if args.dump_outputs and ctx.rank == 0:
+        dump_outputs(args.dump_outputs, ctx.outputs)
     solo = ctx.rank == 0 and ctx.world == 1 and not args.skip_cpu_baseline
     if solo:
         use_all_host_cores()
