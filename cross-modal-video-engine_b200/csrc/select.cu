@@ -449,7 +449,13 @@ select_topk_kernel(const double* __restrict__ score, const IdxT* __restrict__ id
   }
   if (threadIdx.x == 0) {
     if (out_valid) out_valid[r] = n_all;
-    if (cert != nullptr) {
+    if (cert != nullptr && thr == nullptr) {
+      // no threshold (a shard's local list before the merge): report only whether the list is exact -- no candidate
+      // overflow, and every entry that can belong to the top-k fit the sort (else it holds an arbitrary subset of
+      // more than pmax float-tied scores)
+      cert[r] = (!cand_overflow && n_valid <= pmax) ? 1 : 0;
+      if (n_uncertified != nullptr && cert[r] == 0) atomicAdd(n_uncertified, 1);
+    } else if (cert != nullptr) {
       const float t = thr[r];
       const bool enough = n >= k && n_valid <= pmax;
       const double kth = enough ? keys[k - 1] : -CUDART_INF;
@@ -608,14 +614,15 @@ int launch_select(const double* score, const IdxT* idx, int64_t rows, int64_t co
                   int64_t* out_idx, int32_t* out_valid, int32_t* cert, float* thr_next, int32_t* n_uncertified,
                   cudaStream_t st) {
   XMVE_REQUIRE(score && out_score && out_idx && rows >= 0 && cols > 0 && k > 0, "select_topk: bad arguments");
-  XMVE_REQUIRE(cert == nullptr || thr != nullptr, "select_topk: cert needs thr");
+  XMVE_REQUIRE(thr_next == nullptr || thr != nullptr, "select_topk: thr_next needs thr");
   if (rows == 0) return XMVE_OK;
   int pmax = pow2_ceil(cols);
   if (pmax > 16384) pmax = 16384;
   // Many rows: a modest sort capacity keeps several blocks resident per SM (the full 16384-entry buffer is 196 KB:
   // one block per SM, 1.7 ms for 8192 rows of ~500 valid entries each).  Rows with more valid entries than the
-  // capacity are first cut at their k-th largest rounded score (see the kernel); the few rows that still do not fit
-  // come back uncertified and are re-run in a small batch, which gets the full capacity.
+  // capacity are first cut at their k-th largest rounded score (see the kernel); the rows that still do not fit come
+  // back uncertified (without thr: cert = 0) and the engine re-runs them in batches of fewer than 512 rows, which get
+  // the full capacity.
   if (rows >= 512) {
     int small = pow2_ceil(4 * static_cast<int64_t>(k));
     if (small < 2048) small = 2048;

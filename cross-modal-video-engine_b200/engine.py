@@ -157,6 +157,7 @@ class CorpusStore:
         self.norm = torch.empty((len(self.dims), max(self.capacity, 1)), dtype=torch.float64, device=self.device)
         self.resid = torch.zeros((len(self.dims), max(self.capacity, 1)), dtype=torch.float32, device=self.device)
         self._resid_max2 = None
+        self.added = None                                     # CUDA event after the last add's kernels
         self.space_off = (C.c_int32 * (len(self.dims) + 1))(*([0] + list(_cumsum(self.dims))))
 
     # -- ingest ----------------------------------------------------------------------------------
@@ -174,6 +175,9 @@ class CorpusStore:
                          self.op[self.n:], op_off, N.OP_X1, 1.0, self.norm_mode)
                 op_off += dp
                 raw_off += d
+            # a search's head stream (search_shards(head_stream=...)) reads the new rows: it waits for this event
+            self.added = torch.cuda.Event()
+            self.added.record()
         self.n += n
         return self
 
@@ -308,7 +312,8 @@ class CorpusStore:
         cap = cand_score.shape[1]
         if exact is None:
             exact = torch.empty((nq, cap), dtype=torch.float64, device=self.device)
-        N.call("xmve_rescore", N.ptr(q_raw), nq, q_raw.stride(0), N.ptr(q_norm), N.ptr(self.raw), self.n,
+        # the norm planes are [S, capacity]: their row stride, not the number of rows filled, locates space s
+        N.call("xmve_rescore", N.ptr(q_raw), nq, q_raw.stride(0), N.ptr(q_norm), N.ptr(self.raw), self.norm.stride(0),
                self.raw.stride(0), N.ptr(self.norm), len(self.dims), self.space_off, self._weights_arr(wts),
                self.norm_mode, N.ptr(cand_score), N.ptr(cand_idx), N.ptr(cand_count), cap, N.ptr(bound),
                N.ptr(bound_hi), N.ptr(exact), N.stream_ptr())
@@ -323,12 +328,15 @@ class CorpusStore:
         return out
 
     def _select(self, exact, cand, nq, k, excl, thr, eps_t, bound, out_s, out_i, certify, n_bad=None):
-        """Local top-k (global row ids) of the rescored candidates into ``out_s`` / ``out_i`` (+ certificate)."""
+        """Local top-k (global row ids) of the rescored candidates into ``out_s`` / ``out_i`` -> ``(cert, thr_next)``.
+        ``certify=False`` (a shard's list for the merge): ``cert`` says whether the list is exact -- 0 after a
+        candidate-list overflow or when more float-tied scores than the sort holds had to be cut -- and ``thr_next``
+        is None."""
         cand_count, cand_score, cand_idx = cand
         cap = cand_score.shape[1]
-        cert = thr_next = None
+        thr_next = None
+        cert = torch.empty((nq,), dtype=torch.int32, device=self.device)
         if certify:
-            cert = torch.empty((nq,), dtype=torch.int32, device=self.device)
             thr_next = torch.empty((nq,), dtype=torch.float32, device=self.device)
         N.call("xmve_select_topk_i32", N.ptr(exact), N.ptr(cand_idx), nq, cap, N.ptr(cand_count),
                self.index_offset, N.ptr(excl), k, N.ptr(thr) if certify else None, 1.0, N.ptr(eps_t),
@@ -501,6 +509,9 @@ def _segments(parts, comm):
 PILOT_MAX = 1000
 #: ... and the union of the pilots of all shards at most this many (xmve_pilot_bound sorts it in shared memory)
 PILOT_UNION_MAX = 4096
+#: re-run passes select at most this many rows per launch: from 512 rows on, the selection kernels shrink their sort
+#: to max(2048, 4k) entries per row (xmve_select_topk_*), which is what the rows being re-run may not have fitted
+SELECT_RERUN_ROWS = 511
 
 
 class PendingSearch:
@@ -608,28 +619,17 @@ class _Search:
             exacts = [s._rescore(q_sub, qn_sub, n_sub, self.wts, c, bound) for s, c in zip(self.live, cands)]
         ph.mark("rescore")
         # 5: selection.  One shard: the local kernel certifies.  Several: packed local lists, ONE gather, K3.
+        # With 512 rows or more the selection kernels sort at most max(2048, 4k) entries per row; a re-run selects in
+        # smaller batches, so that the rows whose lists did not fit (heavy float ties) get the full 16 384 entries.
         n_bad = torch.zeros((1,), dtype=torch.int32, device=dev)
-        if self.solo:
-            s_ = torch.empty((n_sub, k_eff), dtype=torch.float64, device=dev)
-            i_ = torch.empty((n_sub, k_eff), dtype=torch.int64, device=dev)
-            cert, thr_next = self.live[0]._select(exacts[0], cands[0], n_sub, k_eff, ex_sub, thr_sub, eps_t, bound,
-                                                  s_, i_, True, n_bad)
-            over = ("lists", [cands[0][0]], cap)
+        batch = n_sub if rows is None else SELECT_RERUN_ROWS
+        parts = [self._select_rows(r0, min(n_sub, r0 + batch), cands, exacts, ex_sub, thr_sub, bound, n_bad)
+                 for r0 in range(0, n_sub, batch)]
+        if len(parts) == 1:
+            s_, i_, cert, thr_next, over = parts[0]
         else:
-            seg = packed_bytes(n_sub, k_eff)
-            blocks = torch.empty((max(len(self.live), 1), seg), dtype=torch.uint8, device=dev)
-            for li, (s, c, e) in enumerate(zip(self.live, cands, exacts)):
-                b_s, b_i, b_f = packed_views(blocks[li], n_sub, k_eff)
-                s._select(e, c, n_sub, k_eff, ex_sub, None, eps_t, None, b_s, b_i, False)
-                b_f.copy_(c[0] > cap)
-            if not self.live:
-                b_s, b_i, b_f = packed_views(blocks[0], n_sub, k_eff)
-                b_s.fill_(float("-inf"))
-                b_i.fill_(-1)
-                b_f.zero_()
-            gathered = blocks if comm.world == 1 else comm.gather(blocks).view(-1, seg)
-            s_, i_, cert, thr_next = _merge_packed(gathered, n_sub, k_eff, k_eff, thr_sub, eps_t, n_bad)
-            over = ("packed", gathered, n_sub, k_eff)
+            s_, i_, cert, thr_next = (torch.cat([p[j] for p in parts]) for j in range(4))
+            over = ("parts", [p[4] for p in parts])
         ph.mark("select_merge")
         if self.stats is not None and rows is None:
             st = self.stats
@@ -643,6 +643,35 @@ class _Search:
                 for c, e in zip(cands, exacts)) / max(n_sub, 1)
             ph.mark("stats_bookkeeping")
         return s_, i_, cert, thr_next, over, n_bad, thr_sub
+
+    def _select_rows(self, r0, r1, cands, exacts, ex_sub, thr_sub, bound, n_bad):
+        """Step 5 for rows ``r0:r1`` of a pass -> (scores, idx, cert, thr_next, overflow descriptor)."""
+        dev, k_eff, eps_t, cap = self.dev, self.k_eff, self.eps_t, self.cap
+        n = r1 - r0
+        cands = [tuple(t[r0:r1] for t in c) for c in cands]
+        exacts = [e[r0:r1] for e in exacts]
+        ex = ex_sub[r0:r1] if ex_sub is not None else None
+        thr = thr_sub[r0:r1]
+        if self.solo:
+            s_ = torch.empty((n, k_eff), dtype=torch.float64, device=dev)
+            i_ = torch.empty((n, k_eff), dtype=torch.int64, device=dev)
+            cert, thr_next = self.live[0]._select(exacts[0], cands[0], n, k_eff, ex, thr, eps_t, bound[r0:r1], s_, i_,
+                                                  True, n_bad)
+            return s_, i_, cert, thr_next, ("lists", [cands[0][0]], cap)
+        seg = packed_bytes(n, k_eff)
+        blocks = torch.empty((max(len(self.live), 1), seg), dtype=torch.uint8, device=dev)
+        for li, (s, c, e) in enumerate(zip(self.live, cands, exacts)):
+            b_s, b_i, b_f = packed_views(blocks[li], n, k_eff)
+            exact_list, _ = s._select(e, c, n, k_eff, ex, None, eps_t, None, b_s, b_i, False)
+            b_f.copy_(exact_list == 0)                        # overflowed, or cut short by float ties
+        if not self.live:
+            b_s, b_i, b_f = packed_views(blocks[0], n, k_eff)
+            b_s.fill_(float("-inf"))
+            b_i.fill_(-1)
+            b_f.zero_()
+        gathered = blocks if self.comm.world == 1 else self.comm.gather(blocks).view(-1, seg)
+        s_, i_, cert, thr_next = _merge_packed(gathered, n, k_eff, k_eff, thr, eps_t, n_bad)
+        return s_, i_, cert, thr_next, ("packed", gathered, n, k_eff)
 
     def first_pass(self, in_graph=False, flag_host=None):
         self._cap0 = self.cap
@@ -684,6 +713,8 @@ class _Search:
     @staticmethod
     def _overflowed(over):
         """Per-row overflow flags of a pass (formed only when rows are re-run)."""
+        if over[0] == "parts":
+            return torch.cat([_Search._overflowed(o) for o in over[1]])
         if over[0] == "lists":
             return over[1][0] > over[2]
         _, gathered, n_sub, k_eff = over
@@ -741,7 +772,7 @@ class GraphSearch:
     every rank replays in lockstep (``tools/check_sharded.py`` / ``tools/graph_sharded_check.py``: identical to the
     eager search; 0.94 -> 0.64 ms for 60 queries over two 135 k-row shards, where the ~40 launches of the eager step
     are what bounds it).  The returned tensors are the graph's static output buffers and are overwritten by the
-    next call.
+    next call.  The graph covers the rows the stores held at capture: a call after :meth:`CorpusStore.add` raises.
     """
 
     def __init__(self, stores, n_queries, k, weights=None, with_exclude=False, comm=None, n_total=None,
@@ -773,10 +804,16 @@ class GraphSearch:
                                                small_nv, None, self.comm, n_total, in_graph=True,
                                                flag_host=self._flag_host)
         self.scores, self.idx = self._pending.scores, self._pending.idx
+        self.rows = tuple(s.n for s in self.stores)           # the captured kernels cover exactly these rows
 
     def __call__(self, queries, exclude=None, defer=False):
         q = queries if torch.is_tensor(queries) else torch.as_tensor(queries)
         assert tuple(q.shape) == tuple(self.q_in.shape), "GraphSearch was captured for %s queries" % (self.q_in.shape,)
+        rows = tuple(s.n for s in self.stores)
+        if rows != self.rows:
+            raise RuntimeError("GraphSearch: the corpus changed since the capture (rows per store %s, now %s); the "
+                               "captured kernels would not see the new rows -- capture a new GraphSearch"
+                               % (list(self.rows), list(rows)))
         with torch.cuda.device(self.dev):
             self.q_in.copy_(q, non_blocking=True)
             if self.excl_in is not None:
@@ -836,7 +873,9 @@ def search_shards(stores, queries, k, weights=None, exclude=None, eps=None, smal
     search in flight the K1 / sampling / threshold work of batch i+1 runs next to the rescore / selection / merge of
     batch i as soon as FILTER(i) has left the SMs, instead of behind it -- both are short, latency-bound kernel
     chains (1.2 ms + 1.9 ms of a 31 ms step on 8 GPUs).  The queries must be complete when the call is made, or have
-    been produced on ``head_stream`` (it does not wait for the current stream).
+    been produced on ``head_stream`` (it does not wait for the current stream).  The head does wait for the last
+    :meth:`CorpusStore.add` of every store it reads (an event recorded by ``add``), so a search issued straight after
+    an ``add`` sees the new rows and their residuals.
     """
     comm = comm or SoloComm()
     ref = stores[0]
@@ -876,6 +915,9 @@ def _search_shards(stores, queries, k, weights, exclude, eps, small_nv, stats, c
         for t in (queries if isinstance(queries, (list, tuple)) else (queries, exclude)):
             if torch.is_tensor(t) and t.is_cuda:
                 t.record_stream(head_stream)                  # the caller may drop it while the head still reads it
+        for s in stores:                                      # the head reads the stores' rows and residuals: only
+            if getattr(s, "added", None) is not None:         # their last add, not the whole current stream, must
+                head_stream.wait_event(s.added)               # be complete
     with _head_on(head_stream):
         a_op, q_raw, q_norm, q_res, nq = ref.prepare_queries(queries, wts)
         excl = None

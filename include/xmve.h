@@ -127,7 +127,9 @@ XMVE_API int xmve_row_kth(const float* vals, int64_t rows, int64_t cols, int64_t
  * reference keeps in float64 arrays, evaluation.py:102-105); products and sums are in fp64, i.e.
  * the arithmetic of cal_error on float64 inputs (evaluation.py:19-21) up to rounding order.
  * space_off[n_space+1] (HOST array) are column offsets into the raw rows, weights[n_space] is a HOST
- * array, q_norm/v_norm are DEVICE [n_space, n] fp64.  exact[q, c] is written for c < cand_count[q] only.
+ * array, q_norm is DEVICE [n_space, nq] fp64 and v_norm DEVICE [n_space, nv] fp64: nv is the row stride of v_norm
+ * (a corpus store's capacity, which may exceed the number of rows filled), the norm of corpus row v in space s is
+ * v_norm[s * nv + v].  exact[q, c] is written for c < cand_count[q] only.
  * norm_mode as in xmve_prepare_rows.  Limit: total raw dim <= 6000.
  */
 XMVE_API int xmve_rescore(const float* q_raw, int64_t nq, int64_t q_ld, const double* q_norm,
@@ -171,8 +173,11 @@ XMVE_API int xmve_eps_bound(const float* q_resid, int32_t n_space, int64_t nq, c
  * - 2 eps after a candidate-list overflow).  The sort holds 16384 entries per row; rows with more valid entries
  * are first cut at the k-th largest score rounded to float (a superset of the exact top-k), so only > 16384
  * scores that agree with the k-th to float precision defeat it (reported as not certified).  (With 512 rows or more
- * the sort holds max(2048, 4k) entries so that several rows are resident per SM; the rare row that does not fit comes
- * back uncertified and is re-run in a small batch with the full capacity.)
+ * the sort holds max(2048, 4k) entries so that several rows are resident per SM; a row that does not fit comes
+ * back uncertified and must be re-run in a batch of fewer than 512 rows to get the full capacity.)
+ * Without thr (a shard's local list that a later merge certifies), cert may still be given: cert[r] = 1 iff the
+ * list is exact -- counts[r] <= cols and every entry that can belong to the top-k fit the sort -- and 0 when the
+ * sort held only an arbitrary subset of tied entries; thr_next must then be NULL.
  * eps_dev (DEVICE scalar, may be NULL) multiplies eps.  n_uncertified (DEVICE int32, may be NULL) is incremented once
  * per uncertified row: the caller reads ONE scalar, asynchronously, instead of scanning cert on the host.
  */

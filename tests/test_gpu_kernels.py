@@ -334,46 +334,53 @@ def test_select_topk_more_valid_entries_than_the_sort_holds(N):
 
 
 def test_rescore_is_fp64_exact(N):
+    """Two spaces, a bound and the two-round window.  Second case: the corpus norms sit in planes WIDER than the rows
+    in use (a store filled below its capacity; the padding is NaN, so reading it shows), passed with their row stride
+    as ``nv``, and a space width that is not a multiple of 4 (97 + 31), which takes the scalar fallback loop."""
     import ctypes as C
     nq, nv, cap = 33, 5000, 64
-    dims = (100, 28)
-    g = torch.Generator(device="cuda").manual_seed(4)
-    q = torch.randn((nq, 128), generator=g, device="cuda")
-    v = torch.randn((nv, 128), generator=g, device="cuda")
-    qn = torch.stack([torch.linalg.vector_norm(q[:, :100].double(), dim=1), torch.linalg.vector_norm(q[:, 100:].double(), dim=1)])
-    vn = torch.stack([torch.linalg.vector_norm(v[:, :100].double(), dim=1), torch.linalg.vector_norm(v[:, 100:].double(), dim=1)])
-    idx = torch.randint(0, nv, (nq, cap), generator=g, device="cuda", dtype=torch.int32)
-    approx = torch.randn((nq, cap), generator=g, device="cuda")
-    count = torch.randint(0, cap + 20, (nq,), generator=g, device="cuda", dtype=torch.int32)
-    bound = torch.zeros(nq, device="cuda")
-    exact = torch.full((nq, cap), 123.0, dtype=torch.float64, device="cuda")
-    off = (C.c_int32 * 3)(0, 100, 128)
-    w = (C.c_double * 2)(0.7, 0.3)
-    N.call("xmve_rescore", N.ptr(q), nq, 128, N.ptr(qn), N.ptr(v), nv, 128, N.ptr(vn), 2, off, w, 0, N.ptr(approx),
-           N.ptr(idx), N.ptr(count), cap, N.ptr(bound), None, N.ptr(exact), N.stream_ptr())
-    # two rounds give the same array: [0.5, inf) first, then [-0.3, 0.5) with the first round left untouched
-    hi = torch.full((nq,), 0.5, device="cuda")
-    lo = torch.full((nq,), -0.3, device="cuda")
-    two = torch.full((nq, cap), 123.0, dtype=torch.float64, device="cuda")
-    N.call("xmve_rescore", N.ptr(q), nq, 128, N.ptr(qn), N.ptr(v), nv, 128, N.ptr(vn), 2, off, w, 0, N.ptr(approx),
-           N.ptr(idx), N.ptr(count), cap, N.ptr(hi), None, N.ptr(two), N.stream_ptr())
-    first = two.clone()
-    N.call("xmve_rescore", N.ptr(q), nq, 128, N.ptr(qn), N.ptr(v), nv, 128, N.ptr(vn), 2, off, w, 0, N.ptr(approx),
-           N.ptr(idx), N.ptr(count), cap, N.ptr(lo), N.ptr(hi), N.ptr(two), N.stream_ptr())
-    one = torch.full((nq, cap), 123.0, dtype=torch.float64, device="cuda")
-    N.call("xmve_rescore", N.ptr(q), nq, 128, N.ptr(qn), N.ptr(v), nv, 128, N.ptr(vn), 2, off, w, 0, N.ptr(approx),
-           N.ptr(idx), N.ptr(count), cap, N.ptr(lo), None, N.ptr(one), N.stream_ptr())
-    assert torch.equal(two, one)
-    assert torch.equal(two[approx >= 0.5], first[approx >= 0.5])
-    for r in range(nq):
-        n = min(int(count[r]), cap)
-        rows = v[idx[r, :n].long()].double()
-        s = 0.7 * (rows[:, :100] @ q[r, :100].double()) / (qn[0, r] * vn[0, idx[r, :n].long()]) \
-            + 0.3 * (rows[:, 100:] @ q[r, 100:].double()) / (qn[1, r] * vn[1, idx[r, :n].long()])
-        keep = approx[r, :n] >= 0
-        assert torch.all(exact[r, :n][~keep] == float("-inf"))
-        torch.testing.assert_close(exact[r, :n][keep], s[keep], rtol=0, atol=1e-14)
-        assert torch.all(exact[r, n:] == 123.0)             # slots past the count are never written
+    for d0, pad in ((100, 0), (97, 37)):
+        g = torch.Generator(device="cuda").manual_seed(4)
+        q = torch.randn((nq, 128), generator=g, device="cuda")
+        v = torch.randn((nv, 128), generator=g, device="cuda")
+        qn = torch.stack([torch.linalg.vector_norm(q[:, :d0].double(), dim=1),
+                          torch.linalg.vector_norm(q[:, d0:].double(), dim=1)])
+        vn = torch.full((2, nv + pad), float("nan"), dtype=torch.float64, device="cuda")
+        vn[0, :nv] = torch.linalg.vector_norm(v[:, :d0].double(), dim=1)
+        vn[1, :nv] = torch.linalg.vector_norm(v[:, d0:].double(), dim=1)
+        ld = vn.stride(0)
+        idx = torch.randint(0, nv, (nq, cap), generator=g, device="cuda", dtype=torch.int32)
+        approx = torch.randn((nq, cap), generator=g, device="cuda")
+        count = torch.randint(0, cap + 20, (nq,), generator=g, device="cuda", dtype=torch.int32)
+        bound = torch.zeros(nq, device="cuda")
+        exact = torch.full((nq, cap), 123.0, dtype=torch.float64, device="cuda")
+        off = (C.c_int32 * 3)(0, d0, 128)
+        w = (C.c_double * 2)(0.7, 0.3)
+        N.call("xmve_rescore", N.ptr(q), nq, 128, N.ptr(qn), N.ptr(v), ld, 128, N.ptr(vn), 2, off, w, 0, N.ptr(approx),
+               N.ptr(idx), N.ptr(count), cap, N.ptr(bound), None, N.ptr(exact), N.stream_ptr())
+        # two rounds give the same array: [0.5, inf) first, then [-0.3, 0.5) with the first round left untouched
+        hi = torch.full((nq,), 0.5, device="cuda")
+        lo = torch.full((nq,), -0.3, device="cuda")
+        two = torch.full((nq, cap), 123.0, dtype=torch.float64, device="cuda")
+        N.call("xmve_rescore", N.ptr(q), nq, 128, N.ptr(qn), N.ptr(v), ld, 128, N.ptr(vn), 2, off, w, 0, N.ptr(approx),
+               N.ptr(idx), N.ptr(count), cap, N.ptr(hi), None, N.ptr(two), N.stream_ptr())
+        first = two.clone()
+        N.call("xmve_rescore", N.ptr(q), nq, 128, N.ptr(qn), N.ptr(v), ld, 128, N.ptr(vn), 2, off, w, 0, N.ptr(approx),
+               N.ptr(idx), N.ptr(count), cap, N.ptr(lo), N.ptr(hi), N.ptr(two), N.stream_ptr())
+        one = torch.full((nq, cap), 123.0, dtype=torch.float64, device="cuda")
+        N.call("xmve_rescore", N.ptr(q), nq, 128, N.ptr(qn), N.ptr(v), ld, 128, N.ptr(vn), 2, off, w, 0, N.ptr(approx),
+               N.ptr(idx), N.ptr(count), cap, N.ptr(lo), None, N.ptr(one), N.stream_ptr())
+        assert torch.equal(two, one)
+        assert torch.equal(two[approx >= 0.5], first[approx >= 0.5])
+        for r in range(nq):
+            n = min(int(count[r]), cap)
+            rows = v[idx[r, :n].long()].double()
+            s = 0.7 * (rows[:, :d0] @ q[r, :d0].double()) / (qn[0, r] * vn[0, idx[r, :n].long()]) \
+                + 0.3 * (rows[:, d0:] @ q[r, d0:].double()) / (qn[1, r] * vn[1, idx[r, :n].long()])
+            keep = approx[r, :n] >= 0
+            assert torch.all(exact[r, :n][~keep] == float("-inf"))
+            torch.testing.assert_close(exact[r, :n][keep], s[keep], rtol=0, atol=1e-14)
+            assert torch.all(exact[r, n:] == 123.0)             # slots past the count are never written
 
 
 def test_score_f64_and_normalize(N):
@@ -575,3 +582,42 @@ def test_select_topk_many_rows_use_the_small_sort(N):
     assert int(n_bad) == 0 and bool((cert == 1).all())
     top_s, top_p = torch.topk(score, k, dim=1)
     assert torch.equal(out_s, top_s) and torch.equal(out_i, torch.gather(idx.long(), 1, top_p))
+
+
+@pytest.mark.parametrize("rows", [600, 511])
+def test_select_topk_reports_a_list_cut_by_float_ties(N, rows):
+    """A shard's list before the merge (no threshold): row 7 holds 3 000 float-tied scores on top.  With 512 rows or
+    more the sort holds max(2048, 4k) entries, so the kernel keeps an arbitrary 2 048 of the ties and must say so
+    (cert = 0) for that row only; with 511 rows (the batches the engine re-runs such rows in) the sort holds them all
+    and the list is the 100 smallest indices of the ties."""
+    cols, k = 4096, 100
+    g = torch.Generator(device="cuda").manual_seed(34)
+    score = torch.randn((rows, cols), generator=g, device="cuda", dtype=torch.float64)
+    score[:, 300:] = float("-inf")
+    score[7] = torch.randn(cols, generator=g, device="cuda", dtype=torch.float64) - 5.0
+    score[7, 500:3500] = 0.8                                                                    # 3 000 exact ties
+    idx = torch.stack([torch.randperm(cols, generator=g, device="cuda") for _ in range(rows)]).int()
+    counts = torch.full((rows,), cols, dtype=torch.int32, device="cuda")
+    out_s = torch.empty((rows, k), dtype=torch.float64, device="cuda")
+    out_i = torch.empty((rows, k), dtype=torch.int64, device="cuda")
+    cert = torch.full((rows,), 7, dtype=torch.int32, device="cuda")
+    n_bad = torch.zeros(1, dtype=torch.int32, device="cuda")
+    N.call("xmve_select_topk_i32", N.ptr(score), N.ptr(idx), rows, cols, N.ptr(counts), 0, None, k, None, 0.0,
+           None, None, N.ptr(out_s), N.ptr(out_i), None, N.ptr(cert), None, N.ptr(n_bad), N.stream_ptr())
+    want = torch.ones(rows, dtype=torch.int32, device="cuda")
+    if rows >= 512:
+        want[7] = 0
+    assert torch.equal(cert, want) and int(n_bad) == int((want == 0).sum())
+    ids = idx.long()
+    for r in range(rows):
+        if int(want[r]) == 0:
+            continue
+        order = torch.argsort(ids[r], stable=True)                                 # index ascending ...
+        top = torch.argsort(score[r][order], descending=True, stable=True)[:k]     # ... then score descending
+        assert torch.equal(out_s[r], score[r][order][top]) and torch.equal(out_i[r], ids[r][order][top])
+    if rows < 512:
+        assert torch.equal(out_i[7], torch.sort(ids[7, 500:3500]).values[:k])
+    with pytest.raises(N.XmveError, match="thr_next"):                            # a next threshold needs a threshold
+        N.call("xmve_select_topk_i32", N.ptr(score), N.ptr(idx), rows, cols, N.ptr(counts), 0, None, k, None, 0.0,
+               None, None, N.ptr(out_s), N.ptr(out_i), None, N.ptr(cert), N.ptr(torch.empty(rows, device="cuda")),
+               None, N.stream_ptr())
