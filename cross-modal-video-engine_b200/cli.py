@@ -1,6 +1,7 @@
 """Command-line front ends of the scoring path on precomputed embeddings (SURVEY.md section 8f row 3).
 
     python -m cross_modal_video_engine_b200.cli search --corpus DIR|video_data.pt --queries Q.npy --topK 10
+        [--labels L.npy --label-mask MASK|M.npy]     (only rows whose label bit is set in the query's mask)
     python -m cross_modal_video_engine_b200.cli eval   --corpus DIR|video_data.pt --queries Q.npy --caption-ids ids.txt
     python -m cross_modal_video_engine_b200.cli composed --index index.pt --queries queries.pt [--out results_wo_attn]
 
@@ -67,6 +68,9 @@ def parse_args(argv=None):
     s = sub.choices["search"]
     s.add_argument("--query-ids", default=None)
     s.add_argument("--run-file", default=None, help="write a TREC run file instead of printing id lists")
+    s.add_argument("--labels", default=None, help=".npy of one label in [0, 64) per corpus row (uint8)")
+    s.add_argument("--label-mask", default=None,
+                   help="search only rows whose label bit is set: one 64-bit integer, or a .npy with one per query")
     e = sub.choices["eval"]
     e.add_argument("--caption-ids", required=True, help="caption ids 'video7#enc#3' (util/metrics.py:111), one per query")
     e.add_argument("--save-topk", default=None, help="save {'scores','idx','video_ids'} of the top-K lists here")
@@ -81,6 +85,10 @@ def parse_args(argv=None):
     args.weights = tuple(float(x) for x in args.weights.split(",")) if args.weights else None
     if args.dims and args.weights and len(args.dims) != len(args.weights):
         ap.error("--weights needs one value per entry of --dims")
+    if args.cmd == "search" and args.label_mask is not None:
+        if args.labels is None:
+            ap.error("--label-mask needs --labels")
+        args.label_mask = np.load(args.label_mask) if args.label_mask.endswith(".npy") else int(args.label_mask, 0)
     return args
 
 
@@ -92,7 +100,10 @@ def main(argv=None):
     store, video_ids = _load_corpus(args.corpus, args.dims)
     q = _load_matrix(args.queries)
     if args.cmd == "search":
-        scores, idx = store.search(q, args.topK, weights=args.weights)
+        if args.labels is not None:
+            labels = np.load(args.labels)
+            store.set_labels(np.arange(store.n) + store.index_offset, labels)
+        scores, idx = store.search(q, args.topK, weights=args.weights, label_mask=args.label_mask)
         if args.run_file:
             avs.write_run_file(args.run_file, _ids(args.query_ids, len(q), "q"), idx, scores, video_ids)
         else:

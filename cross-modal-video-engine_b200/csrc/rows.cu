@@ -215,6 +215,18 @@ normalize_f64_kernel(const T* __restrict__ src, int64_t n, int d, int64_t src_ld
   for (int i = lane; i < d; i += 32) o[i] = static_cast<double>(r[i]) / nrm;   // 1.0 * X / norm
 }
 
+// One thread per column: its label is read once, then the column is masked in every row (grid-stride over rows).
+template <typename T>
+__global__ void __launch_bounds__(256)
+mask_scores_kernel(T* __restrict__ scores, int64_t rows, int64_t cols, int64_t ld, const uint8_t* __restrict__ labels,
+                   int64_t label_step, const uint64_t* __restrict__ allow) {
+  const int64_t c = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (c >= cols) return;
+  const uint32_t lab = labels[c * label_step];
+  for (int64_t r = blockIdx.y; r < rows; r += gridDim.y)
+    if (((allow[r] >> lab) & 1ull) == 0) scores[r * ld + c] = -INFINITY;
+}
+
 }  // namespace
 }  // namespace xmve
 
@@ -286,4 +298,24 @@ extern "C" int xmve_normalize_f64(const void* src, int src_dtype, int64_t n, int
     normalize_f64_kernel<double><<<grid, WARPS * 32, 0, st>>>(static_cast<const double*>(src), n, d, src_ld, dst,
                                                               dst_ld, norm_mode);
   return launch_status("normalize_f64_kernel");
+}
+
+extern "C" int xmve_mask_scores(void* scores, int dtype, int64_t rows, int64_t cols, int64_t ld,
+                                const uint8_t* labels, int64_t label_step, const uint64_t* allow, void* stream) {
+  using namespace xmve;
+  XMVE_DEVICE_OR_RETURN();
+  XMVE_REQUIRE(scores != nullptr && labels != nullptr && allow != nullptr && rows >= 0 && cols >= 0 && ld >= cols &&
+                   label_step >= 1,
+               "mask_scores: bad arguments");
+  XMVE_REQUIRE(dtype == XMVE_F32 || dtype == XMVE_F64, "mask_scores: dtype must be f32 or f64");
+  if (rows == 0 || cols == 0) return XMVE_OK;
+  const dim3 grid(static_cast<unsigned>((cols + 255) / 256), static_cast<unsigned>(rows < 65535 ? rows : 65535));
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (dtype == XMVE_F32)
+    mask_scores_kernel<float><<<grid, 256, 0, st>>>(static_cast<float*>(scores), rows, cols, ld, labels, label_step,
+                                                    allow);
+  else
+    mask_scores_kernel<double><<<grid, 256, 0, st>>>(static_cast<double*>(scores), rows, cols, ld, labels,
+                                                     label_step, allow);
+  return launch_status("mask_scores_kernel");
 }

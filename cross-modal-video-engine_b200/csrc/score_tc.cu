@@ -80,6 +80,9 @@ struct Cfg {
   static constexpr int PARK_BYTES = (THREADS - 128) * 2 * 8 * 8;   // two lists of STG (score, index) pairs per
                                                                    // epilogue thread (see flush_parked)
   static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 1024 /*align*/ + 256 /*barriers*/ + PARK_BYTES;
+  static constexpr int LABEL_BYTES = 8 * EPI_COLS;             // labelled FILTER: one label byte per column of the
+                                                               // tile, staged per epilogue warp behind the park lists
+  static constexpr int SMEM_BYTES_LABELED = SMEM_BYTES + LABEL_BYTES;
   static constexpr int TILE_M = BM * CTAS;                     // query rows per tile
   static constexpr int TILE_N = BN * NB;                       // corpus rows per tile
 };
@@ -106,6 +109,11 @@ struct Params {
   int32_t cap;
   int defer_append;                 // FILTER: finish a tile's append one tile later (default; XMVE_DEFER=0 disables)
   int single_hit;                   // FILTER: branch-free extraction of a chunk's only candidate (XMVE_SINGLE_HIT=0 disables)
+  // labelled FILTER: column v has label labels[v * lab_step] < 64; row q lists only columns whose label bit is set
+  // in allow[q] (and counts only those above hi)
+  const uint8_t* labels;
+  const uint64_t* allow;
+  int64_t lab_step;
 };
 
 struct Unit {
@@ -176,7 +184,14 @@ struct RowState {
   int above;         // scores above hi (count_above)
   int n;             // parked candidates
   uint2* stg;
+  uint64_t allow;    // labelled FILTER: label mask of the row
+  const uint8_t* lab;   // ... and the labels of the tile's columns this warp drains (shared memory)
 };
+
+// labelled FILTER: whether column `i` of the chunk starting at tile column `c` may enter the row's list
+__device__ __forceinline__ bool eligible(const RowState& st, int c, int i) {
+  return ((st.allow >> st.lab[c + i]) & 1ull) != 0;
+}
 
 __device__ __forceinline__ void filter_one(const Params& p, RowState& st, float s, int32_t col) {
   if (s > st.hi) {
@@ -191,15 +206,20 @@ __device__ __forceinline__ void filter_one(const Params& p, RowState& st, float 
 }
 
 // 32 consecutive scores of one query row: a tree of 3-input maxima decides whether anything enters the
-// window (rare); only the 3-element groups whose maximum does are examined element by element.
-__device__ __forceinline__ void filter_chunk(const Params& p, const uint32_t (&v)[32], RowState& st, int64_t col) {
+// window (rare); only the 3-element groups whose maximum does are examined element by element.  LABELED: a score
+// that entered the window is dropped (neither listed nor counted) unless its column's label is allowed for the row;
+// the label is read from shared memory only there, so the cost grows with the hits, not with the scores.
+// `c` is the chunk's first column within the warp's share of the tile.
+template <bool LABELED>
+__device__ __forceinline__ void filter_chunk(const Params& p, const uint32_t (&v)[32], RowState& st, int64_t col,
+                                             int c) {
   float m[11];
 #pragma unroll
   for (int g = 0; g < 10; ++g)
     m[g] = max3(__uint_as_float(v[3 * g]), __uint_as_float(v[3 * g + 1]), __uint_as_float(v[3 * g + 2]));
   m[10] = fmaxf(__uint_as_float(v[30]), __uint_as_float(v[31]));
-  const float a = max3(m[0], m[1], m[2]), b = max3(m[3], m[4], m[5]), c = max3(m[6], m[7], m[8]);
-  if (max3(max3(a, b, c), m[9], m[10]) > st.lo) {
+  const float a = max3(m[0], m[1], m[2]), b = max3(m[3], m[4], m[5]), cc = max3(m[6], m[7], m[8]);
+  if (max3(max3(a, b, cc), m[9], m[10]) > st.lo) {
     const int64_t left = p.nv - col;                     // columns of this chunk inside the corpus
     if (p.single_hit && left >= 32) {
       // Only the lanes with a hit are here (the others wait at the reconvergence point), so what this costs is the
@@ -214,7 +234,8 @@ __device__ __forceinline__ void filter_chunk(const Params& p, const uint32_t (&v
         pos = h ? i : pos;
       }
       if (cnt == 1) {                                    // the hit is the chunk's maximum
-        filter_one(p, st, max3(max3(a, b, c), m[9], m[10]), static_cast<int32_t>(col) + pos);
+        if (!LABELED || eligible(st, c, pos))
+          filter_one(p, st, max3(max3(a, b, cc), m[9], m[10]), static_cast<int32_t>(col) + pos);
         return;
       }
     }
@@ -226,7 +247,8 @@ __device__ __forceinline__ void filter_chunk(const Params& p, const uint32_t (&v
         for (int e = 0; e < (g < 10 ? 3 : 2); ++e) {
           const int i = 3 * g + e;
           const float s = __uint_as_float(v[i]);
-          if (s > st.lo && i < lim) filter_one(p, st, s, static_cast<int32_t>(col) + i);
+          if (s > st.lo && i < lim && (!LABELED || eligible(st, c, i)))
+            filter_one(p, st, s, static_cast<int32_t>(col) + i);
         }
       }
     }
@@ -273,7 +295,7 @@ __device__ __forceinline__ void store_chunk(const Params& p, const uint32_t (&v)
 // `release()` hands the slot back to the MMA warp.  It is called as soon as the LAST chunk has arrived in registers,
 // before that chunk is examined: the accumulator is free from then on, and at K = 640 the MMA warp was waiting for
 // this hand-back (profiles/r2b_mma_issue_loop.txt: ~2 try_wait rounds per tile on `tempty`).
-template <int MODE, int COLS, typename Release>
+template <int MODE, int COLS, bool LABELED, typename Release>
 __device__ __forceinline__ void epilogue_slot(const Params& p, uint32_t taddr, RowState& st, int64_t col0,
                                               Release release) {
   const int lane = threadIdx.x & 31;
@@ -284,12 +306,12 @@ __device__ __forceinline__ void epilogue_slot(const Params& p, uint32_t taddr, R
     ptx::tmem_ld_wait();
     ptx::tmem_ld_32x32(taddr + (c + 1) * 32, v1);
     if (MODE == MODE_STORE) store_chunk(p, v0, st.row - lane, col0 + c * 32, reinterpret_cast<float4*>(st.stg - lane * 2 * STG), lane);
-    else filter_chunk(p, v0, st, col0 + c * 32);
+    else filter_chunk<LABELED>(p, v0, st, col0 + c * 32, c * 32);
     ptx::tmem_ld_wait();
     if (c + 2 < COLS / 32) ptx::tmem_ld_32x32(taddr + (c + 2) * 32, v0);
     else release();
     if (MODE == MODE_STORE) store_chunk(p, v1, st.row - lane, col0 + (c + 1) * 32, reinterpret_cast<float4*>(st.stg - lane * 2 * STG), lane);
-    else filter_chunk(p, v1, st, col0 + (c + 1) * 32);
+    else filter_chunk<LABELED>(p, v1, st, col0 + (c + 1) * 32, (c + 1) * 32);
   }
 }
 
@@ -340,7 +362,7 @@ struct UnitFeed {
   }
 };
 
-template <int MODE, bool PAIR, int NB, bool DYN>
+template <int MODE, bool PAIR, int NB, bool DYN, bool LABELED>
 __device__ __forceinline__ void score_body(const CUtensorMap& tm_a, const CUtensorMap& tm_b, const Params& p) {
   using C = Cfg<PAIR, NB>;
   extern __shared__ uint8_t smem_raw[];
@@ -514,6 +536,10 @@ __device__ __forceinline__ void score_body(const CUtensorMap& tm_a, const CUtens
     uint2* const lists = park + (threadIdx.x - EPI_WARP0 * 32) * (2 * STG);
     st.stg = lists;
     st.n = 0;
+    // labelled FILTER: this warp's label bytes, behind the park lists
+    uint8_t* const labs = reinterpret_cast<uint8_t*>(park + (C::THREADS - 128) * 2 * STG) + (warp - EPI_WARP0) * C::EPI_COLS;
+    st.lab = labs;
+    st.allow = 0;
     // the append of the previous tile that is still to be finished (its atomicAdd is in flight)
     int pend_n = 0, pend_base = 0;
     int64_t pend_row = 0;
@@ -534,10 +560,28 @@ __device__ __forceinline__ void score_body(const CUtensorMap& tm_a, const CUtens
         if (MODE == MODE_FILTER && st.row < p.nq) {
           st.lo = p.lo[st.row];
           if (p.hi != nullptr) st.hi = p.hi[st.row];
+          if (LABELED) st.allow = p.allow[st.row];
+        }
+        // labelled FILTER: the loads of the tile's column labels are issued before the wait on the accumulator, so
+        // that they complete behind it; the shared-memory copy is read by the hit paths of every lane
+        uint32_t lab4 = 0;
+        if constexpr (LABELED) {
+#pragma unroll
+          for (int e = 0; e < C::EPI_COLS / 32; ++e) {
+            const int64_t v = col0 + lane * (C::EPI_COLS / 32) + e;
+            const uint32_t l = v < p.nv ? p.labels[v * p.lab_step] : 0u;
+            lab4 |= l << (8 * e);
+          }
         }
         ptx::mbar_wait(&tfull_bar[slot], acc_phase);
         ptx::tc_fence_after_sync();
-        epilogue_slot<MODE, C::EPI_COLS>(p, tmem_base + lane_addr + slot * BN + col_in_slot, st, col0, [&]() {
+        if constexpr (LABELED) {
+          static_assert(C::EPI_COLS == 128, "labelled FILTER: four label bytes per lane");
+          __syncwarp();                                        // every lane is done with the previous tile's labels
+          reinterpret_cast<uint32_t*>(labs)[lane] = lab4;
+          __syncwarp();
+        }
+        epilogue_slot<MODE, C::EPI_COLS, LABELED>(p, tmem_base + lane_addr + slot * BN + col_in_slot, st, col0, [&]() {
           ptx::tc_fence_before_sync();
           __syncwarp();                                        // every lane's last TMEM load has completed
           if (lane == 0) {                                     // one arrival per warp on the LEADER's barrier
@@ -580,41 +624,41 @@ __device__ __forceinline__ void score_body(const CUtensorMap& tm_a, const CUtens
   }
 }
 
-template <int MODE>
+template <int MODE, bool LABELED>
 __global__ void __launch_bounds__(Cfg<false, 1>::THREADS, 1)
 score_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b, const Params p) {
-  score_body<MODE, false, 1, false>(tm_a, tm_b, p);
+  score_body<MODE, false, 1, false, LABELED>(tm_a, tm_b, p);
 }
 
-template <int MODE>
+template <int MODE, bool LABELED>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(Cfg<true, 1>::THREADS, 1)
 score_pair_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b, const Params p) {
-  score_body<MODE, true, 1, false>(tm_a, tm_b, p);
+  score_body<MODE, true, 1, false, LABELED>(tm_a, tm_b, p);
 }
 
-template <int MODE>
+template <int MODE, bool LABELED>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(Cfg<true, 2>::THREADS, 1)
 score_wide_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b, const Params p) {
-  score_body<MODE, true, 2, false>(tm_a, tm_b, p);
+  score_body<MODE, true, 2, false, LABELED>(tm_a, tm_b, p);
 }
 
 // the same kernels with the dynamic unit scheduler
-template <int MODE>
+template <int MODE, bool LABELED>
 __global__ void __launch_bounds__(Cfg<false, 1>::THREADS, 1)
 score_dyn_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b, const Params p) {
-  score_body<MODE, false, 1, true>(tm_a, tm_b, p);
+  score_body<MODE, false, 1, true, LABELED>(tm_a, tm_b, p);
 }
 
-template <int MODE>
+template <int MODE, bool LABELED>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(Cfg<true, 1>::THREADS, 1)
 score_pair_dyn_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b, const Params p) {
-  score_body<MODE, true, 1, true>(tm_a, tm_b, p);
+  score_body<MODE, true, 1, true, LABELED>(tm_a, tm_b, p);
 }
 
-template <int MODE>
+template <int MODE, bool LABELED>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(Cfg<true, 2>::THREADS, 1)
 score_wide_dyn_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b, const Params p) {
-  score_body<MODE, true, 2, true>(tm_a, tm_b, p);
+  score_body<MODE, true, 2, true, LABELED>(tm_a, tm_b, p);
 }
 
 // ---- host side ---------------------------------------------------------------------------------
@@ -718,10 +762,23 @@ int take_sched_counter(unsigned long long** out, cudaStream_t stream) {
   return XMVE_OK;
 }
 
-template <int MODE, bool PAIR, int NB, bool DYN = false>
+// (only the selected kernel is instantiated: there is no labelled wide kernel)
+template <int MODE, bool LABELED, bool PAIR, int NB, bool DYN>
+constexpr auto kernel_for() {
+  if constexpr (DYN && !PAIR) return score_dyn_kernel<MODE, LABELED>;
+  else if constexpr (DYN && NB == 2) return score_wide_dyn_kernel<MODE, LABELED>;
+  else if constexpr (DYN) return score_pair_dyn_kernel<MODE, LABELED>;
+  else if constexpr (!PAIR) return score_kernel<MODE, LABELED>;
+  else if constexpr (NB == 2) return score_wide_kernel<MODE, LABELED>;
+  else return score_pair_kernel<MODE, LABELED>;
+}
+
+template <int MODE, bool LABELED, bool PAIR, int NB, bool DYN = false>
 int launch_cfg(const void* a_op, int64_t nq, int64_t a_ld, const void* b_op, int64_t nv, int64_t b_ld,
                int64_t b_row_step, int k, Params p, cudaStream_t stream) {
   using C = Cfg<PAIR, NB>;
+  constexpr int smem_bytes = LABELED ? C::SMEM_BYTES_LABELED : C::SMEM_BYTES;
+  static_assert(smem_bytes <= 232448, "more dynamic shared memory than a block may have");
   CUtensorMap tm_a, tm_b;
   int s = make_operand_map(&tm_a, a_op, nq, k, a_ld, BM);
   if (s != XMVE_OK) return s;
@@ -737,21 +794,19 @@ int launch_cfg(const void* a_op, int64_t nq, int64_t a_ld, const void* b_op, int
   if (p.n_units >= (int64_t(1) << 31)) return fail(XMVE_ERR_LIMIT, "score: more than 2^31 work units");
   const int workers = static_cast<int>(p.n_units < workers_max ? p.n_units : workers_max);
   const int grid = workers * C::CTAS;
-  void (*kern)(const CUtensorMap, const CUtensorMap, const Params) =
-      DYN ? (!PAIR ? score_dyn_kernel<MODE> : (NB == 2 ? score_wide_dyn_kernel<MODE> : score_pair_dyn_kernel<MODE>))
-          : (!PAIR ? score_kernel<MODE> : (NB == 2 ? score_wide_kernel<MODE> : score_pair_kernel<MODE>));
-  static bool attr_set[MAX_DEVICES] = {};                     // per <MODE, PAIR, NB, DYN> instantiation and device
+  void (*kern)(const CUtensorMap, const CUtensorMap, const Params) = kernel_for<MODE, LABELED, PAIR, NB, DYN>();
+  static bool attr_set[MAX_DEVICES] = {};                     // per <MODE, LABELED, PAIR, NB, DYN> instantiation and device
   const int dev = current_device();
   if (dev < 0) return fail(XMVE_ERR_DEVICE, "score: no current device");
   if (!attr_set[dev]) {
-    XMVE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
+    XMVE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
     attr_set[dev] = true;
   }
   if (DYN) {
     int s2 = take_sched_counter(&p.sched_next, stream);
     if (s2 != XMVE_OK) return s2;
   }
-  kern<<<grid, C::THREADS, C::SMEM_BYTES, stream>>>(tm_a, tm_b, p);
+  kern<<<grid, C::THREADS, smem_bytes, stream>>>(tm_a, tm_b, p);
   return launch_status(!PAIR ? "score_kernel" : (NB == 2 ? "score_wide_kernel" : "score_pair_kernel"));
 }
 
@@ -763,19 +818,29 @@ int launch_cfg(const void* a_op, int64_t nq, int64_t a_ld, const void* b_op, int
 // densities.  The wide tile moves the fewest bytes but cannot overlap its epilogue: since the STORE epilogue writes
 // coalesced row segments the pair tile beats it on every STORE shape measured (sampling passes, the 59 800 x 2 990
 // evaluation), with the static assignment while both operands stay in L2.
-template <int MODE>
+// LABELED (filter only): the wide tile has no shared memory left for the label bytes (2 KB per CTA) and launch()
+// never chooses it, so XMVE_TILE=2 / 6 is refused.
+template <int MODE, bool LABELED = false>
 int launch(const void* a_op, int64_t nq, int64_t a_ld, const void* b_op, int64_t nv, int64_t b_ld, int64_t b_row_step,
            int k, Params p, cudaStream_t stream) {
   const int64_t operand_bytes = (nq + nv) * static_cast<int64_t>(k) * 2;
   int tile = (MODE == MODE_STORE && operand_bytes <= (int64_t(48) << 20)) ? 1 : 4;
   if (nq <= BM) tile = 5;   // a handful of queries (AVS, online search): HBM-bound, half of a 256-row query tile is padding
   if (const char* env = getenv("XMVE_TILE")) tile = atoi(env);
-  if (tile == 2) return launch_cfg<MODE, true, 2>(a_op, nq, a_ld, b_op, nv, b_ld, b_row_step, k, p, stream);
-  if (tile == 1) return launch_cfg<MODE, true, 1>(a_op, nq, a_ld, b_op, nv, b_ld, b_row_step, k, p, stream);
-  if (tile == 4) return launch_cfg<MODE, true, 1, true>(a_op, nq, a_ld, b_op, nv, b_ld, b_row_step, k, p, stream);
-  if (tile == 5) return launch_cfg<MODE, false, 1, true>(a_op, nq, a_ld, b_op, nv, b_ld, b_row_step, k, p, stream);
-  if (tile == 6) return launch_cfg<MODE, true, 2, true>(a_op, nq, a_ld, b_op, nv, b_ld, b_row_step, k, p, stream);
-  return launch_cfg<MODE, false, 1>(a_op, nq, a_ld, b_op, nv, b_ld, b_row_step, k, p, stream);
+  if constexpr (LABELED) {
+    if (tile == 2 || tile == 6) return fail(XMVE_ERR_ARG, "score_filter_labeled: the wide tile (XMVE_TILE=%d) has no "
+                                            "room for the labels; use 0, 1, 4 or 5", tile);
+  } else {
+    if (tile == 2) return launch_cfg<MODE, LABELED, true, 2>(a_op, nq, a_ld, b_op, nv, b_ld, b_row_step, k, p, stream);
+    if (tile == 6)
+      return launch_cfg<MODE, LABELED, true, 2, true>(a_op, nq, a_ld, b_op, nv, b_ld, b_row_step, k, p, stream);
+  }
+  if (tile == 1) return launch_cfg<MODE, LABELED, true, 1>(a_op, nq, a_ld, b_op, nv, b_ld, b_row_step, k, p, stream);
+  if (tile == 4)
+    return launch_cfg<MODE, LABELED, true, 1, true>(a_op, nq, a_ld, b_op, nv, b_ld, b_row_step, k, p, stream);
+  if (tile == 5)
+    return launch_cfg<MODE, LABELED, false, 1, true>(a_op, nq, a_ld, b_op, nv, b_ld, b_row_step, k, p, stream);
+  return launch_cfg<MODE, LABELED, false, 1>(a_op, nq, a_ld, b_op, nv, b_ld, b_row_step, k, p, stream);
 }
 
 }  // namespace
@@ -797,18 +862,12 @@ extern "C" int xmve_score_store(const void* a_op, int64_t nq, int64_t a_ld, cons
   return launch<MODE_STORE>(a_op, nq, a_ld, b_op, nv, b_ld, b_row_step, k, p, static_cast<cudaStream_t>(stream));
 }
 
-extern "C" int xmve_score_filter(const void* a_op, int64_t nq, int64_t a_ld, const void* b_op, int64_t nv,
-                                 int64_t b_ld, int64_t b_row_step, int k, const float* lo, const float* hi,
-                                 int32_t* count_above, int32_t* cand_count, float* cand_score, int32_t* cand_idx,
-                                 int32_t cap, void* stream) {
-  using namespace xmve;
-  XMVE_DEVICE_OR_RETURN();
-  int s = check_operands(a_op, nq, a_ld, b_op, nv, b_ld, b_row_step, k);
-  if (s != XMVE_OK) return s;
+namespace {
+int filter_params(xmve::Params& p, const float* lo, const float* hi, int32_t* count_above, int32_t* cand_count,
+                  float* cand_score, int32_t* cand_idx, int32_t cap) {
   XMVE_REQUIRE(lo != nullptr && cand_count != nullptr && cand_score != nullptr && cand_idx != nullptr && cap > 0,
                "score_filter: lo / candidate buffers are required and cap must be > 0");
   XMVE_REQUIRE(hi == nullptr || count_above != nullptr, "score_filter: hi given without count_above");
-  Params p{};
   p.lo = lo;
   p.hi = hi;
   p.count_above = count_above;
@@ -820,5 +879,40 @@ extern "C" int xmve_score_filter(const void* a_op, int64_t nq, int64_t a_ld, con
   if (const char* env = getenv("XMVE_DEFER")) p.defer_append = atoi(env) != 0;
   p.single_hit = 1;
   if (const char* env = getenv("XMVE_SINGLE_HIT")) p.single_hit = atoi(env) != 0;
+  return XMVE_OK;
+}
+}  // namespace
+
+extern "C" int xmve_score_filter(const void* a_op, int64_t nq, int64_t a_ld, const void* b_op, int64_t nv,
+                                 int64_t b_ld, int64_t b_row_step, int k, const float* lo, const float* hi,
+                                 int32_t* count_above, int32_t* cand_count, float* cand_score, int32_t* cand_idx,
+                                 int32_t cap, void* stream) {
+  using namespace xmve;
+  XMVE_DEVICE_OR_RETURN();
+  int s = check_operands(a_op, nq, a_ld, b_op, nv, b_ld, b_row_step, k);
+  if (s != XMVE_OK) return s;
+  Params p{};
+  s = filter_params(p, lo, hi, count_above, cand_count, cand_score, cand_idx, cap);
+  if (s != XMVE_OK) return s;
   return launch<MODE_FILTER>(a_op, nq, a_ld, b_op, nv, b_ld, b_row_step, k, p, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int xmve_score_filter_labeled(const void* a_op, int64_t nq, int64_t a_ld, const void* b_op, int64_t nv,
+                                         int64_t b_ld, int64_t b_row_step, int k, const float* lo, const float* hi,
+                                         int32_t* count_above, int32_t* cand_count, float* cand_score,
+                                         int32_t* cand_idx, int32_t cap, const uint8_t* labels,
+                                         const uint64_t* allow, void* stream) {
+  using namespace xmve;
+  XMVE_DEVICE_OR_RETURN();
+  int s = check_operands(a_op, nq, a_ld, b_op, nv, b_ld, b_row_step, k);
+  if (s != XMVE_OK) return s;
+  XMVE_REQUIRE(labels != nullptr && allow != nullptr, "score_filter_labeled: labels and allow are required");
+  Params p{};
+  s = filter_params(p, lo, hi, count_above, cand_count, cand_score, cand_idx, cap);
+  if (s != XMVE_OK) return s;
+  p.labels = labels;
+  p.allow = allow;
+  p.lab_step = b_row_step;
+  return launch<MODE_FILTER, true>(a_op, nq, a_ld, b_op, nv, b_ld, b_row_step, k, p,
+                                   static_cast<cudaStream_t>(stream));
 }

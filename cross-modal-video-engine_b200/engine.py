@@ -59,6 +59,8 @@ SAMPLE_DIV = int(os.environ.get("XMVE_SAMPLE_DIV", 128))
 SAMPLE_MIN = int(os.environ.get("XMVE_SAMPLE_MIN", 8192))
 SAMPLE_MAX = int(os.environ.get("XMVE_SAMPLE_MAX", 65536))
 _BM, _BN = 128, 256
+#: corpus row labels are 0 .. N_LABELS - 1: one byte per row, one 64-bit mask per query (filtered search)
+N_LABELS = 64
 
 
 def _round_up(x, m):
@@ -88,6 +90,56 @@ def _to_device(x, device):
         x = x.float()
     x = x.to(device, non_blocking=True)
     return x
+
+
+def _host_ints(x):
+    """ids / labels from a tensor, ndarray, sequence or scalar -> int64 CPU tensor."""
+    if torch.is_tensor(x):
+        return x.detach().to("cpu", torch.int64)
+    import numpy as np
+    return torch.from_numpy(np.asarray(x).astype(np.int64))
+
+
+def _check_labels(labels, n, device):
+    """``n`` row labels in [0, N_LABELS) -> int64 tensor on ``device``; ValueError otherwise."""
+    lab = _host_ints(labels).flatten()
+    if lab.numel() != n:
+        raise ValueError("expected %d labels, got %d" % (n, lab.numel()))
+    if lab.numel() and (int(lab.min()) < 0 or int(lab.max()) >= N_LABELS):
+        raise ValueError("labels must lie in [0, %d)" % N_LABELS)
+    return lab.to(device)
+
+
+def _label_masks(label_mask, nq, device):
+    """``search(label_mask=...)`` -> int64 device tensor ``[nq]`` holding the 64-bit masks (uint64 bit patterns)."""
+    if torch.is_tensor(label_mask):
+        m = label_mask
+        if m.dtype not in (torch.int64, torch.uint64):
+            raise ValueError("label_mask: expected an int64 or uint64 tensor, got %s" % m.dtype)
+        m = m.view(torch.int64) if m.dtype == torch.uint64 else m
+    else:
+        import numpy as np
+        a = np.asarray(label_mask)                     # a Python int of 2^63 or more comes out as uint64
+        if a.dtype == np.uint64:
+            a = a.view(np.int64)
+        elif a.dtype.kind == "i":
+            a = a.astype(np.int64)
+        else:
+            raise ValueError("label_mask: expected 64-bit integer masks, got %s" % a.dtype)
+        m = torch.from_numpy(np.ascontiguousarray(a))
+    if m.dim() == 0 or m.numel() == 1:
+        m = m.reshape(1).expand(nq)
+    if tuple(m.shape) != (nq,):
+        raise ValueError("label_mask: expected one mask per query (%d) or one for all, got shape %s"
+                         % (nq, tuple(m.shape)))
+    return m.to(device, non_blocking=True).contiguous()
+
+
+def _eligible_counts(masks, hist):
+    """``n_elig[q] = sum over the set bits l of masks[q] of hist[l]`` on the device (no host round trip)."""
+    bits = torch.bitwise_and(torch.bitwise_right_shift(masks.unsqueeze(1),
+                                                       torch.arange(N_LABELS, device=masks.device)), 1)
+    return (bits * hist.unsqueeze(0)).sum(1)
 
 
 def _prepare(src, d, raw, raw_off, norm, resid, op, op_off, layout, weight, norm_mode):
@@ -158,15 +210,24 @@ class CorpusStore:
         self.resid = torch.zeros((len(self.dims), max(self.capacity, 1)), dtype=torch.float32, device=self.device)
         self._resid_max2 = None
         self.added = None                                     # CUDA event after the last add's kernels
+        # label plane (uint8 per row, 0 <= label < N_LABELS) and the device histogram of the filled rows' labels;
+        # allocated on first use (add(..., labels) / set_labels / a filtered search)
+        self.labels = None
+        self.label_hist = None
+        self.label_version = 0                                # bumped by set_labels (GraphSearch checks it)
         self.space_off = (C.c_int32 * (len(self.dims) + 1))(*([0] + list(_cumsum(self.dims))))
 
     # -- ingest ----------------------------------------------------------------------------------
-    def add(self, rows):
-        """Append rows: tensor / ndarray ``[n, sum(dims)]`` (or ``[n, T, D]``: mean over T first), or a per-space list."""
+    def add(self, rows, labels=None):
+        """Append rows: tensor / ndarray ``[n, sum(dims)]`` (or ``[n, T, D]``: mean over T first), or a per-space list.
+        ``labels`` (``n`` integers in ``[0, 64)``, see ``search(label_mask=...)``) label the new rows; rows added
+        without labels have label 0."""
         spaces = [_to_device(s, self.device) for s in _as_spaces(rows, self.dims)]
         n = spaces[0].shape[0]
         if self.n + n > self.capacity:
             raise ValueError("CorpusStore capacity %d exceeded" % self.capacity)
+        if labels is not None:
+            labels = _check_labels(labels, n, self.device)
         op_off = raw_off = 0
         with torch.cuda.device(self.device):                  # launch on the store's device, whatever is current
             for s, (src, d, dp) in enumerate(zip(spaces, self.dims, self.dpads)):
@@ -175,11 +236,61 @@ class CorpusStore:
                          self.op[self.n:], op_off, N.OP_X1, 1.0, self.norm_mode)
                 op_off += dp
                 raw_off += d
+            if labels is not None or self.labels is not None:
+                self._ensure_labels()
+                if labels is not None:
+                    self.labels[self.n:self.n + n] = labels.to(torch.uint8)
+                    self.label_hist += torch.bincount(labels, minlength=N_LABELS)
+                else:
+                    self.labels[self.n:self.n + n] = 0
+                    self.label_hist[0] += n
             # a search's head stream (search_shards(head_stream=...)) reads the new rows: it waits for this event
             self.added = torch.cuda.Event()
             self.added.record()
         self.n += n
         return self
+
+    def set_labels(self, ids, labels):
+        """Relabel rows: ``ids`` are global row numbers (as :meth:`search` returns them), ``labels`` one integer in
+        ``[0, 64)`` per id.  The store applies the ids that fall in its rows ``[index_offset, index_offset + n)`` and
+        skips the others, which belong to other shards.  A search issued afterwards, on any stream, sees the new
+        labels.
+
+        For a corpus sharded over several stores or ranks this is a collective call: every shard is given the same
+        ``ids`` and ``labels``, even when none of them is its own.  The searches of all ranks then agree on the label
+        state, whose global histogram they all-reduce once per change."""
+        ids = torch.as_tensor(_host_ints(ids), dtype=torch.int64).flatten()
+        if ids.numel() and int(ids.min()) < 0:
+            raise IndexError("set_labels: negative row id")
+        if torch.unique(ids).numel() != ids.numel():
+            raise ValueError("set_labels: duplicate ids")
+        labels = _check_labels(labels, ids.numel(), self.device)
+        loc = ids - self.index_offset
+        mine = (loc >= 0) & (loc < self.n)
+        loc, labels = loc[mine], labels[mine.to(labels.device)]
+        with torch.cuda.device(self.device):
+            self._ensure_labels()
+            loc = loc.to(self.device)
+            self.label_hist -= torch.bincount(self.labels[loc].long(), minlength=N_LABELS)
+            self.labels[loc] = labels.to(torch.uint8)
+            self.label_hist += torch.bincount(labels, minlength=N_LABELS)
+            self.added = torch.cuda.Event()                   # head-stream searches wait for the new labels
+            self.added.record()
+        self.label_version += 1
+        return self
+
+    def _ensure_labels(self):
+        """Allocate the label plane (every row label 0) and its histogram on first use."""
+        if self.labels is None:
+            self.labels = torch.zeros((max(self.capacity, 1),), dtype=torch.uint8, device=self.device)
+            self.label_hist = torch.zeros((N_LABELS,), dtype=torch.int64, device=self.device)
+            self.label_hist[0] = self.n
+        return self.labels
+
+    def _label_counts(self):
+        """int64 [64]: how many filled rows carry each label (device)."""
+        self._ensure_labels()
+        return self.label_hist
 
     # -- query side ------------------------------------------------------------------------------
     def prepare_queries(self, queries, weights=None):
@@ -200,7 +311,8 @@ class CorpusStore:
         return a_op, q_raw, q_norm, q_res, nq
 
     # -- search ----------------------------------------------------------------------------------
-    def search(self, queries, k, weights=None, exclude=None, eps=None, small_nv=SMALL_NV, stats=None, defer=False):
+    def search(self, queries, k, weights=None, exclude=None, eps=None, small_nv=SMALL_NV, stats=None, defer=False,
+               label_mask=None):
         """Top-``k`` corpus rows per query by fused cosine score, exact (fp64) scores, descending.
 
         Returns ``(scores float64 [nq, k], idx int64 [nq, k])`` on the device; ``idx`` are global row
@@ -209,9 +321,14 @@ class CorpusStore:
         of the query's own reference item (validate.py:76-83).  ``eps`` overrides the measured bound on
         |tensor-core score - exact score| (see :func:`measured_eps`).  ``defer=True`` returns a
         :class:`PendingSearch` as soon as the work is enqueued (``.result()`` gives the tuple).
+
+        ``label_mask`` (filtered search): one 64-bit mask per query (int64 / uint64 tensor or array ``[nq]``) or one
+        for the whole batch.  Row ``v`` is eligible for query ``q`` iff bit ``label[v]`` of ``mask[q]`` is set
+        (labels: :meth:`add`, :meth:`set_labels`); the result is the exact top-``min(k, #eligible)`` of the eligible
+        rows, padded as above.  ``None`` searches every row.
         """
         return search_shards([self], queries, k, weights=weights, exclude=exclude, eps=eps, small_nv=small_nv,
-                             stats=stats, defer=defer)
+                             stats=stats, defer=defer, label_mask=label_mask)
 
     def plan(self, k, n=None):
         return plan(k, self.n if n is None else n)
@@ -226,8 +343,9 @@ class CorpusStore:
     def _weights_arr(self, wts):
         return (C.c_double * len(wts))(*[float(w) for w in wts])
 
-    def _exact_small(self, q_raw, q_norm, nq, k, wts, excl):
-        """fp64 score matrix + bitonic top-k (corpora up to ``small_nv`` rows)."""
+    def _exact_small(self, q_raw, q_norm, nq, k, wts, excl, label_mask=None):
+        """fp64 score matrix + bitonic top-k (corpora up to ``small_nv`` rows); ``label_mask``: ineligible rows are
+        set to -inf first, and the selection skips them."""
         dev, st = self.device, N.stream_ptr()
         acc = None
         o = 0
@@ -245,6 +363,9 @@ class CorpusStore:
                        N.ptr(sc[q0:]), self.n, st)
             acc = sc if acc is None else acc.add_(sc)
             o += d
+        if label_mask is not None:
+            N.call("xmve_mask_scores", N.ptr(acc), N.F64, nq, self.n, acc.stride(0), N.ptr(self._ensure_labels()), 1,
+                   N.ptr(label_mask), st)
         kk = min(k, self.n)
         out_s = torch.full((nq, k), float("-inf"), dtype=torch.float64, device=dev)
         out_i = torch.full((nq, k), -1, dtype=torch.int64, device=dev)
@@ -257,22 +378,31 @@ class CorpusStore:
         return out_s, out_i
 
     # one shard's share of a filtered pass ----------------------------------------------------------
-    def _sample(self, a_op, nq, step):
-        """K2 STORE over every ``step``-th row of this shard -> fp32 ``[nq, ceil(n / step)]``."""
+    def _sample(self, a_op, nq, step, label_mask=None):
+        """K2 STORE over every ``step``-th row of this shard -> fp32 ``[nq, ceil(n / step)]`` (``label_mask``: -inf
+        where the sampled row is not eligible)."""
         n_s = (self.n + step - 1) // step
         sample = torch.empty((nq, n_s), dtype=torch.float32, device=self.device)
         N.call("xmve_score_store", N.ptr(a_op), nq, a_op.stride(0), N.ptr(self.op), n_s, self.op.stride(0), step,
                self.k, 1.0, N.ptr(sample), sample.stride(0), N.stream_ptr())
+        if label_mask is not None:
+            N.call("xmve_mask_scores", N.ptr(sample), N.F32, nq, n_s, sample.stride(0), N.ptr(self._ensure_labels()),
+                   step, N.ptr(label_mask), N.stream_ptr())
         return sample
 
-    def _filter(self, a_op, nq, thr, cap, step=1):
+    def _filter(self, a_op, nq, thr, cap, step=1, label_mask=None):
         """K2 FILTER over the shard (or over every ``step``-th row): candidates (approximate score, local row --
-        sampled-row number when ``step > 1``) above ``thr`` per query."""
+        sampled-row number when ``step > 1``) above ``thr`` per query; ``label_mask``: eligible rows only."""
         dev = self.device
         rows = (self.n + step - 1) // step
         cand_count = torch.zeros((nq,), dtype=torch.int32, device=dev)
         cand_score = torch.empty((nq, cap), dtype=torch.float32, device=dev)
         cand_idx = torch.empty((nq, cap), dtype=torch.int32, device=dev)
+        if label_mask is not None:
+            N.call("xmve_score_filter_labeled", N.ptr(a_op), nq, a_op.stride(0), N.ptr(self.op), rows,
+                   self.op.stride(0), step, self.k, N.ptr(thr), None, None, N.ptr(cand_count), N.ptr(cand_score),
+                   N.ptr(cand_idx), cap, N.ptr(self._ensure_labels()), N.ptr(label_mask), N.stream_ptr())
+            return cand_count, cand_score, cand_idx
         N.call("xmve_score_filter", N.ptr(a_op), nq, a_op.stride(0), N.ptr(self.op), rows, self.op.stride(0), step,
                self.k, N.ptr(thr), None, None, N.ptr(cand_count), N.ptr(cand_score), N.ptr(cand_idx), cap,
                N.stream_ptr())
@@ -290,19 +420,21 @@ class CorpusStore:
                self.k, N.ptr(lo), N.ptr(hi), N.ptr(above), N.ptr(count), N.ptr(c_s), N.ptr(c_i), cap, N.stream_ptr())
         return above, count, c_s, c_i
 
-    def _sample_top(self, a_op, nq, step, big_j):
+    def _sample_top(self, a_op, nq, step, big_j, label_mask=None):
         """The largest scores of the ``step``-strided sample of this shard WITHOUT writing the sample matrix:
         a coarse STORE pass (every ``r * step``-th row, a few thousand columns) gives a per-query floor ``thr0``
         that about ``4 * big_j`` of the fine sample's scores exceed; a FILTER pass over the fine sample keeps those.
         Returns ``(scores fp32 [nq, cap_s], counts int32 [nq], thr0 fp32 [nq])``; rows whose count is below
-        ``big_j`` (the floor came out too high -- vanishingly rare) are handled by the caller through ``thr0``."""
+        ``big_j`` (the floor came out too high -- vanishingly rare) are handled by the caller through ``thr0``.
+        ``label_mask``: both passes see the eligible rows only."""
         n_s = (self.n + step - 1) // step
         r = max(2, min(16, n_s // 2048))
-        coarse = self._sample(a_op, nq, step * r)
+        kw = {} if label_mask is None else {"label_mask": label_mask}
+        coarse = self._sample(a_op, nq, step * r, **kw)
         j0 = min(coarse.shape[1], int(math.ceil(4.0 * big_j / r)))
         thr0 = _row_kth(coarse, None, j0, 0.0, 0)
         cap_s = 1 << max(10, int(math.ceil(math.log2(16 * big_j))))
-        count, score, _ = self._filter(a_op, nq, thr0, cap_s, step=step)
+        count, score, _ = self._filter(a_op, nq, thr0, cap_s, step=step, **kw)
         return score, count, thr0
 
     def _rescore(self, q_raw, q_norm, nq, wts, cand, bound, bound_hi=None, exact=None):
@@ -549,7 +681,7 @@ class _Search:
     """State of one filtered search (every rank holds the same queries, thresholds and outputs)."""
 
     def __init__(self, stores, comm, k, k_eff, kk, wts, excl, eps_t, pl, a_op, q_raw, q_norm, nq, thr, out_s, out_i,
-                 stats, ph):
+                 stats, ph, masks=None, n_elig=None):
         self.stores, self.comm, self.k, self.k_eff, self.kk, self.wts = stores, comm, k, k_eff, kk, wts
         self.excl, self.eps_t, self.pl = excl, eps_t, pl
         self.a_op, self.q_raw, self.q_norm, self.nq, self.thr = a_op, q_raw, q_norm, nq, thr
@@ -565,6 +697,13 @@ class _Search:
         self.cap = cap
         self.n_shard_max = max(s.n for s in self.live) if self.live else 1
         self.pending = None
+        # filtered search: a row with at most `cap` eligible rows in the whole corpus gets thr = -inf -- every shard's
+        # list then holds all its eligible rows, and the list is complete even when it is shorter than k
+        self.masks, self.n_elig = masks, n_elig
+        # (a row with no eligible row at all gets thr = +inf: nothing enters its window, and its answer is empty)
+        if masks is not None:
+            self.thr = torch.where(n_elig == 0, torch.full_like(thr, float("inf")),
+                                   torch.where(n_elig <= cap, torch.full_like(thr, float("-inf")), thr))
 
     # one pass over all rows (rows None) or over the rows that are re-run --------------------------------
     def run_pass(self, rows):
@@ -580,9 +719,12 @@ class _Search:
             thr_sub = self.thr[rows].contiguous()
             ex_sub = self.excl[rows].contiguous() if self.excl is not None else None
         cap = self.cap
+        kw = {}
+        if self.masks is not None:
+            kw["label_mask"] = self.masks if rows is None else self.masks[rows].contiguous()
         # 3: fused score + threshold filter on every local shard
         ph.mark("alloc")
-        cands = [s._filter(a_sub, n_sub, thr_sub, cap) for s in self.live]
+        cands = [s._filter(a_sub, n_sub, thr_sub, cap, **kw) for s in self.live]
         ph.mark("filter")
         # 4: what needs an exact score
         m = kk if self.solo else min(kk, int(math.ceil(1.5 * kk / self.n_shards)) + 10)
@@ -630,6 +772,15 @@ class _Search:
         else:
             s_, i_, cert, thr_next = (torch.cat([p[j] for p in parts]) for j in range(4))
             over = ("parts", [p[4] for p in parts])
+        if self.masks is not None:
+            # a row with thr = -inf whose lists did not overflow holds every eligible row.  When it holds fewer than k
+            # (its last entry is padding) the selection cannot certify it, yet it is exact; a row with k entries or
+            # more keeps the selection's verdict (which also covers float ties cut by the sort).  A row without any
+            # eligible row is empty.
+            n_elig = self.n_elig if rows is None else self.n_elig[rows]
+            short = (thr_sub == float("-inf")) & ~self._overflowed(over) & (i_[:, -1] == -1)
+            cert = torch.where(short | (n_elig == 0), torch.ones_like(cert), cert)
+            n_bad.copy_((cert == 0).sum().reshape(1))
         ph.mark("select_merge")
         if self.stats is not None and rows is None:
             st = self.stats
@@ -641,6 +792,9 @@ class _Search:
             st["rescored_per_query"] = sum(
                 float(((ar[None, :] < c[0][:, None]) & (e[:, :cap] > float("-inf"))).sum())
                 for c, e in zip(cands, exacts)) / max(n_sub, 1)
+            if self.masks is not None:
+                st["eligible_min"], st["eligible_max"] = int(self.n_elig.min()), int(self.n_elig.max())
+                st["thr_inf_rows"] = int((thr_sub == float("-inf")).sum())
             ph.mark("stats_bookkeeping")
         return s_, i_, cert, thr_next, over, n_bad, thr_sub
 
@@ -747,6 +901,9 @@ class _Search:
                 room = max(32768, min(1 << int(math.ceil(math.log2(self.n_shard_max))),
                                       (1 << 27) // max(int(rows.numel()), 1)))
                 self.cap = min(room, self.cap * 4)
+            if self.masks is not None:                        # rows whose eligible rows now fit the lists
+                self.thr[rows] = torch.where(self.n_elig[rows] <= self.cap,
+                                             torch.full_like(self.thr[rows], float("-inf")), self.thr[rows])
             s_, i_, cert, thr_next, over, _, thr_sub = self.run_pass(rows)
             self.out_s[rows, :self.k_eff] = s_
             self.out_i[rows, :self.k_eff] = i_
@@ -773,10 +930,14 @@ class GraphSearch:
     eager search; 0.94 -> 0.64 ms for 60 queries over two 135 k-row shards, where the ~40 launches of the eager step
     are what bounds it).  The returned tensors are the graph's static output buffers and are overwritten by the
     next call.  The graph covers the rows the stores held at capture: a call after :meth:`CorpusStore.add` raises.
+
+    ``with_label_mask=True`` captures a filtered search: ``gs(queries, label_mask=...)`` (one mask per query or one
+    for all; None = every label).  The graph also covers the labels held at capture: a call after
+    :meth:`CorpusStore.set_labels` raises.
     """
 
     def __init__(self, stores, n_queries, k, weights=None, with_exclude=False, comm=None, n_total=None,
-                 small_nv=SMALL_NV):
+                 small_nv=SMALL_NV, with_label_mask=False):
         self.stores = list(stores) if isinstance(stores, (list, tuple)) else [stores]
         ref = self.stores[0]
         self.dev = ref.device
@@ -784,6 +945,7 @@ class GraphSearch:
         self.comm = comm or SoloComm()
         self.q_in = torch.randn((self.nq, ref.dtot), dtype=torch.float32, device=self.dev)   # warm-up queries
         self.excl_in = torch.full((self.nq,), -1, dtype=torch.int64, device=self.dev) if with_exclude else None
+        self.mask_in = torch.full((self.nq,), -1, dtype=torch.int64, device=self.dev) if with_label_mask else None
         kw = dict(weights=weights, exclude=self.excl_in, eps=None, small_nv=small_nv, stats=None, comm=self.comm,
                   n_total=n_total)
         with torch.cuda.device(self.dev):
@@ -794,7 +956,7 @@ class GraphSearch:
             with torch.cuda.stream(side):
                 for _ in range(2):
                     _search_shards(self.stores, self.q_in, self.k, kw["weights"], kw["exclude"], None, small_nv, None,
-                                   self.comm, n_total).result()
+                                   self.comm, n_total, label_mask=self.mask_in).result()
             torch.cuda.current_stream().wait_stream(side)
             torch.cuda.synchronize()
             self._flag_host = torch.empty((1,), dtype=torch.int32).pin_memory()
@@ -802,11 +964,12 @@ class GraphSearch:
             with torch.cuda.graph(self.graph):
                 self._pending = _search_shards(self.stores, self.q_in, self.k, kw["weights"], kw["exclude"], None,
                                                small_nv, None, self.comm, n_total, in_graph=True,
-                                               flag_host=self._flag_host)
+                                               flag_host=self._flag_host, label_mask=self.mask_in)
         self.scores, self.idx = self._pending.scores, self._pending.idx
         self.rows = tuple(s.n for s in self.stores)           # the captured kernels cover exactly these rows
+        self.label_versions = tuple(s.label_version for s in self.stores)   # ... and, filtered, these labels
 
-    def __call__(self, queries, exclude=None, defer=False):
+    def __call__(self, queries, exclude=None, defer=False, label_mask=None):
         q = queries if torch.is_tensor(queries) else torch.as_tensor(queries)
         assert tuple(q.shape) == tuple(self.q_in.shape), "GraphSearch was captured for %s queries" % (self.q_in.shape,)
         rows = tuple(s.n for s in self.stores)
@@ -814,6 +977,9 @@ class GraphSearch:
             raise RuntimeError("GraphSearch: the corpus changed since the capture (rows per store %s, now %s); the "
                                "captured kernels would not see the new rows -- capture a new GraphSearch"
                                % (list(self.rows), list(rows)))
+        if self.mask_in is not None and tuple(s.label_version for s in self.stores) != self.label_versions:
+            raise RuntimeError("GraphSearch: set_labels ran since the capture; the captured eligible-row counts are "
+                               "stale -- capture a new GraphSearch")
         with torch.cuda.device(self.dev):
             self.q_in.copy_(q, non_blocking=True)
             if self.excl_in is not None:
@@ -821,6 +987,10 @@ class GraphSearch:
                 self.excl_in.copy_(e.to(torch.int64), non_blocking=True)
             else:
                 assert exclude is None, "capture with with_exclude=True to pass exclusions"
+            if self.mask_in is not None:
+                self.mask_in.copy_(_label_masks(-1 if label_mask is None else label_mask, self.nq, self.dev))
+            elif label_mask is not None:
+                raise ValueError("capture with with_label_mask=True to pass label masks")
             self.graph.replay()
             ctx = self._pending._ctx_template
             ctx.replayed()
@@ -843,8 +1013,21 @@ def _dv2_global(stores, comm):
     return v
 
 
+def _label_hist_global(stores, comm):
+    """Label histogram over ALL corpus rows (every shard of every rank): device int64 [64], cached per corpus and
+    label state like :func:`_dv2_global` -- the all-reduce is paid when rows or labels change, not per search."""
+    ref = stores[0]
+    key = (tuple((s.n, s.label_version) for s in stores), comm.world)
+    cached = getattr(ref, "_label_hist_cache", None)
+    if cached is not None and cached[0] == key:
+        return cached[1]
+    h = comm.sum_(torch.stack([s._label_counts() for s in stores]).sum(0))
+    ref._label_hist_cache = (key, h)
+    return h
+
+
 def search_shards(stores, queries, k, weights=None, exclude=None, eps=None, small_nv=SMALL_NV, stats=None, comm=None,
-                  n_total=None, defer=False, head_stream=None):
+                  n_total=None, defer=False, head_stream=None, label_mask=None):
     """Exact top-``k`` over a corpus cut into shards: ``stores`` are this process's shards (normally one), ``comm``
     joins the processes of a ``torch.distributed`` group (``distributed.GroupComm``; every rank calls this function
     with the same queries).  All shards work against ONE per-query threshold:
@@ -876,15 +1059,20 @@ def search_shards(stores, queries, k, weights=None, exclude=None, eps=None, smal
     been produced on ``head_stream`` (it does not wait for the current stream).  The head does wait for the last
     :meth:`CorpusStore.add` of every store it reads (an event recorded by ``add``), so a search issued straight after
     an ``add`` sees the new rows and their residuals.
+
+    ``label_mask`` restricts each query to the rows whose label its mask allows (:meth:`CorpusStore.search`).  The
+    samples and the FILTER see eligible rows only; a query with at most ``cap`` eligible rows gets thr = -inf, so its
+    lists are complete and certified however short.  ``None`` runs the unfiltered pipeline unchanged.
     """
     comm = comm or SoloComm()
     ref = stores[0]
     if ref.device.type == "cuda":
         with torch.cuda.device(ref.device):                     # kernels, streams and allocations follow the store
             pending = _search_shards(stores, queries, k, weights, exclude, eps, small_nv, stats, comm, n_total,
-                                     head_stream=head_stream)
+                                     head_stream=head_stream, label_mask=label_mask)
             return pending if defer else pending.result()
-    pending = _search_shards(stores, queries, k, weights, exclude, eps, small_nv, stats, comm, n_total)
+    pending = _search_shards(stores, queries, k, weights, exclude, eps, small_nv, stats, comm, n_total,
+                             label_mask=label_mask)
     return pending if defer else pending.result()
 
 
@@ -894,7 +1082,7 @@ def _head_on(stream):
 
 
 def _search_shards(stores, queries, k, weights, exclude, eps, small_nv, stats, comm, n_total, in_graph=False,
-                   flag_host=None, head_stream=None):
+                   flag_host=None, head_stream=None, label_mask=None):
     ref = stores[0]
     dev, n_space = ref.device, len(ref.dims)
     n_shards = len(stores) * comm.world
@@ -915,6 +1103,8 @@ def _search_shards(stores, queries, k, weights, exclude, eps, small_nv, stats, c
         for t in (queries if isinstance(queries, (list, tuple)) else (queries, exclude)):
             if torch.is_tensor(t) and t.is_cuda:
                 t.record_stream(head_stream)                  # the caller may drop it while the head still reads it
+        if torch.is_tensor(label_mask) and label_mask.is_cuda:
+            label_mask.record_stream(head_stream)
         for s in stores:                                      # the head reads the stores' rows and residuals: only
             if getattr(s, "added", None) is not None:         # their last add, not the whole current stream, must
                 head_stream.wait_event(s.added)               # be complete
@@ -923,6 +1113,10 @@ def _search_shards(stores, queries, k, weights, exclude, eps, small_nv, stats, c
         excl = None
         if exclude is not None:
             excl = torch.as_tensor(exclude, dtype=torch.int64).to(dev)
+        masks = n_elig = None
+        if label_mask is not None:
+            masks = _label_masks(label_mask, nq, dev)
+            n_elig = _eligible_counts(masks, _label_hist_global(stores, comm))
     ph.mark("prepare_queries")
     if nq == 0:
         return PendingSearch.ready(torch.empty((0, k), dtype=torch.float64, device=dev),
@@ -932,7 +1126,8 @@ def _search_shards(stores, queries, k, weights, exclude, eps, small_nv, stats, c
     out_i = torch.full((nq, k), -1, dtype=torch.int64, device=dev)
 
     if n_total <= small_nv:
-        parts = [s._exact_small(q_raw, q_norm, nq, k_eff, wts, excl) for s in stores if s.n]
+        kw = {} if masks is None else {"label_mask": masks}
+        parts = [s._exact_small(q_raw, q_norm, nq, k_eff, wts, excl, **kw) for s in stores if s.n]
         if not parts:
             parts = [(torch.full((nq, k_eff), float("-inf"), dtype=torch.float64, device=dev),
                       torch.full((nq, k_eff), -1, dtype=torch.int64, device=dev))]
@@ -947,17 +1142,17 @@ def _search_shards(stores, queries, k, weights, exclude, eps, small_nv, stats, c
     kk = k_eff + (1 if excl is not None else 0)               # one extra in case the excluded row is among them
     pl = plan(kk, n_total)
     with _head_on(head_stream):
-        eps_t, thr = _threshold(stores, comm, solo, wts, eps, pl, a_op, q_res, nq, ph)
+        eps_t, thr = _threshold(stores, comm, solo, wts, eps, pl, a_op, q_res, nq, ph, masks)
     if head_stream is not None:
         # step 3 onwards runs on the caller's stream: it waits for the head, and the caching allocator must not hand
         # the head's tensors back to the head stream while this stream still reads them
         main = torch.cuda.current_stream()
         main.wait_stream(head_stream)
-        for t in (a_op, q_raw, q_norm, q_res, eps_t, thr, excl):
+        for t in (a_op, q_raw, q_norm, q_res, eps_t, thr, excl, masks, n_elig):
             if t is not None:
                 t.record_stream(main)
     search = _Search(stores, comm, k, k_eff, kk, wts, excl, eps_t, pl, a_op, q_raw, q_norm, nq, thr, out_s, out_i,
-                     stats, ph)
+                     stats, ph, masks, n_elig)
     search.first_pass(in_graph, flag_host)
     pending = PendingSearch(search)
     pending._ctx_template = search
@@ -965,8 +1160,10 @@ def _search_shards(stores, queries, k, weights, exclude, eps, small_nv, stats, c
     return pending
 
 
-def _threshold(stores, comm, solo, wts, eps, pl, a_op, q_res, nq, ph):
-    """Steps 1b-2 of :func:`search_shards`: the error bound and the per-query threshold -> (eps_t, thr)."""
+def _threshold(stores, comm, solo, wts, eps, pl, a_op, q_res, nq, ph, masks=None):
+    """Steps 1b-2 of :func:`search_shards`: the error bound and the per-query threshold -> (eps_t, thr).  With
+    ``masks`` the samples hold eligible rows only: the strided sample keeps its meaning among them (about k / step
+    of a query's top-k eligible rows are sampled), so :func:`plan` applies unchanged."""
     ref = stores[0]
     dev, n_space = ref.device, len(ref.dims)
     w_abs = max(1.0, sum(abs(w) for w in wts))
@@ -979,15 +1176,16 @@ def _threshold(stores, comm, solo, wts, eps, pl, a_op, q_res, nq, ph):
     # 2: one global threshold from the shards' samples
     j_cap = pl["j_cap"] if solo else min(pl["j_cap"], ROW_TOPJ_MAX)      # xmve_row_topj holds 4096 values per row
     big_j = max(pl["j"], j_cap)
+    kw = {} if masks is None else {"label_mask": masks}
     lists, floor = [], torch.full((nq,), float("-inf"), dtype=torch.float32, device=dev)
     for s in live:
         if (s.n + pl["step"] - 1) // pl["step"] >= 16384:
             # two-level: the sample matrix (2.1 GB at 10 M rows) is never written or radix-selected
-            sc, cnt, thr0 = s._sample_top(a_op, nq, pl["step"], big_j)
+            sc, cnt, thr0 = s._sample_top(a_op, nq, pl["step"], big_j, **kw)
             lists.append((sc, cnt))
             floor = thr0 if len(lists) == 1 else torch.minimum(floor, thr0)
         else:                                                 # small shard: the few launches of the plain way win
-            lists.append((s._sample(a_op, nq, pl["step"]), None))
+            lists.append((s._sample(a_op, nq, pl["step"], **kw), None))
             floor = torch.full_like(floor, float("-inf"))     # a complete list needs no floor
     if solo:
         thr = _row_kth(lists[0][0], lists[0][1], pl["j"], pl["margin"], j_cap, eps_t)
@@ -1019,7 +1217,7 @@ def _threshold(stores, comm, solo, wts, eps, pl, a_op, q_res, nq, ph):
 
 
 def rank_of_gt(stores, queries, gt_off, gt_rows, weights=None, comm=None, n_total=None, cap=8192, eps=None,
-               stats=None):
+               stats=None, label_mask=None):
     """EXACT rank of every ground-truth item when the score matrix cannot exist (C3-C5 scale), sharded.
 
     ``gt_off`` int64 ``[nq + 1]`` / ``gt_rows`` int64 ``[E]`` are a CSR of global corpus rows per query (host arrays
@@ -1035,7 +1233,11 @@ def rank_of_gt(stores, queries, gt_off, gt_rows, weights=None, comm=None, n_tota
        worse.  Shards add their counts with ONE all-reduce(sum).
     3. entries whose window holds more than ``cap`` rows (ground truths ranked tens of thousands deep) fall back to
        an exact fp64 pass over the corpus (chunked ``xmve_score_f64`` + ``xmve_count_band_f64``).
+
+    Ranks are over the whole corpus: ``label_mask`` is refused (ValueError).
     """
+    if label_mask is not None:
+        raise ValueError("rank_of_gt: ranks among label-filtered rows are not supported; label_mask must be None")
     comm = comm or SoloComm()
     stores = list(stores) if isinstance(stores, (list, tuple)) else [stores]
     ref = stores[0]
@@ -1154,7 +1356,10 @@ def search_norm_score(stores, queries, k, weights=None, comm=None, n_total=None,
     weighted-cosine search with ``w_s / (max_s - min_s)``; the global extremes are exact: ``max_s`` is the largest
     top-1 score of a one-hot search of space s, ``min_s`` minus the largest top-1 score of the negated queries.
     Costs ``2 S`` extra top-1 searches.  Returns ``(fused scores fp64 [nq, k], idx)``; the errors the reference
-    would rank are ``-fused``."""
+    would rank are ``-fused``.  ``label_mask`` is refused: the normalisation spans the whole matrix, so a filtered
+    variant needs a definition of its own."""
+    if kw.get("label_mask") is not None:
+        raise ValueError("search_norm_score: label_mask is not supported (norm_score normalises over every row)")
     stores = list(stores) if isinstance(stores, (list, tuple)) else [stores]
     ref = stores[0]
     n_space = len(ref.dims)

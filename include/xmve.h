@@ -109,6 +109,28 @@ XMVE_API int xmve_score_filter(const void* a_op, int64_t nq, int64_t a_ld,
                       int32_t* count_above, int32_t* cand_count,
                       float* cand_score, int32_t* cand_idx, int32_t cap, void* stream);
 
+/* filter_labeled: xmve_score_filter restricted per query row to the corpus rows whose label it allows.  Column v
+ * (a sampled row when b_row_step > 1) has the label labels[v * b_row_step], 0 <= label < 64 (DEVICE uint8); row q
+ * may list -- and count above hi -- only columns whose label bit is set in allow[q] (DEVICE uint64 [nq]).  Every
+ * other score is skipped, so cand_count[q] and count_above[q] count eligible columns only.  The labels are read
+ * only for scores that enter the window (lo[q], ...), from a shared-memory copy of the tile's labels: the extra cost
+ * grows with the candidates, not with nv.  The wide tile (XMVE_TILE=2 / 6) has no shared memory left for the
+ * labels and returns XMVE_ERR_ARG.
+ */
+XMVE_API int xmve_score_filter_labeled(const void* a_op, int64_t nq, int64_t a_ld,
+                      const void* b_op, int64_t nv, int64_t b_ld, int64_t b_row_step, int k,
+                      const float* lo, const float* hi,
+                      int32_t* count_above, int32_t* cand_count,
+                      float* cand_score, int32_t* cand_idx, int32_t cap,
+                      const uint8_t* labels, const uint64_t* allow, void* stream);
+
+/* mask_scores: in place, scores[r * ld + c] = -inf for every column c whose label labels[c * label_step] is not set
+ * in allow[r] (DEVICE uint64 [rows]).  dtype XMVE_F32 or XMVE_F64.  Restricts a sampled STORE matrix
+ * or an fp64 score matrix to the eligible corpus rows; the selection kernels skip -inf entries.
+ */
+XMVE_API int xmve_mask_scores(void* scores, int dtype, int64_t rows, int64_t cols, int64_t ld,
+                              const uint8_t* labels, int64_t label_step, const uint64_t* allow, void* stream);
+
 /* ---- order statistics of score rows ------------------------------------------------------------
  * out[r] = max( kth_largest(row r, j1) - sub , kth_largest(row r, j2) )   (j2 <= 0: first term only)
  * Row r holds min(counts[r], cols) valid floats (counts == NULL: cols).  Fewer than j valid values
