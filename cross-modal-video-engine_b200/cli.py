@@ -2,6 +2,7 @@
 
     python -m cross_modal_video_engine_b200.cli search --corpus DIR|video_data.pt --queries Q.npy --topK 10
         [--labels L.npy --label-mask MASK|M.npy]     (only rows whose label bit is set in the query's mask)
+        [--min-score S|S.npy]                        (every row scoring at least S instead of the top K)
     python -m cross_modal_video_engine_b200.cli eval   --corpus DIR|video_data.pt --queries Q.npy --caption-ids ids.txt
     python -m cross_modal_video_engine_b200.cli composed --index index.pt --queries queries.pt [--out results_wo_attn]
 
@@ -71,6 +72,9 @@ def parse_args(argv=None):
     s.add_argument("--labels", default=None, help=".npy of one label in [0, 64) per corpus row (uint8)")
     s.add_argument("--label-mask", default=None,
                    help="search only rows whose label bit is set: one 64-bit integer, or a .npy with one per query")
+    s.add_argument("--min-score", default=None,
+                   help="range search: every row whose fused score is at least this (a float, or a .npy with one per "
+                        "query) instead of the top K; --topK is then unused")
     e = sub.choices["eval"]
     e.add_argument("--caption-ids", required=True, help="caption ids 'video7#enc#3' (util/metrics.py:111), one per query")
     e.add_argument("--save-topk", default=None, help="save {'scores','idx','video_ids'} of the top-K lists here")
@@ -89,6 +93,8 @@ def parse_args(argv=None):
         if args.labels is None:
             ap.error("--label-mask needs --labels")
         args.label_mask = np.load(args.label_mask) if args.label_mask.endswith(".npy") else int(args.label_mask, 0)
+    if args.cmd == "search" and args.min_score is not None:
+        args.min_score = np.load(args.min_score) if args.min_score.endswith(".npy") else float(args.min_score)
     return args
 
 
@@ -103,7 +109,11 @@ def main(argv=None):
         if args.labels is not None:
             labels = np.load(args.labels)
             store.set_labels(np.arange(store.n) + store.index_offset, labels)
-        scores, idx = store.search(q, args.topK, weights=args.weights, label_mask=args.label_mask)
+        if args.min_score is not None:
+            scores, idx = store.range_search(q, args.min_score, weights=args.weights,
+                                             label_mask=args.label_mask).padded()
+        else:
+            scores, idx = store.search(q, args.topK, weights=args.weights, label_mask=args.label_mask)
         if args.run_file:
             avs.write_run_file(args.run_file, _ids(args.query_ids, len(q), "q"), idx, scores, video_ids)
         else:

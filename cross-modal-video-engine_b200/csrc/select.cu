@@ -332,6 +332,30 @@ struct IdxLimits<int64_t> {
   static __device__ int64_t max() { return 0x7fffffffffffffffLL; }
 };
 
+// Bitonic sort of P (a power of two) (score, index) pairs by (score desc, index asc); all threads of the block call
+// it.  keys / ids may live in shared or global memory (__syncthreads orders both within the block).
+template <typename IdxT>
+__device__ __forceinline__ void bitonic_sort_pairs(double* keys, IdxT* ids, int P) {
+  for (int size = 2; size <= P; size <<= 1) {
+    for (int stride = size >> 1; stride > 0; stride >>= 1) {
+      for (int t = threadIdx.x; t < P; t += blockDim.x) {
+        const int o = t ^ stride;
+        if (o > t) {
+          const bool asc = (t & size) == 0;                   // "before" order towards lower indices
+          const double sa = keys[t], sb = keys[o];
+          const IdxT ia = ids[t], ib = ids[o];
+          const bool swap = asc ? before<IdxT>(sb, ib, sa, ia) : before<IdxT>(sa, ia, sb, ib);
+          if (swap) {
+            keys[t] = sb; keys[o] = sa;
+            ids[t] = ib; ids[o] = ia;
+          }
+        }
+      }
+      __syncthreads();
+    }
+  }
+}
+
 // Segmented input of the selection kernel (K3 after ONE all-gather of packed per-rank blocks): n segments, each a
 // [rows, len] block `stride` elements after the previous one; overflow flags [rows] per segment, flag_stride apart.
 struct Segments {
@@ -424,24 +448,7 @@ select_topk_kernel(const double* __restrict__ score, const IdxT* __restrict__ id
     ids[i] = IdxLimits<IdxT>::max();
   }
   __syncthreads();
-  for (int size = 2; size <= P; size <<= 1) {
-    for (int stride = size >> 1; stride > 0; stride >>= 1) {
-      for (int t = threadIdx.x; t < P; t += blockDim.x) {
-        const int o = t ^ stride;
-        if (o > t) {
-          const bool asc = (t & size) == 0;                   // "before" order towards lower indices
-          const double sa = keys[t], sb = keys[o];
-          const IdxT ia = ids[t], ib = ids[o];
-          const bool swap = asc ? before<IdxT>(sb, ib, sa, ia) : before<IdxT>(sa, ia, sb, ib);
-          if (swap) {
-            keys[t] = sb; keys[o] = sa;
-            ids[t] = ib; ids[o] = ia;
-          }
-        }
-      }
-      __syncthreads();
-    }
-  }
+  bitonic_sort_pairs<IdxT>(keys, ids, P);
   for (int i = threadIdx.x; i < k; i += blockDim.x) {
     const bool ok = i < n;
     out_score[r * k + i] = ok ? keys[i] : -CUDART_INF;
@@ -477,6 +484,135 @@ int pow2_ceil(int64_t x) {
   int p = 1;
   while (p < x) p <<= 1;
   return p;
+}
+
+// ---- range search: every rescored candidate whose exact score reaches a per-row minimum ---------------------------
+// Entry c < min(counts[r], cap) of row r matches iff exact > -inf, exact >= min_score[r] (NaN never does) and its
+// global row idx + idx_offset is not exclude[r].  Counting and filling apply the same test, so the fill finds exactly
+// the number of entries the count gave.
+constexpr int RANGE_SMEM_MAX = 16384;                       // entries sorted in shared memory (12 B each)
+
+__device__ __forceinline__ bool range_hit(double s, int64_t row, double lo, int64_t excl) {
+  return s > -CUDART_INF && s >= lo && row != excl;
+}
+
+__global__ void __launch_bounds__(256)
+range_count_kernel(const double* __restrict__ exact, const int32_t* __restrict__ idx, const int32_t* __restrict__ counts,
+                   int cap, int64_t idx_offset, const int64_t* __restrict__ exclude, const double* __restrict__ min_score,
+                   int64_t* __restrict__ out) {
+  __shared__ int part[8];
+  const int64_t r = blockIdx.x;
+  const int n = min(counts[r], cap);
+  const double lo = min_score[r];
+  const int64_t excl = exclude ? exclude[r] : -1;
+  int mine = 0;
+  for (int i = threadIdx.x; i < n; i += blockDim.x)
+    mine += range_hit(exact[r * cap + i], static_cast<int64_t>(idx[r * cap + i]) + idx_offset, lo, excl) ? 1 : 0;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) mine += __shfl_xor_sync(0xffffffffu, mine, o);
+  if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = mine;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    int64_t t = 0;
+    for (int w = 0; w < static_cast<int>(blockDim.x >> 5); ++w) t += part[w];
+    out[r] = t;
+  }
+}
+
+// Row r's m = len[r] matches are compacted, sorted by (score desc, row asc) with bitonic_sort_pairs and written to
+// [off[r], off[r] + m).  Rows of up to smem_cap entries sort in shared memory; longer rows in the caller's scratch, row
+// r at byte 24 * off[r]: 2m fp64 keys then 2m int32 rows (room for the power-of-two padding, P < 2m).
+__global__ void __launch_bounds__(1024)
+range_fill_kernel(const double* __restrict__ exact, const int32_t* __restrict__ idx, const int32_t* __restrict__ counts,
+                  int cap, int64_t idx_offset, const int64_t* __restrict__ exclude, const double* __restrict__ min_score,
+                  const int64_t* __restrict__ off, const int64_t* __restrict__ len, int smem_cap, uint8_t* scratch,
+                  double* __restrict__ out_score, int64_t* __restrict__ out_idx) {
+  extern __shared__ __align__(16) uint8_t range_smem[];
+  __shared__ int n_s;
+  const int64_t r = blockIdx.x;
+  const int64_t m = len[r];
+  if (m == 0) return;
+  const int64_t o = off[r];
+  double* keys;
+  int32_t* ids;
+  if (m <= smem_cap) {
+    keys = reinterpret_cast<double*>(range_smem);
+    ids = reinterpret_cast<int32_t*>(keys + smem_cap);
+  } else {
+    keys = reinterpret_cast<double*>(scratch + 24 * o);
+    ids = reinterpret_cast<int32_t*>(scratch + 24 * o + 16 * m);
+  }
+  const int n = min(counts[r], cap);
+  const double lo = min_score[r];
+  const int64_t excl = exclude ? exclude[r] : -1;
+  if (threadIdx.x == 0) n_s = 0;
+  __syncthreads();
+  for (int base = threadIdx.x & ~31; base < n; base += blockDim.x) {          // warp-aggregated compaction
+    const int i = base + (threadIdx.x & 31);
+    const double s = i < n ? exact[r * cap + i] : -CUDART_INF;
+    const int32_t v = i < n ? idx[r * cap + i] : 0;
+    const bool keep = i < n && range_hit(s, static_cast<int64_t>(v) + idx_offset, lo, excl);
+    const unsigned mk = __ballot_sync(0xffffffffu, keep);
+    if (mk != 0) {
+      int pos = 0;
+      if ((threadIdx.x & 31) == 0) pos = atomicAdd(&n_s, __popc(mk));
+      pos = __shfl_sync(0xffffffffu, pos, 0) + __popc(mk & ((1u << (threadIdx.x & 31)) - 1u));
+      if (keep && pos < m) { keys[pos] = s; ids[pos] = v; }
+    }
+  }
+  __syncthreads();
+  const int got = static_cast<int>(min(static_cast<int64_t>(n_s), m));
+  int P = 1;
+  while (P < got) P <<= 1;
+  for (int i = got + threadIdx.x; i < P; i += blockDim.x) {
+    keys[i] = -CUDART_INF;
+    ids[i] = IdxLimits<int32_t>::max();
+  }
+  __syncthreads();
+  bitonic_sort_pairs<int32_t>(keys, ids, P);
+  for (int i = threadIdx.x; i < m; i += blockDim.x) {
+    const bool ok = i < got;
+    out_score[o + i] = ok ? keys[i] : -CUDART_INF;
+    out_idx[o + i] = ok ? static_cast<int64_t>(ids[i]) + idx_offset : -1;
+  }
+}
+
+// Merge of n_seg sorted runs per row: an entry's output position is its position in its own run plus, for every other
+// run, the number of entries there that precede it (binary search) -- no sort, no scratch, any run length.
+__global__ void __launch_bounds__(256)
+range_merge_kernel(const double* __restrict__ score, const int64_t* __restrict__ idx, int n_seg,
+                   const int64_t* __restrict__ seg_off, int64_t rows, const int64_t* __restrict__ off,
+                   double* __restrict__ out_score, int64_t* __restrict__ out_idx) {
+  const int64_t r = blockIdx.x;
+  const int64_t o = off[r], total = off[r + 1] - o;
+  for (int64_t j = static_cast<int64_t>(blockIdx.y) * blockDim.x + threadIdx.x; j < total;
+       j += static_cast<int64_t>(gridDim.y) * blockDim.x) {
+    int s = 0;
+    int64_t i = j;
+    for (; s < n_seg; ++s) {
+      const int64_t len = seg_off[s * (rows + 1) + r + 1] - seg_off[s * (rows + 1) + r];
+      if (i < len) break;
+      i -= len;
+    }
+    if (s == n_seg) break;                                   // the runs hold fewer entries than off says
+    const int64_t p = seg_off[s * (rows + 1) + r] + i;
+    const double x = score[p];
+    const int64_t v = idx[p];
+    int64_t pos = i;
+    for (int h = 0; h < n_seg; ++h) {
+      if (h == s) continue;
+      const int64_t b = seg_off[h * (rows + 1) + r];
+      int64_t lo = b, hi = seg_off[h * (rows + 1) + r + 1];
+      while (lo < hi) {
+        const int64_t mid = lo + (hi - lo) / 2;
+        if (before<int64_t>(score[mid], idx[mid], x, v)) lo = mid + 1;
+        else hi = mid;
+      }
+      pos += lo - b;
+    }
+    out_score[o + pos] = x;
+    out_idx[o + pos] = v;
+  }
 }
 
 // ---- two-round rescore: the pilot ------------------------------------------------------------------
@@ -712,6 +848,56 @@ extern "C" int xmve_merge_topk_packed(const void* packed, int32_t n_seg, int64_t
 extern "C" int64_t xmve_packed_topk_bytes(int64_t rows, int32_t len) {
   const int64_t b = rows * len * 16 + rows * 4;
   return (b + 15) / 16 * 16;
+}
+
+extern "C" int xmve_range_select(const double* exact, const int32_t* cand_idx, const int32_t* cand_count, int64_t rows,
+                                 int32_t cap, int64_t idx_offset, const int64_t* exclude, const double* min_score,
+                                 int64_t* counts, const int64_t* off, int64_t max_len, void* scratch,
+                                 double* out_score, int64_t* out_idx, void* stream) {
+  using namespace xmve;
+  XMVE_DEVICE_OR_RETURN();
+  XMVE_REQUIRE(exact && cand_idx && cand_count && min_score && counts && rows >= 0 && cap > 0,
+               "range_select: bad arguments");
+  if (rows == 0) return XMVE_OK;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (off == nullptr) {
+    range_count_kernel<<<static_cast<unsigned>(rows), 256, 0, st>>>(exact, cand_idx, cand_count, cap, idx_offset,
+                                                                      exclude, min_score, counts);
+    return launch_status("range_count_kernel");
+  }
+  XMVE_REQUIRE(out_score && out_idx && max_len >= 0 && max_len <= cap, "range_select: fill needs outputs, 0 <= max_len <= cap");
+  if (max_len > RANGE_SMEM_MAX && scratch == nullptr)
+    return fail(XMVE_ERR_LIMIT, "range_select: a row has %lld entries (> %d): pass scratch (24 bytes per output entry)",
+                static_cast<long long>(max_len), RANGE_SMEM_MAX);
+  const int smem_cap = pow2_ceil(max_len < 1 ? 1 : (max_len > RANGE_SMEM_MAX ? RANGE_SMEM_MAX : max_len));
+  const int smem_bytes = smem_cap * static_cast<int>(sizeof(double) + sizeof(int32_t));
+  static int attr_bytes[MAX_DEVICES] = {};
+  const int dev = current_device();
+  if (dev < 0) return fail(XMVE_ERR_DEVICE, "range_select: no current device");
+  if (smem_bytes > attr_bytes[dev]) {
+    XMVE_CUDA(cudaFuncSetAttribute(range_fill_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
+    attr_bytes[dev] = smem_bytes;
+  }
+  range_fill_kernel<<<static_cast<unsigned>(rows), max_len > 2048 ? 1024 : 256, smem_bytes, st>>>(
+      exact, cand_idx, cand_count, cap, idx_offset, exclude, min_score, off, counts, smem_cap,
+      static_cast<uint8_t*>(scratch), out_score, out_idx);
+  return launch_status("range_fill_kernel");
+}
+
+extern "C" int xmve_range_merge(const double* score, const int64_t* idx, int32_t n_seg, const int64_t* seg_off,
+                                int64_t rows, const int64_t* off, int64_t max_len, double* out_score, int64_t* out_idx,
+                                void* stream) {
+  using namespace xmve;
+  XMVE_DEVICE_OR_RETURN();
+  XMVE_REQUIRE(seg_off && off && out_score && out_idx && n_seg >= 1 && rows >= 0 && max_len >= 0,
+               "range_merge: bad arguments");
+  if (rows == 0 || max_len == 0) return XMVE_OK;
+  XMVE_REQUIRE(score && idx, "range_merge: bad arguments");
+  int64_t gy = (max_len + 4095) / 4096;
+  if (gy > 65535) gy = 65535;
+  range_merge_kernel<<<dim3(static_cast<unsigned>(rows), static_cast<unsigned>(gy)), 256, 0,
+                       static_cast<cudaStream_t>(stream)>>>(score, idx, n_seg, seg_off, rows, off, out_score, out_idx);
+  return launch_status("range_merge_kernel");
 }
 
 extern "C" int xmve_row_topj(const float* vals, int64_t rows, int64_t cols, int64_t ld, const int32_t* counts,

@@ -107,3 +107,22 @@ def sharded_search(store, queries, k, group=None, n_total=None, **kw):
     if not dist.is_initialized() or dist.get_world_size(group) == 1:
         return search_shards(stores, queries, k, **kw)
     return search_shards(stores, queries, k, comm=GroupComm(group), n_total=n_total, **kw)
+
+
+def sharded_range_search(store, queries, min_score, group=None, **kw):
+    """Range search (``engine.range_search_shards``) over the corpus whose rows are sharded over the ranks of
+    ``group``; every rank passes the same queries and gets the same global ``RangeResult``."""
+    from .engine import range_search_shards
+    stores = list(store) if isinstance(store, (list, tuple)) else [store]
+    if not dist.is_initialized() or dist.get_world_size(group) == 1:
+        return range_search_shards(stores, queries, min_score, **kw)
+    return range_search_shards(stores, queries, min_score, comm=GroupComm(group), **kw)
+
+
+def sharded_range_count(store, queries, min_score, group=None, **kw):
+    """``engine.range_count_shards`` over the ranks of ``group``: the global length of every range-search list."""
+    from .engine import range_count_shards
+    stores = list(store) if isinstance(store, (list, tuple)) else [store]
+    if not dist.is_initialized() or dist.get_world_size(group) == 1:
+        return range_count_shards(stores, queries, min_score, **kw)
+    return range_count_shards(stores, queries, min_score, comm=GroupComm(group), **kw)

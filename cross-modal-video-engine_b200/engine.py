@@ -330,6 +330,21 @@ class CorpusStore:
         return search_shards([self], queries, k, weights=weights, exclude=exclude, eps=eps, small_nv=small_nv,
                              stats=stats, defer=defer, label_mask=label_mask)
 
+    def range_search(self, queries, min_score, weights=None, exclude=None, label_mask=None, eps=None, stats=None):
+        """Every corpus row whose exact fused score reaches ``min_score`` (a float, or one per query), per query,
+        sorted by (score desc, global row asc) -> :class:`RangeResult`.  Scores are the fp64 scores :meth:`search`
+        returns; the lists are complete.  ``+inf`` gives an empty list, ``-inf`` every eligible row.  ``exclude`` and
+        ``label_mask`` as in :meth:`search`.  A result too large for the free device memory raises a sized
+        ``MemoryError`` before it is allocated (:meth:`range_count` counts without listing)."""
+        return range_search_shards([self], queries, min_score, weights=weights, exclude=exclude,
+                                   label_mask=label_mask, eps=eps, stats=stats)
+
+    def range_count(self, queries, min_score, weights=None, exclude=None, label_mask=None, eps=None):
+        """int64 ``[nq]`` on the device: the length of each :meth:`range_search` list for the same arguments, without
+        listing the rows -- only the rows within the error bound of ``min_score`` are listed and rescored."""
+        return range_count_shards([self], queries, min_score, weights=weights, exclude=exclude,
+                                  label_mask=label_mask, eps=eps)
+
     def plan(self, k, n=None):
         return plan(k, self.n if n is None else n)
 
@@ -408,14 +423,20 @@ class CorpusStore:
                N.stream_ptr())
         return cand_count, cand_score, cand_idx
 
-    def _filter_band(self, a_op, nq, lo, hi, cap):
+    def _filter_band(self, a_op, nq, lo, hi, cap, label_mask=None):
         """K2 FILTER with a two-sided window per row: rows scoring above ``hi`` are counted, rows in ``(lo, hi]``
-        are listed -> (above int32 [nq], count int32 [nq], scores fp32 [nq, cap], local rows int32 [nq, cap])."""
+        are listed -> (above int32 [nq], count int32 [nq], scores fp32 [nq, cap], local rows int32 [nq, cap]).
+        ``label_mask``: eligible rows only, counted and listed."""
         dev = self.device
         above = torch.zeros((nq,), dtype=torch.int32, device=dev)
         count = torch.zeros((nq,), dtype=torch.int32, device=dev)
         c_s = torch.empty((nq, cap), dtype=torch.float32, device=dev)
         c_i = torch.empty((nq, cap), dtype=torch.int32, device=dev)
+        if label_mask is not None:
+            N.call("xmve_score_filter_labeled", N.ptr(a_op), nq, a_op.stride(0), N.ptr(self.op), self.n,
+                   self.op.stride(0), 1, self.k, N.ptr(lo), N.ptr(hi), N.ptr(above), N.ptr(count), N.ptr(c_s),
+                   N.ptr(c_i), cap, N.ptr(self._ensure_labels()), N.ptr(label_mask), N.stream_ptr())
+            return above, count, c_s, c_i
         N.call("xmve_score_filter", N.ptr(a_op), nq, a_op.stride(0), N.ptr(self.op), self.n, self.op.stride(0), 1,
                self.k, N.ptr(lo), N.ptr(hi), N.ptr(above), N.ptr(count), N.ptr(c_s), N.ptr(c_i), cap, N.stream_ptr())
         return above, count, c_s, c_i
@@ -999,6 +1020,15 @@ class GraphSearch:
         return p if defer else p.result()
 
 
+def _eps_for(stores, comm, wts, eps, q_res):
+    """The error bound as a device fp32 ``[1]``: measured (:func:`_eps_device`), or the caller's ``eps`` per unit of
+    fusion weight."""
+    ref = stores[0]
+    if eps is None:
+        return _eps_device(q_res, _dv2_global(stores, comm), wts, len(ref.dims), ref.k)
+    return torch.full((1,), float(eps) * max(1.0, sum(abs(w) for w in wts)), dtype=torch.float32, device=ref.device)
+
+
 def _dv2_global(stores, comm):
     """max over ALL corpus rows (every shard of every rank) of the squared bf16 residual: device fp32 [1], cached per
     corpus state -- the one all-reduce it needs is paid when the corpus changes, not per search."""
@@ -1164,13 +1194,8 @@ def _threshold(stores, comm, solo, wts, eps, pl, a_op, q_res, nq, ph, masks=None
     """Steps 1b-2 of :func:`search_shards`: the error bound and the per-query threshold -> (eps_t, thr).  With
     ``masks`` the samples hold eligible rows only: the strided sample keeps its meaning among them (about k / step
     of a query's top-k eligible rows are sampled), so :func:`plan` applies unchanged."""
-    ref = stores[0]
-    dev, n_space = ref.device, len(ref.dims)
-    w_abs = max(1.0, sum(abs(w) for w in wts))
-    if eps is None:
-        eps_t = _eps_device(q_res, _dv2_global(stores, comm), wts, n_space, ref.k)
-    else:
-        eps_t = torch.full((1,), float(eps) * w_abs, dtype=torch.float32, device=dev)
+    dev = stores[0].device
+    eps_t = _eps_for(stores, comm, wts, eps, q_res)
     ph.mark("eps")
     live = [s for s in stores if s.n]
     # 2: one global threshold from the shards' samples
@@ -1255,10 +1280,7 @@ def rank_of_gt(stores, queries, gt_off, gt_rows, weights=None, comm=None, n_tota
         if n_ent == 0:
             return torch.zeros((0,), dtype=torch.int32, device=dev)
         owner = torch.repeat_interleave(torch.arange(nq), off[1:] - off[:-1]).to(dev)        # entry -> query row
-        if eps is None:
-            eps_t = _eps_device(q_res, _dv2_global(stores, comm), wts, n_space, ref.k)
-        else:
-            eps_t = torch.full((1,), float(eps) * max(1.0, sum(abs(w) for w in wts)), dtype=torch.float32, device=dev)
+        eps_t = _eps_for(stores, comm, wts, eps, q_res)
         # one operand / raw row per entry
         a_ent = torch.zeros((_round_up(n_ent, _BM), ref.k), dtype=torch.bfloat16, device=dev)
         a_ent[:n_ent] = a_op[owner]
@@ -1266,45 +1288,69 @@ def rank_of_gt(stores, queries, gt_off, gt_rows, weights=None, comm=None, n_tota
         qn_ent = q_norm[:, owner].contiguous()
         live = [s for s in stores if s.n]
         # 1: exact score of every ground-truth item, from the shard that owns it
-        s_gt = torch.full((n_ent,), float("-inf"), dtype=torch.float64, device=dev)
-        for s in live:
-            mine = (g >= s.index_offset) & (g < s.index_offset + s.n)
-            loc = torch.where(mine, g - s.index_offset, torch.zeros_like(g)).to(torch.int32).unsqueeze(1).contiguous()
-            cnt = mine.to(torch.int32)
-            ex = s._rescore(q_ent, qn_ent, n_ent, wts, (cnt, torch.zeros((n_ent, 1), device=dev), loc), None)
-            s_gt = torch.where(mine, ex[:, 0], s_gt)
-        s_gt = comm.max_(s_gt)
+        s_gt = comm.max_(_row_scores(live, q_ent, qn_ent, n_ent, wts, g))
         if bool((s_gt == float("-inf")).any()):
             raise IndexError("rank_of_gt: a ground-truth row is outside the corpus (or its score is not finite)")
-        # 2: window around s(g), widened by the float roundings of its ends
-        e64 = eps_t.double()
-        lo = (s_gt - 1.001 * e64 - 1e-7).float()
-        hi = (s_gt + 1.001 * e64 + 1e-7).float()
-        tally = torch.zeros((2, n_ent), dtype=torch.int64, device=dev)                        # [before, overflowed]
-        for s in live:
-            above, count, c_s, c_i = s._filter_band(a_ent, n_ent, lo, hi, cap)
-            ex = s._rescore(q_ent, qn_ent, n_ent, wts, (count, c_s, c_i), None)
-            tally[0] += above
-            _count_before(ex, c_i, count, s.index_offset, s_gt, g, tally[0])
-            tally[1] += (count > cap)
-            del ex, c_s, c_i
-        tally = comm.sum_(tally)
-        deep = torch.nonzero(tally[1] != 0).flatten()                                         # host sync
+        # 2-3: rows before g
+        before, n_deep = _count_before_all(live, comm, a_ent, q_ent, qn_ent, n_ent, wts, s_gt, g, eps_t, cap)
         if stats is not None:
             stats["eps"] = float(eps_t)
-            stats["deep_entries"] = int(deep.numel())
-        # 3: exact fp64 pass for the entries whose window overflowed
-        if deep.numel():
-            fix = _rank_deep(live, q_ent[deep].contiguous(), qn_ent[:, deep].contiguous(), s_gt[deep].contiguous(),
-                             g[deep].contiguous(), wts)
-            tally[0, deep] = comm.sum_(fix)
-        return (tally[0] + 1).to(torch.int32)
+            stats["deep_entries"] = n_deep
+        return (before + 1).to(torch.int32)
 
 
-def _rank_deep(live, q_ent, qn_ent, s_gt, g, wts, chunk=1 << 17, band_cap=64, delta=1e-13):
+def _row_scores(live, q_ent, qn_ent, n_ent, wts, g, masks=None):
+    """Exact fp64 score of global row ``g[e]`` for entry ``e``, from the local shard that owns it; -inf where no local
+    shard owns ``g[e]`` (or, with ``masks``, where its label is not allowed).  The caller all-reduces (max) over
+    ranks."""
+    dev = q_ent.device
+    s_gt = torch.full((n_ent,), float("-inf"), dtype=torch.float64, device=dev)
+    for s in live:
+        mine = (g >= s.index_offset) & (g < s.index_offset + s.n)
+        loc = torch.where(mine, g - s.index_offset, torch.zeros_like(g)).to(torch.int32).unsqueeze(1).contiguous()
+        cnt = mine.to(torch.int32)
+        ex = s._rescore(q_ent, qn_ent, n_ent, wts, (cnt, torch.zeros((n_ent, 1), device=dev), loc), None)
+        if masks is not None:
+            lab = s._ensure_labels()[loc[:, 0].long()].long()
+            mine = mine & (torch.bitwise_and(torch.bitwise_right_shift(masks, lab), 1) != 0)
+        s_gt = torch.where(mine, ex[:, 0], s_gt)
+    return s_gt
+
+
+def _count_before_all(live, comm, a_ent, q_ent, qn_ent, n_ent, wts, s_gt, g, eps_t, cap, masks=None):
+    """Steps 2-3 of :func:`rank_of_gt`: int64 ``[n_ent]`` = #{corpus rows v of every shard of every rank (eligible
+    under ``masks``) : s(v) > s_gt[e], or s(v) == s_gt[e] and v < g[e]} -> (counts, entries settled by the fp64
+    fallback).  With ``g = INT64_MAX`` that is #{v : s(v) >= s_gt[e]}."""
+    dev = q_ent.device
+    # 2: window around s(g), widened by the float roundings of its ends
+    e64 = eps_t.double()
+    lo = (s_gt - 1.001 * e64 - 1e-7).float()
+    hi = (s_gt + 1.001 * e64 + 1e-7).float()
+    kw = {} if masks is None else {"label_mask": masks}
+    tally = torch.zeros((2, n_ent), dtype=torch.int64, device=dev)                            # [before, overflowed]
+    for s in live:
+        above, count, c_s, c_i = s._filter_band(a_ent, n_ent, lo, hi, cap, **kw)
+        ex = s._rescore(q_ent, qn_ent, n_ent, wts, (count, c_s, c_i), None)
+        tally[0] += above
+        _count_before(ex, c_i, count, s.index_offset, s_gt, g, tally[0])
+        tally[1] += (count > cap)
+        del ex, c_s, c_i
+    tally = comm.sum_(tally)
+    deep = torch.nonzero(tally[1] != 0).flatten()                                             # host sync
+    # 3: exact fp64 pass for the entries whose window overflowed
+    if deep.numel():
+        kw = {} if masks is None else {"masks": masks[deep].contiguous()}
+        fix = _rank_deep(live, q_ent[deep].contiguous(), qn_ent[:, deep].contiguous(), s_gt[deep].contiguous(),
+                         g[deep].contiguous(), wts, **kw)
+        tally[0, deep] = comm.sum_(fix)
+    return tally[0], int(deep.numel())
+
+
+def _rank_deep(live, q_ent, qn_ent, s_gt, g, wts, chunk=1 << 17, band_cap=64, delta=1e-13, masks=None):
     """#{rows before the ground truth} over this rank's shards from an exact fp64 score matrix, chunk by chunk.
     Scores more than ``delta`` above ``s_gt`` are counted; the handful within ``delta`` (the fp64 matrix and the
-    rescore kernel sum in different orders, ~1e-15 apart) are settled by the rescore kernel itself."""
+    rescore kernel sum in different orders, ~1e-15 apart) are settled by the rescore kernel itself.  ``masks``
+    (int64 ``[n_ent]``): ineligible rows are set to -inf first."""
     dev = q_ent.device
     n_ent = q_ent.shape[0]
     before = torch.zeros((n_ent,), dtype=torch.int64, device=dev)
@@ -1333,18 +1379,374 @@ def _rank_deep(live, q_ent, qn_ent, s_gt, g, wts, chunk=1 << 17, band_cap=64, de
                            N.ptr(sc), r1 - r0, st)
                     acc = sc if acc is None else acc.add_(sc)
                     o += d
-                bcount = torch.zeros((ne,), dtype=torch.int32, device=dev)
-                bidx = torch.zeros((ne, band_cap), dtype=torch.int32, device=dev)
-                N.call("xmve_count_band_f64", N.ptr(acc), ne, r1 - r0, r1 - r0, r0, N.ptr(s_gt[e0:]), float(delta),
-                       N.ptr(before[e0:]), N.ptr(bcount), N.ptr(bidx), band_cap, st)
-                if bool((bcount > band_cap).any()):
-                    raise N.XmveError("rank_of_gt: more than %d corpus rows tie with a ground truth to 1e-13" % band_cap)
+                if masks is not None:
+                    N.call("xmve_mask_scores", N.ptr(acc), N.F64, ne, r1 - r0, acc.stride(0),
+                           N.ptr(s._ensure_labels()[r0:]), 1, N.ptr(masks[e0:e1]), st)
+                # band_count keeps counting past the capacity: a band that did not fit (many rows tied to 1e-13, e.g.
+                # exact duplicates) is listed again with room for all of it
+                cap_b, above = band_cap, torch.zeros((ne,), dtype=torch.int64, device=dev)
+                while True:
+                    bcount = torch.zeros((ne,), dtype=torch.int32, device=dev)
+                    bidx = torch.zeros((ne, cap_b), dtype=torch.int32, device=dev)
+                    N.call("xmve_count_band_f64", N.ptr(acc), ne, r1 - r0, r1 - r0, r0, N.ptr(s_gt[e0:]),
+                           float(delta), N.ptr(above), N.ptr(bcount), N.ptr(bidx), cap_b, st)
+                    longest = int(bcount.max())
+                    if longest <= cap_b:
+                        break
+                    cap_b = _pow2(longest)
+                    above.zero_()
+                before[e0:e1] += above
                 bidx += r0                                                                    # shard-local rows
                 ex = s._rescore(q_ent[e0:e1], qn_ent[:, e0:e1].contiguous(), ne, wts,
-                                (bcount, torch.zeros((ne, band_cap), device=dev), bidx), None)
+                                (bcount, torch.zeros((ne, cap_b), device=dev), bidx), None)
                 _count_before(ex, bidx, bcount, s.index_offset, s_gt[e0:e1], g[e0:e1], before[e0:e1])
                 del acc, ex
     return before
+
+
+#: range search: candidate lists of the first FILTER pass; longer lists are sized from the exact counts and re-run
+RANGE_CAP0 = 2048
+#: ... in passes of at most this many list entries (rows x cap), as the top-k re-run bounds its lists
+RANGE_PASS_ENTRIES = 1 << 27
+#: ... and at most this many re-run passes (the counts are exact, so one suffices unless the FILTER disagrees with
+#: itself)
+RANGE_PASSES = 4
+#: xmve_range_select sorts rows of up to this many matches in shared memory, longer ones in a scratch buffer
+RANGE_SMEM_MAX = 16384
+
+
+class RangeResult:
+    """The lists of a range search as a CSR on the device: query ``q``'s rows are ``idx[offsets[q]:offsets[q + 1]]``
+    (int64 global rows) with their exact scores ``scores[...]`` (fp64), sorted by (score desc, row asc).
+    ``offsets`` is int64 ``[nq + 1]``."""
+
+    def __init__(self, offsets, scores, idx):
+        self.offsets, self.scores, self.idx = offsets, scores, idx
+
+    def padded(self):
+        """``(scores fp64 [nq, max_count], idx int64 [nq, max_count])``, padded with -inf / -1: the layout of
+        :meth:`CorpusStore.search` (``avs.write_run_file``, the CLI)."""
+        nq = self.offsets.numel() - 1
+        lens = self.offsets[1:] - self.offsets[:-1]
+        width = int(lens.max()) if nq else 0
+        dev = self.offsets.device
+        out_s = torch.full((nq, width), float("-inf"), dtype=torch.float64, device=dev)
+        out_i = torch.full((nq, width), -1, dtype=torch.int64, device=dev)
+        if self.idx.numel():
+            row = torch.repeat_interleave(torch.arange(nq, device=dev), lens)
+            col = torch.arange(self.idx.numel(), device=dev) - self.offsets[row]
+            out_s[row, col] = self.scores
+            out_i[row, col] = self.idx
+        return out_s, out_i
+
+
+def _min_scores(min_score, nq, device):
+    """``min_score`` (a float or one per query) -> fp64 device tensor ``[nq]``; ValueError on NaN or a wrong shape."""
+    if torch.is_tensor(min_score):
+        m = min_score.detach().to("cpu", torch.float64)
+    else:
+        import numpy as np
+        m = torch.from_numpy(np.array(min_score, dtype=np.float64))
+    if m.dim() == 0 or m.numel() == 1:
+        m = m.reshape(1).expand(nq)
+    if tuple(m.shape) != (nq,):
+        raise ValueError("min_score: expected one value per query (%d) or one for all, got shape %s"
+                         % (nq, tuple(m.shape)))
+    if bool(torch.isnan(m).any()):
+        raise ValueError("min_score: NaN")
+    return m.contiguous().to(device)
+
+
+def _range_setup(stores, queries, min_score, weights, exclude, label_mask, eps, comm):
+    """K1 on the queries, the per-query minimum, exclusions, label masks and the error bound of a range call."""
+    ref = stores[0]
+    dev = ref.device
+    wts = _weights(weights, len(ref.dims))
+    a_op, q_raw, q_norm, q_res, nq = ref.prepare_queries(queries, wts)
+    ms = _min_scores(min_score, nq, dev)
+    excl = None
+    if exclude is not None:
+        excl = torch.as_tensor(exclude, dtype=torch.int64).reshape(-1).to(dev)
+        if excl.numel() != nq:
+            raise ValueError("exclude: expected one row (or -1) per query (%d), got %d" % (nq, excl.numel()))
+    masks = None if label_mask is None else _label_masks(label_mask, nq, dev)
+    eps_t = _eps_for(stores, comm, wts, eps, q_res)
+    return wts, a_op, q_raw, q_norm, nq, ms, excl, masks, eps_t
+
+
+def _device_ctx(dev):
+    import contextlib
+    return torch.cuda.device(dev) if dev.type == "cuda" else contextlib.nullcontext()
+
+
+def _range_select(exact, cand, idx_offset, excl, ms, counts=None, off=None, max_len=0, out_s=None, out_i=None):
+    """xmve_range_select over one shard's rescored lists.  Count mode (``off`` None) -> int64 ``[rows]`` matches per
+    row.  Fill mode: the ``counts[r]`` matches of row r, sorted, to ``out_s`` / ``out_i`` ``[off[r], off[r] +
+    counts[r])``; ``max_len`` >= every ``counts[r]``."""
+    cand_count, _, cand_idx = cand
+    rows, cap = cand_idx.shape
+    st = N.stream_ptr()
+    if off is None:
+        counts = torch.empty((rows,), dtype=torch.int64, device=exact.device)
+        if rows:
+            N.call("xmve_range_select", N.ptr(exact), N.ptr(cand_idx), N.ptr(cand_count), rows, cap, int(idx_offset),
+                   N.ptr(excl), N.ptr(ms), N.ptr(counts), None, 0, None, None, None, st)
+        return counts
+    scratch = None
+    if max_len > RANGE_SMEM_MAX:
+        scratch = torch.empty((24 * out_s.numel(),), dtype=torch.uint8, device=exact.device)
+    if rows and max_len:
+        N.call("xmve_range_select", N.ptr(exact), N.ptr(cand_idx), N.ptr(cand_count), rows, cap, int(idx_offset),
+               N.ptr(excl), N.ptr(ms), N.ptr(counts), N.ptr(off), int(max_len), N.ptr(scratch), N.ptr(out_s),
+               N.ptr(out_i), st)
+
+
+def _range_merge(score, idx, seg_off, off, max_len, out_s, out_i):
+    """xmve_range_merge: the sorted runs ``score`` / ``idx [seg_off[s, r], seg_off[s, r + 1])`` of every segment s
+    -> row r of the CSR ``out_s`` / ``out_i`` at ``off``."""
+    n_seg, rows = seg_off.shape[0], seg_off.shape[1] - 1
+    if rows and max_len:
+        N.call("xmve_range_merge", N.ptr(score), N.ptr(idx), n_seg, N.ptr(seg_off), rows, N.ptr(off), int(max_len),
+               N.ptr(out_s), N.ptr(out_i), N.stream_ptr())
+
+
+def _pow2(x):
+    return 1 << max(0, int(x) - 1).bit_length()
+
+
+def range_search_shards(stores, queries, min_score, weights=None, exclude=None, label_mask=None, eps=None, stats=None,
+                        comm=None):
+    """Range search over a corpus cut into shards (:meth:`CorpusStore.range_search` is the one-shard case; ``comm`` as
+    in :func:`search_shards`, every rank passes the same queries and gets the same :class:`RangeResult`).
+
+    1. K1 on the queries; the error bound ``eps`` (``|approx - exact| <= eps``).
+    2. ``lo = round_down(min_score - 1.001 eps - 1e-7)``: a row with exact score >= min_score has an approximate score
+       above ``lo``.
+    3. K2 FILTER at ``lo`` over every shard, ``RANGE_CAP0`` entries per list.  The FILTER counts past the capacity, so
+       the maximum over shards of every list's length is known exactly after one all-gather of the counts.
+    4. rows whose list overflowed are re-run with their own capacity (the next power of two of that length), in
+       passes of at most ``RANGE_PASS_ENTRIES`` list entries.  All ranks take the same decisions from the same counts.
+    5. exact fp64 rescore of every listed candidate; ``xmve_range_select`` counts the rows with exact >= min_score.
+    6. one shard: cumsum, fill the sorted lists, done.  Several: the counts are gathered, every rank fills its
+       shards' runs into one packed block, the blocks are gathered and ``xmve_range_merge`` joins the runs.
+
+    ``stats`` (a dict) receives eps, candidates and results per query, re-run rows and passes, and ``phases_ms``.
+    The output size depends on the data, so the host reads the counts: a range search is never deferred or captured.
+    There is no ``n_total`` (``search_shards`` takes one): nothing here depends on the global row count.
+    """
+    comm = comm or SoloComm()
+    with _device_ctx(stores[0].device):
+        return _range_search(stores, queries, min_score, weights, exclude, label_mask, eps, stats, comm)
+
+
+def _range_search(stores, queries, min_score, weights, exclude, label_mask, eps, stats, comm):
+    ref = stores[0]
+    dev = ref.device
+    ph = _Phases(stats is not None and dev.type == "cuda")
+    ph.mark("start")
+    wts, a_op, q_raw, q_norm, nq, ms, excl, masks, eps_t = _range_setup(stores, queries, min_score, weights, exclude,
+                                                                        label_mask, eps, comm)
+    if nq == 0:
+        return RangeResult(torch.zeros((1,), dtype=torch.int64, device=dev),
+                           torch.empty((0,), dtype=torch.float64, device=dev),
+                           torch.empty((0,), dtype=torch.int64, device=dev))
+    # 2: the FILTER floor, rounded down so that exact >= min_score implies approx > lo
+    x = ms - (1.001 * eps_t.double() + 1e-7)
+    lo = x.float()
+    lo = torch.where(lo.double() > x, torch.nextafter(lo, torch.full_like(lo, float("-inf"))), lo)
+    ph.mark("prepare_queries")
+    n_st = len(stores)
+    solo = n_st * comm.world == 1
+
+    def sub(t, rows, dim=0):
+        if t is None or rows is None:
+            return t
+        return t.index_select(dim, rows).contiguous()
+
+    def filter_pass(rows, cap):
+        """FILTER over every local store for ``rows`` (None: all) -> (per-store lists, all-shard max count, host)."""
+        if rows is None:
+            a_sub, n_sub = a_op, nq
+        else:
+            n_sub = rows.numel()
+            a_sub = torch.zeros((_round_up(n_sub, _BM), ref.k), dtype=a_op.dtype, device=dev)
+            a_sub[:n_sub] = a_op[rows]
+        kw = {} if masks is None else {"label_mask": sub(masks, rows)}
+        cands = [s._filter(a_sub, n_sub, sub(lo, rows), cap, **kw) if s.n else None for s in stores]
+        cnt = torch.stack([c[0] if c is not None else torch.zeros((n_sub,), dtype=torch.int32, device=dev)
+                           for c in cands])
+        allc = _segments(list(cnt.unbind(0)), comm).to("cpu", torch.int64)        # one collective; host sync
+        return cands, allc
+
+    # 3: first pass
+    cands, allc = filter_pass(None, RANGE_CAP0)
+    need = allc.max(dim=0).values                                                   # longest list per row
+    bound = int(allc.sum())                                                         # >= the number of results
+    todo = torch.nonzero(need > RANGE_CAP0).flatten()
+    ph.mark("filter")
+    if dev.type == "cuda":
+        # what the call still allocates, at most: the re-run lists (scores + rows + fp64 rescore, 16 B per entry and
+        # local store, all kept until the fill) and the first pass's rescore; 16 B per result for the output and 24 B
+        # for the sort scratch of the block it is filled into; sharded, the block is padded to the largest rank's
+        # candidates and gathered from every rank
+        n_loc = sum(1 for s in stores if s.n)
+        want = 16 * n_loc * (sum(_pow2(int(c)) for c in need[todo]) + nq * RANGE_CAP0) + 16 * bound
+        if solo:
+            want += 24 * bound
+        else:
+            block = int(allc.sum(1).view(comm.world, n_st).sum(1).max())
+            want += (24 + 16 + 16 * comm.world) * block
+        free = torch.cuda.mem_get_info(dev)[0] + torch.cuda.memory_reserved(dev) - torch.cuda.memory_allocated(dev)
+        if want > free:
+            raise MemoryError(
+                "range_search: up to %d results (%.1f per query) need %.1f GB of device memory for the lists and their "
+                "buffers, but only %.1f GB are free on %s; range_count gives the exact counts without listing the "
+                "rows -- raise min_score or split the queries" % (bound, bound / nq, want / 1e9, free / 1e9, dev))
+    # pieces: (rows or None, per-store lists, cap); the last piece holding a row owns it.  The first pass's lists of
+    # the rows that are re-run are emptied, so that they are not rescored.
+    if todo.numel():
+        over = torch.zeros((nq,), dtype=torch.bool)
+        over[todo] = True
+        over = over.to(dev)
+        for c in cands:
+            if c is not None:
+                c[0].masked_fill_(over, 0)
+    pieces = [(None, cands, RANGE_CAP0)]
+    owner = torch.zeros((nq,), dtype=torch.int64)
+    passes = rerun_rows = 0
+    # 4: re-run the overflowed rows with lists sized from their exact counts
+    while todo.numel():
+        passes += 1
+        if passes > RANGE_PASSES:
+            raise N.XmveError("range_search: %d list(s) still overflow after %d re-run passes"
+                              % (todo.numel(), RANGE_PASSES))
+        rerun_rows += int(todo.numel())
+        caps = torch.tensor([_pow2(int(c)) for c in need[todo]], dtype=torch.int64)
+        nxt = []
+        for cap in sorted(set(caps.tolist())):
+            rows_c = todo[caps == cap]
+            per_pass = max(1, RANGE_PASS_ENTRIES // cap)
+            for r0 in range(0, rows_c.numel(), per_pass):
+                rows = rows_c[r0:r0 + per_pass]
+                cs, allc_r = filter_pass(rows.to(dev), cap)
+                got = allc_r.max(dim=0).values
+                need[rows] = got
+                nxt.append(rows[got > cap])
+                owner[rows] = len(pieces)
+                pieces.append((rows.to(dev), cs, cap))
+        todo = torch.cat(nxt)
+    ph.mark("rerun")
+    # 5: rescore every listed candidate, count the matches (rows a later piece owns count 0 here)
+    counts = torch.zeros((n_st, nq), dtype=torch.int64, device=dev)
+    done = []
+    for p, (rows, cs, cap) in enumerate(pieces):
+        own = (owner == p) if rows is None else (owner[rows.cpu()] == p)
+        own = own.to(dev)
+        q_sub, qn_sub, n_sub = sub(q_raw, rows), sub(q_norm, rows, 1), nq if rows is None else rows.numel()
+        ex_sub, ms_sub = sub(excl, rows), sub(ms, rows)
+        ex_p = []
+        for li, (s, c) in enumerate(zip(stores, cs)):
+            if c is None:
+                ex_p.append(None)
+                continue
+            e = s._rescore(q_sub, qn_sub, n_sub, wts, c, None)
+            cp = torch.where(own, _range_select(e, c, s.index_offset, ex_sub, ms_sub), torch.zeros((), dtype=torch.int64,
+                                                                                                  device=dev))
+            if rows is None:
+                counts[li] += cp
+            else:
+                counts[li].index_add_(0, rows, cp)
+            ex_p.append((e, cp))
+        done.append((rows, cs, cap, ex_sub, ms_sub, ex_p))
+    ph.mark("rescore_count")
+
+    def fill(li, s, starts, out_s, out_i):
+        """Fill store ``li``'s matches of every piece; row r's run starts at ``starts[r]``."""
+        for rows, cs, cap, ex_sub, ms_sub, ex_p in done:
+            if ex_p[li] is None:
+                continue
+            e, cp = ex_p[li]
+            max_len = min(cap, int(counts_h[li].max())) if rows is None else min(cap, int(counts_h[li][rows.cpu()].max()))
+            _range_select(e, cs[li], s.index_offset, ex_sub, ms_sub, counts=cp, off=sub(starts, rows), max_len=max_len,
+                          out_s=out_s, out_i=out_i)
+
+    # 6: lay the lists out
+    if solo:
+        counts_h = counts.cpu()                                                                     # host sync
+        off_h = torch.zeros((nq + 1,), dtype=torch.int64)
+        off_h[1:] = torch.cumsum(counts_h[0], 0)
+        total = int(off_h[-1])
+        off = off_h.to(dev)
+        out_s = torch.empty((total,), dtype=torch.float64, device=dev)
+        out_i = torch.empty((total,), dtype=torch.int64, device=dev)
+        fill(0, ref, off[:-1], out_s, out_i)
+    else:
+        counts_h = counts.cpu()
+        allc = _segments(list(counts.unbind(0)), comm).cpu()                       # [G * L, nq]: one collective
+        off_h = torch.zeros((nq + 1,), dtype=torch.int64)
+        off_h[1:] = torch.cumsum(allc.sum(0), 0)
+        total = int(off_h[-1])
+        seg_tot = allc.sum(1).view(comm.world, n_st)
+        block_len = max(1, int(seg_tot.sum(1).max()))                              # padded to the largest rank's
+        # this rank's block: [scores fp64 | rows int64], each block_len long; store li's runs from base[li]
+        block = torch.empty((2 * block_len,), dtype=torch.int64, device=dev)
+        b_s, b_i = block[:block_len].view(torch.float64), block[block_len:]
+        loc_tot = counts_h.sum(1)
+        base = torch.cumsum(loc_tot, 0) - loc_tot
+        for li, s in enumerate(stores):
+            starts = torch.cumsum(counts_h[li], 0) - counts_h[li] + base[li]
+            fill(li, s, starts.to(dev), b_s, b_i)
+        ph.mark("fill")
+        gathered = block.unsqueeze(0) if comm.world == 1 else comm.gather(block)   # [G, 2 * block_len]
+        # run (segment g * L + l, row r) starts at g * 2 block_len + (store l's base on rank g) + its offset
+        seg_base = (torch.cumsum(seg_tot, 1) - seg_tot) + (torch.arange(comm.world) * 2 * block_len)[:, None]
+        seg_off = torch.zeros((comm.world * n_st, nq + 1), dtype=torch.int64)
+        seg_off[:, 1:] = torch.cumsum(allc, 1)
+        seg_off += seg_base.reshape(-1, 1)
+        flat = gathered.reshape(-1)
+        off = off_h.to(dev)
+        out_s = torch.empty((total,), dtype=torch.float64, device=dev)
+        out_i = torch.empty((total,), dtype=torch.int64, device=dev)
+        _range_merge(flat.view(torch.float64), flat[block_len:], seg_off.to(dev), off,
+                     int((off_h[1:] - off_h[:-1]).max()), out_s, out_i)
+    ph.mark("select_merge")
+    if stats is not None:
+        stats["eps"] = float(eps_t)
+        stats["cap"] = RANGE_CAP0
+        stats["candidates_per_query"] = bound / nq
+        stats["rerun_rows"] = rerun_rows
+        stats["passes"] = passes
+        stats["results_per_query"] = total / nq
+        stats["phases_ms"] = ph.result()
+    return RangeResult(off, out_s, out_i)
+
+
+def range_count_shards(stores, queries, min_score, weights=None, exclude=None, label_mask=None, eps=None, comm=None,
+                       cap=8192, stats=None):
+    """int64 ``[nq]`` on the device: the length of every :func:`range_search_shards` list for the same arguments,
+    without listing the rows.  :func:`rank_of_gt`'s count with ``s = min_score`` and ``g = INT64_MAX``: rows whose
+    approximate score is more than eps above ``min_score`` are counted by the FILTER, the rows within eps of it
+    (at most ``cap`` per query; beyond, an exact fp64 pass) are rescored and compared exactly; ONE all-reduce adds
+    the shards.  An excluded row is subtracted where its exact score reaches ``min_score`` (and its label is
+    allowed).  No ``n_total``, as for :func:`range_search_shards`."""
+    comm = comm or SoloComm()
+    stores = list(stores) if isinstance(stores, (list, tuple)) else [stores]
+    with _device_ctx(stores[0].device):
+        wts, a_op, q_raw, q_norm, nq, ms, excl, masks, eps_t = _range_setup(stores, queries, min_score, weights,
+                                                                            exclude, label_mask, eps, comm)
+        dev = stores[0].device
+        if nq == 0:
+            return torch.zeros((0,), dtype=torch.int64, device=dev)
+        live = [s for s in stores if s.n]
+        g = torch.full((nq,), torch.iinfo(torch.int64).max, dtype=torch.int64, device=dev)
+        count, n_deep = _count_before_all(live, comm, a_op, q_raw, q_norm, nq, wts, ms, g, eps_t, cap, masks)
+        if excl is not None:
+            s_ex = comm.max_(_row_scores(live, q_raw, q_norm, nq, wts, excl, masks))
+            count = count - ((s_ex > float("-inf")) & (s_ex >= ms)).to(torch.int64)
+        if stats is not None:
+            stats["eps"] = float(eps_t)
+            stats["deep_entries"] = n_deep
+        return count
 
 
 def search_norm_score(stores, queries, k, weights=None, comm=None, n_total=None, **kw):

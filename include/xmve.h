@@ -226,6 +226,34 @@ XMVE_API int xmve_merge_topk_packed(const void* packed, int32_t n_seg, int64_t s
                            const int64_t* exclude, int32_t k, const float* thr, float eps, const float* eps_dev,
                            double* out_score, int64_t* out_idx, int32_t* cert, float* thr_next,
                            int32_t* n_uncertified, void* stream);
+/* ---- range search: every corpus row whose exact score reaches a per-row minimum -------------------------------
+ * A new capability with no counterpart in the reference, which only ranks whole score rows.  The caller has listed,
+ * with xmve_score_filter at lo[r] <= min_score[r] - eps, every row that can reach min_score[r] and rescored the list
+ * (xmve_rescore, bound = NULL).  Entry c < min(cand_count[r], cap) of row r matches iff exact[r, c] > -inf,
+ * exact[r, c] >= min_score[r] (NaN never matches) and its global row cand_idx + idx_offset differs from exclude[r]
+ * (exclude may be NULL).  min_score fp64 [rows], exact fp64 [rows, cap], cand_idx int32 [rows, cap].
+ *   count (off == NULL): counts[r] = the number of matches of row r (int64 [rows], written).
+ *   fill  (off != NULL): counts is the count mode's result (read); the matches of row r are written, sorted by
+ *         (score desc, global row asc), to out_score / out_idx [off[r], off[r] + counts[r]).  off int64 [rows] holds
+ *         the start positions, normally the exclusive cumsum of counts (the first rows of a CSR's offsets); any starts
+ *         whose ranges do not overlap will do, so a subset of rows can be filled into a larger CSR.  max_len >=
+ *         max_r counts[r] sizes the sort.  Rows of up to 16384 matches are sorted in shared memory; longer rows need
+ *         scratch (DEVICE, 24 bytes per output entry: row r uses bytes [24 off[r], 24 (off[r] + counts[r]))) and
+ *         return XMVE_ERR_LIMIT without it.
+ * xmve_range_merge joins the per-shard results: run (s, r) of segment s < n_seg is the sorted entries
+ * score / idx [seg_off[s, r], seg_off[s, r + 1]) (seg_off int64 [n_seg, rows + 1], positions into score and idx,
+ * which are DEVICE fp64 / int64 with global rows).  Row r's runs are merged, in the same order, into
+ * out_score / out_idx [off[r], off[r + 1]) (off int64 [rows + 1]); the runs of a row must hold off[r + 1] - off[r]
+ * entries in all and no (score, row) pair twice (shards own disjoint rows).  max_len >= max_r off[r + 1] - off[r]
+ * sizes the grid.  Runs are merged by binary search, so runs of any length need no scratch.
+ */
+XMVE_API int xmve_range_select(const double* exact, const int32_t* cand_idx, const int32_t* cand_count, int64_t rows,
+                      int32_t cap, int64_t idx_offset, const int64_t* exclude, const double* min_score,
+                      int64_t* counts, const int64_t* off, int64_t max_len, void* scratch,
+                      double* out_score, int64_t* out_idx, void* stream);
+XMVE_API int xmve_range_merge(const double* score, const int64_t* idx, int32_t n_seg, const int64_t* seg_off,
+                     int64_t rows, const int64_t* off, int64_t max_len, double* out_score, int64_t* out_idx,
+                     void* stream);
 /* The j largest values of each row in descending order, -inf padded: out fp32 [rows, j] (j <= 4096).
  * Row r holds min(counts[r], cols) valid values (counts == NULL: cols).  The j-th largest value of a corpus
  * that is sharded over GPUs is the j-th largest of the union of the shards' top-j lists. */

@@ -1,6 +1,7 @@
-"""Compare the SASS instruction streams of the score kernels in two builds of score_tc.o:
+"""Compare the SASS instruction streams of the kernels in two builds of one object file:
 
     python tools/compare_sass.py OLD/score_tc.o NEW/score_tc.o
+    python tools/compare_sass.py OLD/select.o NEW/select.o
 
 Kernels are matched by name with the anonymous-namespace hash removed and an added ``bool = false`` template argument
 dropped; instruction offsets and encodings are ignored.  Prints ``identical`` / ``DIFFERENT`` per kernel of the old
@@ -32,7 +33,7 @@ def kernels(obj):
 
 
 def normalised(name):
-    name = re.sub(r"_GLOBAL__N__[0-9a-f]+_\d+_score_tc_cu_[0-9a-f]+", "", name)
+    name = re.sub(r"_GLOBAL__N__[0-9a-f]+_\d+_\w+?_cu_[0-9a-f]+", "", name)
     return name.replace("ELb0EEE", "EEE")
 
 
