@@ -3,6 +3,8 @@
     python -m cross_modal_video_engine_b200.cli search --corpus DIR|video_data.pt --queries Q.npy --topK 10
         [--labels L.npy --label-mask MASK|M.npy]     (only rows whose label bit is set in the query's mask)
         [--min-score S|S.npy]                        (every row scoring at least S instead of the top K)
+    python -m cross_modal_video_engine_b200.cli pairs  --corpus DIR|video_data.pt --min-score S [--out FILE]
+        (every pair of corpus rows scoring at least S, each once: one line 'id_i id_j score' per pair)
     python -m cross_modal_video_engine_b200.cli eval   --corpus DIR|video_data.pt --queries Q.npy --caption-ids ids.txt
     python -m cross_modal_video_engine_b200.cli composed --index index.pt --queries queries.pt [--out results_wo_attn]
 
@@ -75,6 +77,12 @@ def parse_args(argv=None):
     s.add_argument("--min-score", default=None,
                    help="range search: every row whose fused score is at least this (a float, or a .npy with one per "
                         "query) instead of the top K; --topK is then unused")
+    pr = sub.add_parser("pairs")
+    pr.add_argument("--corpus", required=True, help="BigFile directory or video_data.pt")
+    pr.add_argument("--min-score", required=True, type=float, help="list every pair of rows scoring at least this")
+    pr.add_argument("--dims", default=None, help="comma-separated embedding-space dims (default: one space)")
+    pr.add_argument("--weights", default=None, help="comma-separated fusion weights, one per space")
+    pr.add_argument("--out", default=None, help="write the pairs here instead of printing them")
     e = sub.choices["eval"]
     e.add_argument("--caption-ids", required=True, help="caption ids 'video7#enc#3' (util/metrics.py:111), one per query")
     e.add_argument("--save-topk", default=None, help="save {'scores','idx','video_ids'} of the top-K lists here")
@@ -104,6 +112,8 @@ def main(argv=None):
         return _composed(args)
     from . import avs
     store, video_ids = _load_corpus(args.corpus, args.dims)
+    if args.cmd == "pairs":
+        return _pairs(args, store, video_ids)
     q = _load_matrix(args.queries)
     if args.cmd == "search":
         if args.labels is not None:
@@ -156,6 +166,19 @@ def _eval(args, store, video_ids, q):
     if args.save_topk:
         scores, idx = store.search(q, args.topK, weights=args.weights)
         torch.save({"scores": scores.cpu(), "idx": idx.cpu(), "video_ids": video_ids}, args.save_topk)
+    return 0
+
+
+def _pairs(args, store, video_ids):
+    """One line ``id_i id_j score`` per pair (i < j), in the order of ``similar_pairs``: by row i, then score desc."""
+    i, j, s = (t.cpu().numpy() for t in store.similar_pairs(args.min_score, weights=args.weights).pairs())
+    lines = ["%s %s %r" % (video_ids[a], video_ids[b], float(c)) for a, b, c in zip(i, j, s)]
+    if args.out:
+        with open(args.out, "w") as f:
+            f.write("".join(ln + "\n" for ln in lines))
+    else:
+        for ln in lines:
+            print(ln)
     return 0
 
 

@@ -488,26 +488,30 @@ int pow2_ceil(int64_t x) {
 
 // ---- range search: every rescored candidate whose exact score reaches a per-row minimum ---------------------------
 // Entry c < min(counts[r], cap) of row r matches iff exact > -inf, exact >= min_score[r] (NaN never does) and its
-// global row idx + idx_offset is not exclude[r].  Counting and filling apply the same test, so the fill finds exactly
-// the number of entries the count gave.
+// global row idx + idx_offset is not exclude[r]; with kAfter (similar pairs) its global row must also exceed
+// after[r].  Counting and filling apply the same test, so the fill finds exactly the number of entries the count gave.
 constexpr int RANGE_SMEM_MAX = 16384;                       // entries sorted in shared memory (12 B each)
 
-__device__ __forceinline__ bool range_hit(double s, int64_t row, double lo, int64_t excl) {
-  return s > -CUDART_INF && s >= lo && row != excl;
+template <bool kAfter>
+__device__ __forceinline__ bool range_hit(double s, int64_t row, double lo, int64_t excl, int64_t floor) {
+  return s > -CUDART_INF && s >= lo && row != excl && (!kAfter || row > floor);
 }
 
+template <bool kAfter>
 __global__ void __launch_bounds__(256)
 range_count_kernel(const double* __restrict__ exact, const int32_t* __restrict__ idx, const int32_t* __restrict__ counts,
                    int cap, int64_t idx_offset, const int64_t* __restrict__ exclude, const double* __restrict__ min_score,
-                   int64_t* __restrict__ out) {
+                   int64_t* __restrict__ out, const int64_t* __restrict__ after) {
   __shared__ int part[8];
   const int64_t r = blockIdx.x;
   const int n = min(counts[r], cap);
   const double lo = min_score[r];
   const int64_t excl = exclude ? exclude[r] : -1;
+  const int64_t floor = kAfter ? after[r] : 0;
   int mine = 0;
   for (int i = threadIdx.x; i < n; i += blockDim.x)
-    mine += range_hit(exact[r * cap + i], static_cast<int64_t>(idx[r * cap + i]) + idx_offset, lo, excl) ? 1 : 0;
+    mine += range_hit<kAfter>(exact[r * cap + i], static_cast<int64_t>(idx[r * cap + i]) + idx_offset, lo, excl, floor)
+                ? 1 : 0;
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) mine += __shfl_xor_sync(0xffffffffu, mine, o);
   if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = mine;
@@ -522,11 +526,12 @@ range_count_kernel(const double* __restrict__ exact, const int32_t* __restrict__
 // Row r's m = len[r] matches are compacted, sorted by (score desc, row asc) with bitonic_sort_pairs and written to
 // [off[r], off[r] + m).  Rows of up to smem_cap entries sort in shared memory; longer rows in the caller's scratch, row
 // r at byte 24 * off[r]: 2m fp64 keys then 2m int32 rows (room for the power-of-two padding, P < 2m).
+template <bool kAfter>
 __global__ void __launch_bounds__(1024)
 range_fill_kernel(const double* __restrict__ exact, const int32_t* __restrict__ idx, const int32_t* __restrict__ counts,
                   int cap, int64_t idx_offset, const int64_t* __restrict__ exclude, const double* __restrict__ min_score,
                   const int64_t* __restrict__ off, const int64_t* __restrict__ len, int smem_cap, uint8_t* scratch,
-                  double* __restrict__ out_score, int64_t* __restrict__ out_idx) {
+                  double* __restrict__ out_score, int64_t* __restrict__ out_idx, const int64_t* __restrict__ after) {
   extern __shared__ __align__(16) uint8_t range_smem[];
   __shared__ int n_s;
   const int64_t r = blockIdx.x;
@@ -545,13 +550,14 @@ range_fill_kernel(const double* __restrict__ exact, const int32_t* __restrict__ 
   const int n = min(counts[r], cap);
   const double lo = min_score[r];
   const int64_t excl = exclude ? exclude[r] : -1;
+  const int64_t floor = kAfter ? after[r] : 0;
   if (threadIdx.x == 0) n_s = 0;
   __syncthreads();
   for (int base = threadIdx.x & ~31; base < n; base += blockDim.x) {          // warp-aggregated compaction
     const int i = base + (threadIdx.x & 31);
     const double s = i < n ? exact[r * cap + i] : -CUDART_INF;
     const int32_t v = i < n ? idx[r * cap + i] : 0;
-    const bool keep = i < n && range_hit(s, static_cast<int64_t>(v) + idx_offset, lo, excl);
+    const bool keep = i < n && range_hit<kAfter>(s, static_cast<int64_t>(v) + idx_offset, lo, excl, floor);
     const unsigned mk = __ballot_sync(0xffffffffu, keep);
     if (mk != 0) {
       int pos = 0;
@@ -850,38 +856,60 @@ extern "C" int64_t xmve_packed_topk_bytes(int64_t rows, int32_t len) {
   return (b + 15) / 16 * 16;
 }
 
-extern "C" int xmve_range_select(const double* exact, const int32_t* cand_idx, const int32_t* cand_count, int64_t rows,
-                                 int32_t cap, int64_t idx_offset, const int64_t* exclude, const double* min_score,
-                                 int64_t* counts, const int64_t* off, int64_t max_len, void* scratch,
-                                 double* out_score, int64_t* out_idx, void* stream) {
+namespace {
+// count / fill of xmve_range_select (kAfter false) and xmve_pair_select (kAfter true)
+template <bool kAfter>
+int range_select(const char* name, const double* exact, const int32_t* cand_idx, const int32_t* cand_count,
+                 int64_t rows, int32_t cap, int64_t idx_offset, const int64_t* exclude, const double* min_score,
+                 int64_t* counts, const int64_t* off, int64_t max_len, void* scratch, double* out_score,
+                 int64_t* out_idx, const int64_t* after, void* stream) {
   using namespace xmve;
   XMVE_DEVICE_OR_RETURN();
-  XMVE_REQUIRE(exact && cand_idx && cand_count && min_score && counts && rows >= 0 && cap > 0,
-               "range_select: bad arguments");
+  XMVE_REQUIRE(exact && cand_idx && cand_count && min_score && counts && rows >= 0 && cap > 0 && (!kAfter || after),
+               "%s: bad arguments", name);
   if (rows == 0) return XMVE_OK;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (off == nullptr) {
-    range_count_kernel<<<static_cast<unsigned>(rows), 256, 0, st>>>(exact, cand_idx, cand_count, cap, idx_offset,
-                                                                      exclude, min_score, counts);
+    range_count_kernel<kAfter><<<static_cast<unsigned>(rows), 256, 0, st>>>(exact, cand_idx, cand_count, cap,
+                                                                              idx_offset, exclude, min_score, counts,
+                                                                              after);
     return launch_status("range_count_kernel");
   }
-  XMVE_REQUIRE(out_score && out_idx && max_len >= 0 && max_len <= cap, "range_select: fill needs outputs, 0 <= max_len <= cap");
+  XMVE_REQUIRE(out_score && out_idx && max_len >= 0 && max_len <= cap, "%s: fill needs outputs, 0 <= max_len <= cap",
+               name);
   if (max_len > RANGE_SMEM_MAX && scratch == nullptr)
-    return fail(XMVE_ERR_LIMIT, "range_select: a row has %lld entries (> %d): pass scratch (24 bytes per output entry)",
+    return fail(XMVE_ERR_LIMIT, "%s: a row has %lld entries (> %d): pass scratch (24 bytes per output entry)", name,
                 static_cast<long long>(max_len), RANGE_SMEM_MAX);
   const int smem_cap = pow2_ceil(max_len < 1 ? 1 : (max_len > RANGE_SMEM_MAX ? RANGE_SMEM_MAX : max_len));
   const int smem_bytes = smem_cap * static_cast<int>(sizeof(double) + sizeof(int32_t));
   static int attr_bytes[MAX_DEVICES] = {};
   const int dev = current_device();
-  if (dev < 0) return fail(XMVE_ERR_DEVICE, "range_select: no current device");
+  if (dev < 0) return fail(XMVE_ERR_DEVICE, "%s: no current device", name);
   if (smem_bytes > attr_bytes[dev]) {
-    XMVE_CUDA(cudaFuncSetAttribute(range_fill_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
+    XMVE_CUDA(cudaFuncSetAttribute(range_fill_kernel<kAfter>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
     attr_bytes[dev] = smem_bytes;
   }
-  range_fill_kernel<<<static_cast<unsigned>(rows), max_len > 2048 ? 1024 : 256, smem_bytes, st>>>(
+  range_fill_kernel<kAfter><<<static_cast<unsigned>(rows), max_len > 2048 ? 1024 : 256, smem_bytes, st>>>(
       exact, cand_idx, cand_count, cap, idx_offset, exclude, min_score, off, counts, smem_cap,
-      static_cast<uint8_t*>(scratch), out_score, out_idx);
+      static_cast<uint8_t*>(scratch), out_score, out_idx, after);
   return launch_status("range_fill_kernel");
+}
+}  // namespace
+
+extern "C" int xmve_range_select(const double* exact, const int32_t* cand_idx, const int32_t* cand_count, int64_t rows,
+                                 int32_t cap, int64_t idx_offset, const int64_t* exclude, const double* min_score,
+                                 int64_t* counts, const int64_t* off, int64_t max_len, void* scratch,
+                                 double* out_score, int64_t* out_idx, void* stream) {
+  return range_select<false>("range_select", exact, cand_idx, cand_count, rows, cap, idx_offset, exclude, min_score,
+                             counts, off, max_len, scratch, out_score, out_idx, nullptr, stream);
+}
+
+extern "C" int xmve_pair_select(const double* exact, const int32_t* cand_idx, const int32_t* cand_count, int64_t rows,
+                                int32_t cap, int64_t idx_offset, const int64_t* exclude, const double* min_score,
+                                int64_t* counts, const int64_t* off, int64_t max_len, void* scratch,
+                                double* out_score, int64_t* out_idx, const int64_t* after, void* stream) {
+  return range_select<true>("pair_select", exact, cand_idx, cand_count, rows, cap, idx_offset, exclude, min_score,
+                            counts, off, max_len, scratch, out_score, out_idx, after, stream);
 }
 
 extern "C" int xmve_range_merge(const double* score, const int64_t* idx, int32_t n_seg, const int64_t* seg_off,

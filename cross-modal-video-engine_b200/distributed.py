@@ -126,3 +126,13 @@ def sharded_range_count(store, queries, min_score, group=None, **kw):
     if not dist.is_initialized() or dist.get_world_size(group) == 1:
         return range_count_shards(stores, queries, min_score, **kw)
     return range_count_shards(stores, queries, min_score, comm=GroupComm(group), **kw)
+
+
+def sharded_similar_pairs(store, min_score, group=None, **kw):
+    """Similar pairs (``engine.similar_pairs_shards``) of the corpus whose rows are sharded over the ranks of ``group``:
+    every pair of rows ``i < j`` scoring at least ``min_score``, each once; every rank gets the same ``RangeResult``."""
+    from .engine import similar_pairs_shards
+    stores = list(store) if isinstance(store, (list, tuple)) else [store]
+    if not dist.is_initialized() or dist.get_world_size(group) == 1:
+        return similar_pairs_shards(stores, min_score, **kw)
+    return similar_pairs_shards(stores, min_score, comm=GroupComm(group), **kw)

@@ -345,6 +345,30 @@ class CorpusStore:
         return range_count_shards([self], queries, min_score, weights=weights, exclude=exclude,
                                   label_mask=label_mask, eps=eps)
 
+    def similar_pairs(self, min_score, weights=None, eps=None, stats=None):
+        """Every pair of stored rows ``i < j`` whose exact fused score reaches ``min_score`` (one float), each pair once
+        -> :class:`RangeResult` with one list per row ``i``: the rows ``j > i`` with ``s(i, j) >= min_score``, sorted
+        by (score desc, j asc).  ``s(i, j)`` is the fp64 score :meth:`range_search` gives row ``j`` for the stored
+        row ``i`` as the query.  ``+inf`` gives no pairs, ``-inf`` every pair; NaN raises ``ValueError``.
+        :meth:`RangeResult.pairs` gives the COO form.  See :func:`similar_pairs_shards`."""
+        return similar_pairs_shards([self], min_score, weights=weights, eps=eps, stats=stats)
+
+    def _suffix(self, start):
+        """This store's rows ``[start, n)`` as a store of their own, without copies (global rows keep their numbers):
+        operand, raw rows, norm and residual planes and labels offset by ``start``.  The norm planes keep their
+        ``[S, capacity]`` row stride, which is what the rescore reads; the operand's row stride is a multiple of 128 B,
+        so its tensor map may start at any row.  The error bound reads this store's residuals over EVERY row."""
+        start = min(int(start), self.n)
+        v = object.__new__(type(self))
+        v.__dict__.update(self.__dict__)
+        v.op, v.raw = self.op[start:], self.raw[start:]
+        v.norm, v.resid = self.norm[:, start:], self.resid[:, start:]
+        v.labels = None if self.labels is None else self.labels[start:]
+        v.n, v.capacity, v.index_offset = self.n - start, self.capacity - start, self.index_offset + start
+        v.resid_max2 = self.resid_max2
+        v._dv2_cache = None                                   # (keyed by row counts: a view's must not hit it)
+        return v
+
     def plan(self, k, n=None):
         return plan(k, self.n if n is None else n)
 
@@ -1439,6 +1463,13 @@ class RangeResult:
             out_i[row, col] = self.idx
         return out_s, out_i
 
+    def pairs(self):
+        """COO form in CSR order: ``(row int64, idx int64, scores fp64)`` on the device, ``row[e]`` the list (query,
+        or stored row of :meth:`CorpusStore.similar_pairs`) that entry ``e`` belongs to."""
+        n = self.offsets.numel() - 1
+        row = torch.repeat_interleave(torch.arange(n, device=self.offsets.device), self.offsets[1:] - self.offsets[:-1])
+        return row, self.idx, self.scores
+
 
 def _min_scores(min_score, nq, device):
     """``min_score`` (a float or one per query) -> fp64 device tensor ``[nq]``; ValueError on NaN or a wrong shape."""
@@ -1479,26 +1510,29 @@ def _device_ctx(dev):
     return torch.cuda.device(dev) if dev.type == "cuda" else contextlib.nullcontext()
 
 
-def _range_select(exact, cand, idx_offset, excl, ms, counts=None, off=None, max_len=0, out_s=None, out_i=None):
+def _range_select(exact, cand, idx_offset, excl, ms, counts=None, off=None, max_len=0, out_s=None, out_i=None,
+                  after=None):
     """xmve_range_select over one shard's rescored lists.  Count mode (``off`` None) -> int64 ``[rows]`` matches per
     row.  Fill mode: the ``counts[r]`` matches of row r, sorted, to ``out_s`` / ``out_i`` ``[off[r], off[r] +
-    counts[r])``; ``max_len`` >= every ``counts[r]``."""
+    counts[r])``; ``max_len`` >= every ``counts[r]``.  ``after`` (int64 ``[rows]``, :func:`similar_pairs_shards`):
+    xmve_pair_select, which also drops every global row ``<= after[r]``."""
     cand_count, _, cand_idx = cand
     rows, cap = cand_idx.shape
     st = N.stream_ptr()
+    fn, tail = ("xmve_range_select", ()) if after is None else ("xmve_pair_select", (N.ptr(after),))
     if off is None:
         counts = torch.empty((rows,), dtype=torch.int64, device=exact.device)
         if rows:
-            N.call("xmve_range_select", N.ptr(exact), N.ptr(cand_idx), N.ptr(cand_count), rows, cap, int(idx_offset),
-                   N.ptr(excl), N.ptr(ms), N.ptr(counts), None, 0, None, None, None, st)
+            N.call(fn, N.ptr(exact), N.ptr(cand_idx), N.ptr(cand_count), rows, cap, int(idx_offset),
+                   N.ptr(excl), N.ptr(ms), N.ptr(counts), None, 0, None, None, None, *tail, st)
         return counts
     scratch = None
     if max_len > RANGE_SMEM_MAX:
         scratch = torch.empty((24 * out_s.numel(),), dtype=torch.uint8, device=exact.device)
     if rows and max_len:
-        N.call("xmve_range_select", N.ptr(exact), N.ptr(cand_idx), N.ptr(cand_count), rows, cap, int(idx_offset),
+        N.call(fn, N.ptr(exact), N.ptr(cand_idx), N.ptr(cand_count), rows, cap, int(idx_offset),
                N.ptr(excl), N.ptr(ms), N.ptr(counts), N.ptr(off), int(max_len), N.ptr(scratch), N.ptr(out_s),
-               N.ptr(out_i), st)
+               N.ptr(out_i), *tail, st)
 
 
 def _range_merge(score, idx, seg_off, off, max_len, out_s, out_i):
@@ -1539,7 +1573,9 @@ def range_search_shards(stores, queries, min_score, weights=None, exclude=None, 
         return _range_search(stores, queries, min_score, weights, exclude, label_mask, eps, stats, comm)
 
 
-def _range_search(stores, queries, min_score, weights, exclude, label_mask, eps, stats, comm):
+def _range_search(stores, queries, min_score, weights, exclude, label_mask, eps, stats, comm, after=None, held=None):
+    """``after`` and ``held``: one block of :func:`similar_pairs_shards` -- row r keeps only the global rows above
+    ``after[r]``; ``held`` pairs found by the earlier blocks are counted into the memory check."""
     ref = stores[0]
     dev = ref.device
     ph = _Phases(stats is not None and dev.type == "cuda")
@@ -1597,6 +1633,13 @@ def _range_search(stores, queries, min_score, weights, exclude, label_mask, eps,
             block = int(allc.sum(1).view(comm.world, n_st).sum(1).max())
             want += (24 + 16 + 16 * comm.world) * block
         free = torch.cuda.mem_get_info(dev)[0] + torch.cuda.memory_reserved(dev) - torch.cuda.memory_allocated(dev)
+        if held is not None:
+            want += 16 * (held + bound) + 8 * nq                    # the final concatenation of every block's lists
+            if want > free:
+                raise MemoryError(
+                    "similar_pairs: %d pairs found so far and up to %d more in the next %d rows need %.1f GB of device "
+                    "memory for the lists, their buffers and the final result, but only %.1f GB are free on %s; raise "
+                    "min_score" % (held, bound, nq, want / 1e9, free / 1e9, dev))
         if want > free:
             raise MemoryError(
                 "range_search: up to %d results (%.1f per query) need %.1f GB of device memory for the lists and their "
@@ -1644,31 +1687,32 @@ def _range_search(stores, queries, min_score, weights, exclude, label_mask, eps,
         own = own.to(dev)
         q_sub, qn_sub, n_sub = sub(q_raw, rows), sub(q_norm, rows, 1), nq if rows is None else rows.numel()
         ex_sub, ms_sub = sub(excl, rows), sub(ms, rows)
+        fl = {} if after is None else {"after": sub(after, rows)}
         ex_p = []
         for li, (s, c) in enumerate(zip(stores, cs)):
             if c is None:
                 ex_p.append(None)
                 continue
             e = s._rescore(q_sub, qn_sub, n_sub, wts, c, None)
-            cp = torch.where(own, _range_select(e, c, s.index_offset, ex_sub, ms_sub), torch.zeros((), dtype=torch.int64,
-                                                                                                  device=dev))
+            cp = torch.where(own, _range_select(e, c, s.index_offset, ex_sub, ms_sub, **fl),
+                             torch.zeros((), dtype=torch.int64, device=dev))
             if rows is None:
                 counts[li] += cp
             else:
                 counts[li].index_add_(0, rows, cp)
             ex_p.append((e, cp))
-        done.append((rows, cs, cap, ex_sub, ms_sub, ex_p))
+        done.append((rows, cs, cap, ex_sub, ms_sub, fl, ex_p))
     ph.mark("rescore_count")
 
     def fill(li, s, starts, out_s, out_i):
         """Fill store ``li``'s matches of every piece; row r's run starts at ``starts[r]``."""
-        for rows, cs, cap, ex_sub, ms_sub, ex_p in done:
+        for rows, cs, cap, ex_sub, ms_sub, fl, ex_p in done:
             if ex_p[li] is None:
                 continue
             e, cp = ex_p[li]
             max_len = min(cap, int(counts_h[li].max())) if rows is None else min(cap, int(counts_h[li][rows.cpu()].max()))
             _range_select(e, cs[li], s.index_offset, ex_sub, ms_sub, counts=cp, off=sub(starts, rows), max_len=max_len,
-                          out_s=out_s, out_i=out_i)
+                          out_s=out_s, out_i=out_i, **fl)
 
     # 6: lay the lists out
     if solo:
@@ -1747,6 +1791,91 @@ def range_count_shards(stores, queries, min_score, weights=None, exclude=None, l
             stats["eps"] = float(eps_t)
             stats["deep_entries"] = n_deep
         return count
+
+
+#: similar pairs: the stored rows are walked in blocks of this many query rows.  8192 x 2048 bf16 rows is one FILTER
+#: super-block, so each corpus line streams from HBM once per block.
+PAIR_BLOCK = 8192
+
+
+def similar_pairs_shards(stores, min_score, weights=None, eps=None, stats=None, comm=None):
+    """Every pair of corpus rows ``i < j`` whose exact fused score reaches ``min_score`` (one float), each pair once,
+    over a corpus cut into shards (:meth:`CorpusStore.similar_pairs` is the one-shard case; ``comm`` as in
+    :func:`search_shards`, every rank gets the same result) -> :class:`RangeResult` with one list per global row ``i <
+    N``, ``N`` the largest ``index_offset + n`` of all shards (rows no shard holds get empty lists).  Row ``i``'s list
+    holds the rows ``j > i`` with ``s(i, j) >= min_score``, sorted by (score desc, j asc); ``s(i, j)`` is the score
+    :func:`range_search_shards` gives row ``j`` for the stored row ``i`` as the query.
+
+    1. the global rows are cut into blocks of ``PAIR_BLOCK`` rows, none spanning two shards; every rank derives the
+       same schedule from one gather of every shard's ``(index_offset, n)``.
+    2. a block's queries are its rows' stored fp32 ``raw`` rows (K1 applies the weights as for any query batch).  With
+       several ranks the owner's rows reach the others through one all-reduce(sum) of a zero-filled buffer that only
+       the owner fills, so the sum is exact.
+    3. every shard scans only its rows ``j >= r0`` (a suffix view, :meth:`CorpusStore._suffix`); the wasted lower half
+       of the diagonal block is ``PAIR_BLOCK / n`` of the work.  The range pipeline (:func:`range_search_shards`: the
+       FILTER at ``round_down(min_score - 1.001 eps - 1e-7)``, the re-run from exact counts, the fp64 rescore, the
+       count gather and merge) runs on those views, with ``xmve_pair_select`` keeping only ``j > i``.  eps bounds the
+       residuals of every stored row, a superset of the scanned ones.
+    4. the blocks' lists are appended.  Before a block allocates, the memory it needs, the pairs found so far and the
+       final concatenation are checked against the free device memory: an output that cannot fit raises a sized
+       ``MemoryError``.
+
+    ``stats`` (a dict) receives eps (the largest of the blocks'), blocks, candidates, pairs, re-run rows and passes,
+    and ``phases_ms`` summed over the blocks."""
+    comm = comm or SoloComm()
+    stores = list(stores) if isinstance(stores, (list, tuple)) else [stores]
+    with _device_ctx(stores[0].device):
+        return _similar_pairs(stores, min_score, weights, eps, stats, comm)
+
+
+def _similar_pairs(stores, min_score, weights, eps, stats, comm):
+    ms = float(min_score)
+    if math.isnan(ms):
+        raise ValueError("min_score: NaN")
+    ref = stores[0]
+    dev = ref.device
+    d_all = sum(ref.dims)
+    shards = _segments([torch.tensor([s.index_offset, s.n], dtype=torch.int64, device=dev) for s in stores],
+                       comm).cpu()                                            # [G * L, 2]: one collective
+    n_all = int((shards[:, 0] + shards[:, 1]).max())
+    blocks = sorted((r0, min(o + n, r0 + PAIR_BLOCK)) for o, n in shards.tolist() for r0 in range(o, o + n, PAIR_BLOCK))
+    counts = torch.zeros((n_all,), dtype=torch.int64, device=dev)
+    scores, idx = [], []
+    held = 0
+    tot = {"eps": 0.0, "blocks": len(blocks), "candidates": 0, "pairs": 0, "rerun_rows": 0, "passes": 0,
+           "phases_ms": {}}
+    for r0, r1 in blocks:
+        owner = [s for s in stores if s.index_offset <= r0 < s.index_offset + s.n]
+        if comm.world == 1:
+            q = owner[0].raw[r0 - owner[0].index_offset: r1 - owner[0].index_offset, :d_all]
+        else:
+            q = torch.zeros((r1 - r0, d_all), dtype=torch.float32, device=dev)
+            if owner:
+                q.copy_(owner[0].raw[r0 - owner[0].index_offset: r1 - owner[0].index_offset, :d_all])
+            q = comm.sum_(q)
+        views = [s._suffix(max(0, r0 - s.index_offset)) for s in stores]
+        after = torch.arange(r0, r1, dtype=torch.int64, device=dev)
+        st = None if stats is None else {}
+        res = _range_search(views, q, ms, weights, None, None, eps, st, comm, after=after, held=held)
+        counts[r0:r1] = res.offsets[1:] - res.offsets[:-1]
+        scores.append(res.scores)
+        idx.append(res.idx)
+        held += res.idx.numel()
+        if st is not None:
+            tot["eps"] = max(tot["eps"], st["eps"])
+            tot["candidates"] += int(round(st["candidates_per_query"] * (r1 - r0)))
+            tot["rerun_rows"] += st["rerun_rows"]
+            tot["passes"] += st["passes"]
+            for k, v in st["phases_ms"].items():
+                tot["phases_ms"][k] = tot["phases_ms"].get(k, 0.0) + v
+    off = torch.zeros((n_all + 1,), dtype=torch.int64, device=dev)
+    off[1:] = torch.cumsum(counts, 0)
+    out_s = torch.cat(scores) if scores else torch.empty((0,), dtype=torch.float64, device=dev)
+    out_i = torch.cat(idx) if idx else torch.empty((0,), dtype=torch.int64, device=dev)
+    if stats is not None:
+        tot["pairs"] = held
+        stats.update(tot)
+    return RangeResult(off, out_s, out_i)
 
 
 def search_norm_score(stores, queries, k, weights=None, comm=None, n_total=None, **kw):

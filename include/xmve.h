@@ -251,6 +251,15 @@ XMVE_API int xmve_range_select(const double* exact, const int32_t* cand_idx, con
                       int32_t cap, int64_t idx_offset, const int64_t* exclude, const double* min_score,
                       int64_t* counts, const int64_t* off, int64_t max_len, void* scratch,
                       double* out_score, int64_t* out_idx, void* stream);
+/* xmve_pair_select is xmve_range_select with one more condition, for the similar-pairs join of a corpus with itself
+ * (row r of the lists is the stored row after[r] used as a query): an entry matches only if, in addition, its global
+ * row cand_idx + idx_offset is greater than after[r] (after int64 [rows], DEVICE, never NULL).  This drops the row
+ * itself and every pair the join lists from the other side.  Count and fill apply the same test; arguments, modes and
+ * limits are those of xmve_range_select.  after[r] = -1 gives xmve_range_select's result. */
+XMVE_API int xmve_pair_select(const double* exact, const int32_t* cand_idx, const int32_t* cand_count, int64_t rows,
+                     int32_t cap, int64_t idx_offset, const int64_t* exclude, const double* min_score,
+                     int64_t* counts, const int64_t* off, int64_t max_len, void* scratch,
+                     double* out_score, int64_t* out_idx, const int64_t* after, void* stream);
 XMVE_API int xmve_range_merge(const double* score, const int64_t* idx, int32_t n_seg, const int64_t* seg_off,
                      int64_t rows, const int64_t* off, int64_t max_len, double* out_score, int64_t* out_idx,
                      void* stream);

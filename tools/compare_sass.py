@@ -3,9 +3,10 @@
     python tools/compare_sass.py OLD/score_tc.o NEW/score_tc.o
     python tools/compare_sass.py OLD/select.o NEW/select.o
 
-Kernels are matched by name with the anonymous-namespace hash removed and an added ``bool = false`` template argument
-dropped; instruction offsets and encodings are ignored.  Prints ``identical`` / ``DIFFERENT`` per kernel of the old
-build and lists the kernels only the new build has.
+Kernels are matched by their demangled name without the anonymous namespace, the parameter list and an added
+``bool = false`` template argument, so a kernel that gained a compile-time flag (and the parameters only its ``true``
+instantiation reads) is compared with its old self; instruction offsets and encodings are ignored.  Prints
+``identical`` / ``DIFFERENT`` per kernel of the old build and lists the kernels only the new build has.
 """
 import re
 import subprocess
@@ -32,14 +33,27 @@ def kernels(obj):
     return result
 
 
-def normalised(name):
-    name = re.sub(r"_GLOBAL__N__[0-9a-f]+_\d+_\w+?_cu_[0-9a-f]+", "", name)
-    return name.replace("ELb0EEE", "EEE")
+def normalised(names):
+    """{mangled name: key}: ``void xmve::<unnamed>::k<1, (bool)0>(...)`` -> ``xmve::k<1>``."""
+    out = subprocess.run(["cu++filt"], input="\n".join(names), capture_output=True, text=True, check=True).stdout
+    keys = {}
+    for name, dem in zip(names, out.splitlines()):
+        key = dem.replace("<unnamed>::", "").replace("(anonymous namespace)::", "")
+        key = key.replace("(bool)0", "false").replace("(bool)1", "true")
+        key = re.sub(r"\(\w+\)(-?\d+)", r"\1", key)                # (int)1 -> 1
+        key = re.sub(r"^void ", "", key)
+        key = re.sub(r"\(.*\)$", "", key)
+        key = key.replace(", false>", ">").replace("<false>", "")
+        keys[name] = key
+    assert len(set(keys.values())) == len(keys), "two kernels share a key"
+    return keys
 
 
 def main():
-    old = {normalised(k): v for k, v in kernels(sys.argv[1]).items()}
-    new = {normalised(k): v for k, v in kernels(sys.argv[2]).items()}
+    old, new = kernels(sys.argv[1]), kernels(sys.argv[2])
+    key_old, key_new = normalised(list(old)), normalised(list(new))
+    old = {key_old[k]: v for k, v in old.items()}
+    new = {key_new[k]: v for k, v in new.items()}
     different = 0
     for name in sorted(old):
         if name not in new:
