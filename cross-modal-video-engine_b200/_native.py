@@ -83,7 +83,7 @@ launch_count = 0
 _LAUNCHES = {"xmve_prepare_rows": 1, "xmve_score_store": 1, "xmve_score_filter": 1, "xmve_score_filter_labeled": 1, "xmve_mask_scores": 1,
              "xmve_row_kth": 1,
              "xmve_rescore": 1, "xmve_pilot_top": 1, "xmve_pilot_bound": 1, "xmve_eps_bound": 1, "xmve_merge_topk_packed": 1, "xmve_select_topk_i32": 1, "xmve_select_topk_i64": 1, "xmve_range_select": 1, "xmve_pair_select": 1, "xmve_range_merge": 1, "xmve_row_topj": 1, "xmve_normalize_f64": 1,
-             "xmve_score_f64": 1, "xmve_score_f64_fused": 1, "xmve_pairwise_f64": 1, "xmve_triplet_cost": 1, "xmve_gt_ranks": 1, "xmve_rank_metrics": 1, "xmve_list_ranks": 1, "xmve_count_before": 1, "xmve_count_band_f64": 1, "xmve_norm_score": 3, "xmve_fuse_accumulate": 1}
+             "xmve_score_f64": 1, "xmve_score_f64_fused": 1, "xmve_pairwise_f64": 1, "xmve_triplet_cost": 1, "xmve_gt_ranks": 2, "xmve_rank_metrics": 1, "xmve_list_ranks": 1, "xmve_count_before": 1, "xmve_count_band_f64": 1, "xmve_norm_score": 3, "xmve_fuse_accumulate": 1}
 
 
 def call(name, *args):

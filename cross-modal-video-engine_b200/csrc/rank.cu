@@ -99,7 +99,7 @@ gt_ranks_cols_kernel(const T* __restrict__ x, int64_t n_row, int64_t n_col, int6
         const int gi = gt_ids[e_lo + base + g];
         T gv = x[static_cast<int64_t>(gi) * ld + col];
         int gr = gi;
-        if (gv != gv) { gv = -inf; gr = -1; }           // NaN ground truth: nothing compares below it (rank 1)
+        if (gv != gv) { gv = -inf; gr = -1; }           // NaN ground truth: ranked by gt_ranks_nan_kernel afterwards
         int pos = ng;
         while (pos > 0 && (s_key[pos - 1][lane] > gv || (s_key[pos - 1][lane] == gv && s_row[pos - 1][lane] > gr))) {
           s_key[pos][lane] = s_key[pos - 1][lane];
@@ -156,6 +156,38 @@ gt_ranks_cols_kernel(const T* __restrict__ x, int64_t n_row, int64_t n_col, int6
     }
     __syncthreads();                                     // the sorted lists are rebuilt by the next pass
   }
+}
+
+// NaN ground truths.  NumPy's argsort (the reference's ranking) places every NaN after every number, NaNs in index
+// order, so an entry whose value is NaN has rank 1 + #{non-NaN elements of the line} + #{NaN elements m < g}.  The two
+// kernels above order numbers only; this pass runs after either of them and overwrites the ranks of those entries.
+// One warp per CSR entry: it leaves at once unless the entry's value is NaN, else its lanes scan the line.  Query q's
+// line is x[q * q_step + m * m_step], m < n_mem.
+template <typename T>
+__global__ void __launch_bounds__(256)
+gt_ranks_nan_kernel(const T* __restrict__ x, int64_t n_mem, int64_t q_step, int64_t m_step,
+                    const int64_t* __restrict__ gt_off, const int32_t* __restrict__ gt_ids, int64_t n_query,
+                    int64_t n_entries, int32_t* __restrict__ ranks) {
+  const int64_t e = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (e >= n_entries) return;
+  int64_t lo = 0, hi = n_query;                                 // owner: the last q with gt_off[q] <= e
+  while (hi - lo > 1) {
+    const int64_t mid = (lo + hi) >> 1;
+    if (gt_off[mid] <= e) lo = mid; else hi = mid;
+  }
+  const T* line = x + lo * q_step;
+  const int64_t g = gt_ids[e];
+  const T gv = line[g * m_step];
+  if (gv == gv) return;
+  int64_t c = 0;
+  for (int64_t m = lane; m < n_mem; m += 32) {
+    const T v = line[m * m_step];
+    c += (v == v || m < g) ? 1 : 0;
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
+  if (lane == 0) ranks[e] = static_cast<int32_t>(1 + c);
 }
 
 // One block per query: sort the query's ranks, reduce to best rank / AP, bump the global tallies.
@@ -244,10 +276,12 @@ template <typename T>
 __global__ void __launch_bounds__(256)
 minmax_kernel(const T* __restrict__ x, int64_t n_row, int64_t n_col, int64_t ld, unsigned long long* keys) {
   double mn = CUDART_INF, mx = -CUDART_INF;
+  bool nan = false;
   const int64_t total = n_row * n_col;
   for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < total;
        i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
     const double s = -static_cast<double>(x[(i / n_col) * ld + (i % n_col)]);   // score = -error
+    nan |= s != s;
     mn = fmin(mn, s);
     mx = fmax(mx, s);
   }
@@ -256,9 +290,13 @@ minmax_kernel(const T* __restrict__ x, int64_t n_row, int64_t n_col, int64_t ld,
     mn = fmin(mn, __shfl_xor_sync(0xffffffffu, mn, o));
     mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, o));
   }
+  nan = __any_sync(0xffffffffu, nan);
   if ((threadIdx.x & 31) == 0) {
-    atomicMin(&keys[0], dkey(mn));
-    atomicMax(&keys[1], dkey(mx));
+    // np.min / np.max are NaN if any element is, while fmin / fmax skip NaN.  A NaN's own key is no help: its sign is
+    // arbitrary (s = -x flips it) and a negative NaN's key sorts below -inf.  So the flag stores the extreme keys 0 and
+    // ~0, which both decode to NaN.
+    atomicMin(&keys[0], nan ? 0ull : dkey(mn));
+    atomicMax(&keys[1], nan ? ~0ull : dkey(mx));
   }
 }
 
@@ -268,7 +306,9 @@ __global__ void __launch_bounds__(256)
 norm_apply_kernel(const T* __restrict__ x, int64_t n_row, int64_t n_col, int64_t ld, T* __restrict__ out,
                   int64_t out_ld, const unsigned long long* __restrict__ keys) {
   const T mn = static_cast<T>(key_d(keys[0]));
-  const T mx = static_cast<T>(key_d(keys[1])) - mn;            // max(s - min) == max(s) - min (monotone)
+  // max(s - min) == max(s) - min (rounding is monotone).  With an infinite min NumPy's max(s - min) is NaN and this
+  // one may be inf, but then every s - min is +-inf or NaN and every output NaN either way.
+  const T mx = static_cast<T>(key_d(keys[1])) - mn;
   const int64_t total = n_row * n_col;
   for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < total;
        i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
@@ -293,6 +333,8 @@ extern "C" int xmve_gt_ranks(const void* errors, int dtype, int64_t n_row, int64
   XMVE_REQUIRE(n_entries >= 0 && max_gt >= 0, "gt_ranks: negative CSR sizes");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (n_entries == 0 || max_gt == 0) return XMVE_OK;
+  const int64_t nan_blocks = (n_entries + 7) / 8;               // gt_ranks_nan_kernel: one warp per entry
+  if (nan_blocks > 2147483647LL) return fail(XMVE_ERR_LIMIT, "gt_ranks: too many entries");
   if (axis == 0) {
     const int G = max_gt == 1 ? 1 : 8;
     const int n_groups = (max_gt + G - 1) / G;
@@ -321,7 +363,14 @@ extern "C" int xmve_gt_ranks(const void* errors, int dtype, int64_t n_row, int64
       gt_ranks_cols_kernel<double><<<grid, 256, 0, st>>>(static_cast<const double*>(errors), n_row, n_col, ld, gt_off,
                                                          gt_ids, max_gt, rows_per_slice, ranks);
   }
-  return launch_status("gt_ranks kernel");
+  const int64_t n_mem = axis == 0 ? n_col : n_row, q_step = axis == 0 ? ld : 1, m_step = axis == 0 ? 1 : ld;
+  if (dtype == XMVE_F32)
+    gt_ranks_nan_kernel<float><<<static_cast<unsigned>(nan_blocks), 256, 0, st>>>(
+        static_cast<const float*>(errors), n_mem, q_step, m_step, gt_off, gt_ids, n_query, n_entries, ranks);
+  else
+    gt_ranks_nan_kernel<double><<<static_cast<unsigned>(nan_blocks), 256, 0, st>>>(
+        static_cast<const double*>(errors), n_mem, q_step, m_step, gt_off, gt_ids, n_query, n_entries, ranks);
+  return launch_status("gt_ranks kernels");
 }
 
 namespace xmve {

@@ -14,7 +14,10 @@ host arithmetic is the final ``100.0 * count / n``, ``sum / n`` and ``np.mean`` 
 written exactly as the reference writes them so the returned floats are identical.
 
 Ties: the reference sorts with NumPy's default (unstable) argsort, so the order of exactly equal
-scores is unspecified there; the kernels use the stable order (lower index first).
+scores is unspecified there; the kernels use the stable order (lower index first), i.e. the ranks are
+those of ``np.argsort(line, kind="stable")``.  NaN is ordered as NumPy orders it: after every number,
+NaNs by index.  A NaN ground truth (a zero embedding normalised without epsilon) is thus ranked behind
+every number, not first, and a NaN element never precedes a number.
 """
 from __future__ import annotations
 

@@ -315,7 +315,9 @@ XMVE_API int xmve_triplet_cost(const double* scores, int64_t n, int64_t ld, doub
  * axis = 0: query i is ROW i, memories are columns   (eval_q2m(errors, t2v_gt), util/metrics.py:124-157)
  * axis = 1: query i is COLUMN i, memories are rows   (eval_q2m(errors.T, v2t_gt), validate.py:22)
  * ranks[e] (1-based, one per CSR entry) = 1 + #{m : x[m] < x[g]} + #{m < g : x[m] == x[g]}, the
- * position of g in a stable ascending argsort.  n_entries = gt_off[n_query] and max_gt = the largest
+ * position of g in a stable ascending argsort (np.argsort(line, kind="stable")).  As there, NaN sorts after every
+ * number, NaNs in index order: a NaN x[g] has rank 1 + #{m : x[m] is not NaN} + #{m < g : x[m] is NaN}, and a NaN
+ * element never precedes a number.  -0.0 and +0.0 are equal.  n_entries = gt_off[n_query] and max_gt = the largest
  * number of entries of any query are passed by the caller (it built the CSR) to avoid a device sync.
  */
 XMVE_API int xmve_gt_ranks(const void* errors, int dtype, int64_t n_row, int64_t n_col, int64_t ld, int axis,
@@ -363,7 +365,10 @@ XMVE_API int xmve_count_band_f64(const double* scores, int64_t n_entries, int64_
 
 /* ---- norm_score (LINAS-engine/validate.py:7-11) -------------------------------------------------
  * minmax[0] = min(-E), minmax[1] = max(-E - min) over the whole matrix (two launches inside);
- * xmve_norm_score_apply writes out = -((-E - min) / max) with the reference's operation order.
+ * then out = -((-E - min) / max) with the reference's operation order, in the input's precision.  NumPy semantics on
+ * non-finite input: a NaN anywhere makes min, max and every output NaN; an infinite min (an error of +inf, or all
+ * errors -inf) makes every output NaN; an error of -inf alone makes max = inf, so that element's output is NaN and
+ * every other one -0.0; a constant matrix gives 0 / 0 = NaN.  minmax_scratch: DEVICE, 2 doubles.
  */
 XMVE_API int xmve_norm_score(const void* errors, int dtype, int64_t n_row, int64_t n_col, int64_t ld,
                     void* out, int64_t out_ld, double* minmax_scratch, void* stream);
