@@ -19,15 +19,14 @@ from __future__ import annotations
 import ctypes as C
 import math
 import os
+import struct
 
 import torch
 
 from . import _native as N
 
-#: a-priori bound on |bf16-operand score - exact cosine| per unit of fusion weight: bf16 keeps 8 significant bits,
-#: so rounding moves a vector by at most 2^-8 of its norm and a product of two unit vectors by at most 2 * 2^-8
-#: (Cauchy-Schwarz); plus fp32 accumulation slack.  Used only when no measured residuals are available
-#: (search(eps=...) callers, NaN rows); the search itself uses :func:`measured_eps` (typically 3.5e-3 - 4e-3).
+#: former fallback bound per unit of fusion weight (2 * 2^-8 plus accumulation slack for rows up to K ~ 2800); it stays
+#: the floor of :func:`eps_fallback`, which raises it to the a-priori bound where the accumulation term needs more
 EPS_X1 = 8.5e-3
 SMALL_NV = 16384
 #: multiples of eps subtracted from the sampled threshold kth(sample, j) -- see :func:`thr_margin`.  Round 1 always
@@ -544,15 +543,36 @@ def measured_eps(dq, dv, wts, n_space, k_len):
     ``<Q,V> - <Qb,Vb> = <Q-Qb, V> + <Qb, V-Vb>``, so by Cauchy-Schwarz the operand rounding costs at most
     ``dq * |V| + |Qb| * dv`` with ``dq = max_q |Q-Qb|``, ``dv = max_v |V-Vb|`` (K1 measures both), ``|V| = sqrt(S)``
     and ``|Qb| <= sqrt(sum w^2) + dq``.  The bf16 x bf16 products are exact in fp32; accumulating ``k_len`` of them
-    in fp32 (with truncation at worst) costs at most ``k_len * 2^-22 * |Qb| * |Vb|``.  The a-priori worst case is
-    2 * 2^-8 per unit weight (``EPS_X1``); Gaussian-like rows measure ``dq, dv ~ 1.7e-3`` of the norm, i.e. about half.
+    in fp32 (with truncation at worst) costs at most ``k_len * 2^-22 * |Qb| * |Vb|``.  Without measurements the bound
+    is :func:`eps_fallback`; Gaussian-like rows measure ``dq, dv ~ 1.7e-3`` of the norm, about half the worst case.
     """
     qn = math.sqrt(sum(w * w for w in wts)) + dq
     vn = math.sqrt(n_space) * (1.0 + 2.0 ** -8)
     e = dq * vn + qn * dv + k_len * 2.0 ** -22 * qn * vn + 1e-6
     if not math.isfinite(e) or e <= 0.0:                   # NaN rows (zero vectors under 'plain' normalisation)
-        return EPS_X1 * max(1.0, sum(abs(w) for w in wts))
+        return eps_fallback(wts, n_space, k_len)
     return e
+
+
+def eps_fallback(wts, n_space, k_len):
+    """Bound on |tensor-core score - exact score| that needs no measured residual; used when a residual is NaN.
+
+    bf16 keeps 8 significant bits, so rounding moves each space's operand by at most ``u = 2^-8`` of its norm: the
+    product of space ``s`` moves by at most ``|w_s| * (2u + u^2)`` (Cauchy-Schwarz, both sides).  Accumulating
+    ``k_len`` products in fp32 adds ``k_len * 2^-22 * |Qb| * |Vb|`` with ``|Qb| <= |w| (1 + u)`` and
+    ``|Vb| <= sqrt(S) (1 + u)``; ``1e-6`` covers the fp32 rounding of the operand before its bf16 rounding.  The
+    accumulation term grows with ``k_len``, so no constant per unit weight bounds every layout: ``EPS_X1`` alone fell
+    below it from K = 2816 on.  Returns the larger of ``EPS_X1 * max(1, sum |w|)`` (unchanged where it was sound) and
+    that bound, as the smallest fp32 value at or above it, since the device takes it as a float."""
+    u = 2.0 ** -8
+    e = (sum(abs(w) for w in wts) * (2 * u + u * u)
+         + k_len * 2.0 ** -22 * math.sqrt(sum(w * w for w in wts)) * (1 + u) * math.sqrt(n_space) * (1 + u) + 1e-6)
+    e = max(e, EPS_X1 * max(1.0, sum(abs(w) for w in wts)))
+    e *= 1 + 1e-12                                          # the float64 evaluation above rounds either way
+    f = struct.unpack("<f", struct.pack("<f", e))[0]         # nearest fp32
+    if f < e:
+        f = struct.unpack("<f", struct.pack("<I", struct.unpack("<I", struct.pack("<f", f))[0] + 1))[0]
+    return f
 
 
 class _Phases:
@@ -616,7 +636,7 @@ def _eps_device(q_res, dv2, wts, n_space, k_len):
     """:func:`measured_eps` on the device: fp32 ``[1]`` tensor (no host round trip)."""
     out = torch.empty((1,), dtype=torch.float32, device=q_res.device)
     N.call("xmve_eps_bound", N.ptr(q_res), n_space, q_res.shape[1], N.ptr(dv2), math.sqrt(sum(w * w for w in wts)),
-           int(k_len), EPS_X1 * max(1.0, sum(abs(w) for w in wts)), N.ptr(out), N.stream_ptr())
+           int(k_len), eps_fallback(wts, n_space, k_len), N.ptr(out), N.stream_ptr())
     return out
 
 
@@ -1166,7 +1186,7 @@ def _search_shards(stores, queries, k, weights, exclude, eps, small_nv, stats, c
         a_op, q_raw, q_norm, q_res, nq = ref.prepare_queries(queries, wts)
         excl = None
         if exclude is not None:
-            excl = torch.as_tensor(exclude, dtype=torch.int64).to(dev)
+            excl = torch.as_tensor(exclude, dtype=torch.int64).to(dev).contiguous()   # the kernels read excl[q]
         masks = n_elig = None
         if label_mask is not None:
             masks = _label_masks(label_mask, nq, dev)
@@ -1497,7 +1517,7 @@ def _range_setup(stores, queries, min_score, weights, exclude, label_mask, eps, 
     ms = _min_scores(min_score, nq, dev)
     excl = None
     if exclude is not None:
-        excl = torch.as_tensor(exclude, dtype=torch.int64).reshape(-1).to(dev)
+        excl = torch.as_tensor(exclude, dtype=torch.int64).reshape(-1).to(dev).contiguous()
         if excl.numel() != nq:
             raise ValueError("exclude: expected one row (or -1) per query (%d), got %d" % (nq, excl.numel()))
     masks = None if label_mask is None else _label_masks(label_mask, nq, dev)

@@ -559,6 +559,12 @@ def test_eps_bound_matches_the_host_formula(N):
     assert want <= got <= want * (1 + 1e-6)                                                   # rounded UP to float
     q_res[1, 17] = float("nan")                                                               # a zero row: a-priori bound
     assert float(engine._eps_device(q_res, dv2, wts, 2, 2048)) == pytest.approx(engine.EPS_X1, rel=1e-6)
+    assert float(engine._eps_device(q_res, dv2, wts, 2, 2048)) == engine.eps_fallback(wts, 2, 2048)
+    assert engine.measured_eps(float("nan"), 1e-3, wts, 2, 2048) == engine.eps_fallback(wts, 2, 2048)
+    q_res[1, 17] = 0.0
+    dv2[0] = float("nan")                                                                     # a zero corpus row
+    e_long = float(engine._eps_device(q_res, dv2, wts, 2, 6016))                             # past the constant
+    assert e_long == engine.eps_fallback(wts, 2, 6016) > engine.EPS_X1
 
 
 def test_select_topk_many_rows_use_the_small_sort(N):

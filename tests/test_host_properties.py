@@ -63,3 +63,39 @@ def test_measured_eps_is_monotone_and_covers_the_cauchy_schwarz_terms(dq, dv, wt
     assert engine.measured_eps(dq * 1.5, dv, wts, len(wts), k_len) > e
     assert engine.measured_eps(dq, dv * 1.5, wts, len(wts), k_len) > e
     assert engine.measured_eps(dq, dv, wts, len(wts), 2 * k_len) > e
+
+
+def _apriori_bound(wts, dims):
+    """|bf16-operand score - exact score| without measured residuals: each space's product moves by at most
+    |w_s| (2u + u^2) under rounding to bf16 (u = 2^-8), the fp32 accumulation of K products by at most
+    K 2^-22 |Qb| |Vb| with |Qb| <= |w| (1 + u), |Vb| <= sqrt(S) (1 + u), plus 1e-6 for the fp32 rounding of the operand."""
+    u = 2.0 ** -8
+    k_len = sum(-(-d // 64) * 64 for d in dims)
+    w_norm = math.sqrt(sum(w * w for w in wts))
+    return (sum(abs(w) for w in wts) * (2 * u + u * u)
+            + k_len * 2.0 ** -22 * w_norm * (1 + u) * math.sqrt(len(dims)) * (1 + u) + 1e-6), k_len
+
+
+@settings(max_examples=300, deadline=None)
+@given(st.lists(st.tuples(st.integers(1, 6000), st.floats(0.05, 2.0), st.booleans()), min_size=1, max_size=4)
+       .filter(lambda sp: sum(d for d, _, _ in sp) <= 6000))
+def test_fallback_eps_covers_the_a_priori_bound(spaces):
+    """A NaN residual (a zero row under 'plain') makes eps the fallback bound: it must cover the a-priori bound for every
+    layout the store accepts (up to 6000 raw columns), whatever K, and reach the device as a float without rounding
+    down.  Where 8.5e-3 per unit weight already covered it, the fallback stays that constant."""
+    import numpy as np
+    dims = [d for d, _, _ in spaces]
+    wts = [-w if neg else w for _, w, neg in spaces]
+    bound, k_len = _apriori_bound(wts, dims)
+    e = engine.measured_eps(float("nan"), 1e-3, wts, len(dims), k_len)
+    assert e >= bound
+    assert e <= max(bound, engine.EPS_X1 * max(1.0, sum(abs(w) for w in wts))) * (1 + 1e-6)
+    assert float(np.float32(e)) == e
+
+
+def test_fallback_eps_for_long_rows():
+    """The layouts where a constant 8.5e-3 per unit weight fell below the bound."""
+    for dims, wts in (((2048,), (1.0,)), ((2816,), (1.0,)), ((6000,), (1.0,)), ((3000, 3000), (1.0, 1.0)),
+                      ((3000, 2000), (0.5, 0.5)), ((1536, 512), (0.6, -0.4))):
+        bound, k_len = _apriori_bound(wts, dims)
+        assert engine.measured_eps(float("nan"), float("nan"), wts, len(dims), k_len) >= bound, (dims, wts)
