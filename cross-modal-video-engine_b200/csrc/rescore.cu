@@ -549,6 +549,9 @@ extern "C" int xmve_rescore(const float* q_raw, int64_t nq, int64_t q_ld, const 
   if (dev < 0) return fail(XMVE_ERR_DEVICE, "rescore: no current device");
   if (resident[dev][1] == 0 || resident[dev][0] != static_cast<int>(dyn_smem)) {
     int per_sm = 0;
+    // from about 5 000 dims the query row and the static lists exceed the 48 KB a launch gets without opting in
+    XMVE_CUDA(cudaFuncSetAttribute(rescore_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                   static_cast<int>(dyn_smem)));
     XMVE_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, rescore_kernel, RS_WARPS * 32, dyn_smem));
     const int sms = sm_count();
     if (per_sm <= 0 || sms <= 0) return fail(XMVE_ERR_DEVICE, "rescore: cannot query the occupancy");

@@ -29,6 +29,8 @@ from . import _native as N
 #: the floor of :func:`eps_fallback`, which raises it to the a-priori bound where the accumulation term needs more
 EPS_X1 = 8.5e-3
 SMALL_NV = 16384
+#: small-corpus path: the fp64 score matrices of one query batch (two [batch, n] matrices) take at most this many bytes
+SMALL_BATCH_BYTES = 1 << 30
 #: multiples of eps subtracted from the sampled threshold kth(sample, j) -- see :func:`thr_margin`.  Round 1 always
 #: used 2: "the k-th best exact score is at least kth_approx - eps, a row's approximate score at most eps above its
 #: exact one".  But j already carries a 5.5-sigma sampling slack (plan()): the j-th largest of the sample sits near
@@ -382,35 +384,63 @@ class CorpusStore:
         return (C.c_double * len(wts))(*[float(w) for w in wts])
 
     def _exact_small(self, q_raw, q_norm, nq, k, wts, excl, label_mask=None):
-        """fp64 score matrix + bitonic top-k (corpora up to ``small_nv`` rows); ``label_mask``: ineligible rows are
-        set to -inf first, and the selection skips them."""
+        """Top-``k`` rows of this store per query by the DMMA fp64 score ``sum_s w_s * <normalize(q_s),
+        normalize(v_s)>`` (the approximate score of the small-corpus path, within :func:`small_delta` of the rescore
+        kernel's) -> ``(scores fp64 [nq, k], global rows int64 [nq, k])``, -inf / -1 padded.  The score matrix is
+        formed ``SMALL_BATCH_BYTES`` at a time.  ``label_mask``: ineligible rows are set to -inf first, and the
+        selection skips them, as it skips ``excl``.  The list is the exact top-``k``: with 512 rows or more in a launch
+        the selection sorts at most ``max(2048, 4k)`` entries per row and cuts float ties beyond that; the rows it
+        reports as cut are selected again, 511 rows per launch, with the full 16 384-entry sort (stores of more than
+        16 384 rows, with a ``small_nv`` above the default, could still be cut by more float ties than that)."""
         dev, st = self.device, N.stream_ptr()
-        acc = None
-        o = 0
-        for s, d in enumerate(self.dims):
-            qn = torch.empty((nq, d), dtype=torch.float64, device=dev)
-            vn = torch.empty((self.n, d), dtype=torch.float64, device=dev)
-            qs, vs = q_raw[:nq, o:o + d], self.raw[:self.n, o:o + d]
-            N.call("xmve_normalize_f64", N.ptr(qs), N.F32, nq, d, q_raw.stride(0), N.ptr(qn), d, self.norm_mode, st)
-            N.call("xmve_normalize_f64", N.ptr(vs), N.F32, self.n, d, self.raw.stride(0), N.ptr(vn), d,
-                   self.norm_mode, st)
-            sc = torch.empty((nq, self.n), dtype=torch.float64, device=dev)
-            for q0 in range(0, nq, 1 << 21):
-                q1 = min(nq, q0 + (1 << 21))
-                N.call("xmve_score_f64", N.ptr(qn[q0:]), q1 - q0, d, N.ptr(vn), self.n, d, d, float(wts[s]),
-                       N.ptr(sc[q0:]), self.n, st)
-            acc = sc if acc is None else acc.add_(sc)
-            o += d
-        if label_mask is not None:
-            N.call("xmve_mask_scores", N.ptr(acc), N.F64, nq, self.n, acc.stride(0), N.ptr(self._ensure_labels()), 1,
-                   N.ptr(label_mask), st)
         kk = min(k, self.n)
+        vn, o = [], 0
+        for d in self.dims:
+            v = torch.empty((self.n, d), dtype=torch.float64, device=dev)
+            N.call("xmve_normalize_f64", N.ptr(self.raw[:, o:o + d]), N.F32, self.n, d, self.raw.stride(0), N.ptr(v), d,
+                   self.norm_mode, st)
+            vn.append(v)
+            o += d
         out_s = torch.full((nq, k), float("-inf"), dtype=torch.float64, device=dev)
         out_i = torch.full((nq, k), -1, dtype=torch.int64, device=dev)
         s_ = torch.empty((nq, kk), dtype=torch.float64, device=dev)
         i_ = torch.empty((nq, kk), dtype=torch.int64, device=dev)
-        N.call("xmve_select_topk_i32", N.ptr(acc), None, nq, self.n, None, self.index_offset, N.ptr(excl), kk,
-               None, 0.0, None, None, N.ptr(s_), N.ptr(i_), None, None, None, None, st)
+        exact = torch.empty((nq,), dtype=torch.int32, device=dev)
+        batch = max(1, min(1 << 21, SMALL_BATCH_BYTES // (16 * self.n)))      # two fp64 [batch, n] matrices
+        cut_free = self.n <= max(2048, _pow2(4 * kk))                       # no row can hold more than the sort
+        for q0 in range(0, nq, batch):
+            q1 = min(nq, q0 + batch)
+            acc, o = None, 0
+            for s, d in enumerate(self.dims):
+                qn = torch.empty((q1 - q0, d), dtype=torch.float64, device=dev)
+                N.call("xmve_normalize_f64", N.ptr(q_raw[q0:q1, o:o + d]), N.F32, q1 - q0, d, q_raw.stride(0), N.ptr(qn),
+                       d, self.norm_mode, st)
+                sc = torch.empty((q1 - q0, self.n), dtype=torch.float64, device=dev)
+                N.call("xmve_score_f64", N.ptr(qn), q1 - q0, d, N.ptr(vn[s]), self.n, d, d, float(wts[s]), N.ptr(sc),
+                       self.n, st)
+                acc = sc if acc is None else acc.add_(sc)
+                o += d
+            if label_mask is not None:
+                N.call("xmve_mask_scores", N.ptr(acc), N.F64, q1 - q0, self.n, acc.stride(0),
+                       N.ptr(self._ensure_labels()), 1, N.ptr(label_mask[q0:q1]), st)
+            ex = N.ptr(excl[q0:q1]) if excl is not None else None
+            N.call("xmve_select_topk_i32", N.ptr(acc), None, q1 - q0, self.n, None, self.index_offset, ex, kk, None,
+                   0.0, None, None, N.ptr(s_[q0:]), N.ptr(i_[q0:]), None, None if cut_free else N.ptr(exact[q0:q1]),
+                   None, None, st)
+            if not cut_free and q1 - q0 >= 512:
+                # the rows whose ties were cut again, in launches of fewer than 512 rows; the others get no entries
+                cnt = torch.where(exact[q0:q1] == 0, self.n, 0).to(torch.int32)
+                s2 = torch.empty((q1 - q0, kk), dtype=torch.float64, device=dev)
+                i2 = torch.empty((q1 - q0, kk), dtype=torch.int64, device=dev)
+                for r0 in range(0, q1 - q0, SELECT_RERUN_ROWS):
+                    r1 = min(q1 - q0, r0 + SELECT_RERUN_ROWS)
+                    N.call("xmve_select_topk_i32", N.ptr(acc[r0:]), None, r1 - r0, self.n, N.ptr(cnt[r0:]),
+                           self.index_offset, N.ptr(excl[q0 + r0:q0 + r1]) if excl is not None else None, kk, None, 0.0,
+                           None, None, N.ptr(s2[r0:]), N.ptr(i2[r0:]), None, None, None, None, st)
+                redo = (exact[q0:q1] == 0).unsqueeze(1)
+                s_[q0:q1] = torch.where(redo, s2, s_[q0:q1])
+                i_[q0:q1] = torch.where(redo, i2, i_[q0:q1])
+            del acc, sc
         out_s[:, :kk] = s_
         out_i[:, :kk] = i_
         return out_s, out_i
@@ -573,6 +603,39 @@ def eps_fallback(wts, n_space, k_len):
     if f < e:
         f = struct.unpack("<f", struct.pack("<I", struct.unpack("<I", struct.pack("<f", f))[0] + 1))[0]
     return f
+
+
+def small_delta(wts, dims):
+    """Bound on |DMMA score - rescore score| for one (query, row) pair on the small-corpus path, as the smallest fp32
+    value at or above it.
+
+    Both are fp64 statements of ``sum_s w_s * c_s`` with ``c_s = <a, b>``, ``a = q / |q|``, ``b = v / |v|`` (fp32
+    rows, so ``sum |a_i b_i| <= 1``); ``u = 2^-53`` and ``g_d = d u / (1 - d u)`` bounds ``d`` products and sums.
+
+    - rescore (``xmve_rescore``): ``<q, v>`` with exact products, ``|error| <= g_d |q| |v|``; the norms carry ``g_d / 2
+      + u`` each (sum of squares, square root), their product and the quotient one ``u`` each: ``|r_s - c_s| <= 2 g_d
+      + 4 u``.
+    - DMMA (``xmve_normalize_f64`` + ``xmve_score_f64``): every ``a_i``, ``b_i`` carries ``g_d / 2 + 2 u`` (norm and
+      division), which moves the dot product by at most ``g_d + 4 u``, and the dot product itself costs ``g_d``:
+      ``|m_s - c_s| <= 2 g_d + 4 u``.
+    - each side multiplies by ``w_s`` and adds the ``S`` spaces: ``g_S sum |w_s|`` per side.
+
+    Hence ``|DMMA - rescore| <= u sum_s |w_s| (4 d_s + 8 + 2 S)`` up to terms of order ``d u^2``, which the factor
+    ``1 + 2^-20`` covers.  The bound holds at any row scale the fp32 inputs allow (the squares of fp32 values neither
+    overflow nor underflow in fp64) and under both norm modes (``max(|x|, 1e-12)`` is exact)."""
+    u = 2.0 ** -53
+    s = len(dims)
+    e = u * sum(abs(w) * (4 * d + 8 + 2 * s) for w, d in zip(wts, dims)) * (1 + 2.0 ** -20)
+    f = struct.unpack("<f", struct.pack("<f", e))[0]
+    if f < e:
+        f = struct.unpack("<f", struct.pack("<I", struct.unpack("<I", struct.pack("<f", f))[0] + 1))[0]
+    return f
+
+
+def _float_above(x):
+    """fp64 tensor -> the smallest fp32 values strictly above it."""
+    f = x.float()
+    return torch.where(f.double() <= x, torch.nextafter(f, torch.full_like(f, float("inf"))), f)
 
 
 class _Phases:
@@ -978,6 +1041,97 @@ class _Search:
                               "or candidate capacity; heavy score ties?)" % int(bad.numel()))
 
 
+class _SmallSearch(_Search):
+    """State of one search over a corpus of at most ``small_nv`` rows.  Steps 2-4 of :func:`search_shards` become:
+    every store forms its fp64 score matrix with the DMMA kernel (:meth:`CorpusStore._exact_small`), keeps its
+    ``cap`` best rows by that score, and the rescore kernel gives them their exact scores -- the scores every other
+    API returns.  Step 5 is the filtered path's selection and merge, certified with the threshold ``thr`` (strictly
+    above every left-out row's DMMA score) and ``eps = small_delta``: a row outside the lists scores below
+    ``thr + eps <= kth``.  Step 6 re-runs the rows without a certificate with four times the lists, selecting in
+    batches of ``SELECT_RERUN_ROWS`` rows; lists that hold a whole store are complete."""
+
+    def __init__(self, stores, comm, k, k_eff, wts, excl, eps_t, q_raw, q_norm, nq, out_s, out_i, stats, ph, masks):
+        self.stores, self.comm, self.k, self.k_eff, self.wts = stores, comm, k, k_eff, wts
+        self.excl, self.eps_t, self.masks = excl, eps_t, masks
+        self.q_raw, self.q_norm, self.nq, self.thr = q_raw, q_norm, nq, None
+        self.out_s, self.out_i, self.stats, self.ph = out_s, out_i, stats, ph
+        self.ref = stores[0]
+        self.dev = self.ref.device
+        self.live = [s for s in stores if s.n]
+        self.n_shards = len(stores) * comm.world
+        self.solo = self.n_shards == 1
+        self.n_shard_max = max(s.n for s in self.live) if self.live else 1
+        self.cap = 2 * k_eff + 32                             # candidates per row and store: the k best and slack
+        self.pending = None
+
+    def run_pass(self, rows):
+        dev, k_eff = self.dev, self.k_eff
+        if rows is None:
+            q_sub, qn_sub, ex_sub, mk, n_sub = self.q_raw, self.q_norm, self.excl, self.masks, self.nq
+        else:
+            n_sub = rows.numel()
+            q_sub = self.q_raw[rows].contiguous()
+            qn_sub = self.q_norm[:, rows].contiguous()
+            ex_sub = self.excl[rows].contiguous() if self.excl is not None else None
+            mk = self.masks[rows].contiguous() if self.masks is not None else None
+        width = max(min(self.cap, self.n_shard_max), k_eff)
+        kw = {} if mk is None else {"label_mask": mk}
+        ninf = torch.full((n_sub,), float("-inf"), dtype=torch.float32, device=dev)
+        self.ph.mark("alloc")
+        cands, thr = [], ninf
+        for s in self.live:
+            m = min(self.cap, s.n)
+            top_s, top_i = s._exact_small(q_sub, qn_sub, n_sub, m, self.wts, ex_sub, **kw)
+            # every row left out scores at most the m-th DMMA score: thr lies strictly above it (-inf when the list
+            # holds every valid row of the store)
+            t = torch.where(top_i[:, -1] >= 0, _float_above(top_s[:, -1]), ninf) if m < s.n else ninf
+            thr = torch.maximum(thr, t)
+            c_s = torch.full((n_sub, width), float("-inf"), dtype=torch.float32, device=dev)
+            c_i = torch.zeros((n_sub, width), dtype=torch.int32, device=dev)
+            c_s[:, :m] = top_s.float()
+            c_i[:, :m] = torch.where(top_i < 0, torch.zeros_like(top_i), top_i - s.index_offset).to(torch.int32)
+            cands.append(((top_i >= 0).sum(1).to(torch.int32), c_s, c_i))
+        if self.comm.world > 1:
+            thr = self.comm.max_(thr)
+        self.ph.mark("score_f64")
+        exacts = [s._rescore(q_sub, qn_sub, n_sub, self.wts, c, None) for s, c in zip(self.live, cands)]
+        self.ph.mark("rescore")
+        n_bad = torch.zeros((1,), dtype=torch.int32, device=dev)
+        batch = n_sub if rows is None else SELECT_RERUN_ROWS
+        parts = [self._select_rows(r0, min(n_sub, r0 + batch), cands, exacts, ex_sub, thr, thr, n_bad)
+                 for r0 in range(0, n_sub, batch)]
+        s_, i_, cert, thr_next = (torch.cat([p[j] for p in parts]) for j in range(4))
+        # a row whose lists hold every valid row of every store is exact however short (fewer than k eligible rows,
+        # or k >= n with an exclusion); the selection cannot certify it, as its k-th entry is padding
+        short = (thr == float("-inf")) & (i_[:, -1] == -1)
+        cert = torch.where(short, torch.ones_like(cert), cert)
+        n_bad.copy_((cert == 0).sum().reshape(1))
+        self.ph.mark("select_merge")
+        if self.stats is not None and rows is None:
+            self.stats["eps"] = float(self.eps_t)
+            self.stats["cap"] = self.cap
+        return s_, i_, cert, thr_next, None, n_bad, thr
+
+    def _rerun(self):
+        cert = self._last[0]
+        rows = None
+        for attempt in range(12):
+            bad = torch.nonzero(cert == 0).flatten()            # device -> host sync (identical on every rank)
+            if bad.numel() == 0:
+                return
+            rows = bad if rows is None else rows[bad]
+            self.cap = min(4 * self.cap, self.n_shard_max, 16384)   # (the selection sorts at most 16 384 entries)
+            if self.stats is not None:
+                self.stats["reruns"] = self.stats.get("reruns", 0) + 1
+                self.stats["rerun_rows"] = self.stats.get("rerun_rows", 0) + int(rows.numel())
+            s_, i_, cert = self.run_pass(rows)[:3]
+            self.out_s[rows, :self.k_eff] = s_
+            self.out_i[rows, :self.k_eff] = i_
+        if bool((cert == 0).any()):
+            raise N.XmveError("search: %d row(s) could not be certified after 12 passes (heavy score ties?)"
+                              % int((cert == 0).sum()))
+
+
 class GraphSearch:
     """A search of fixed shape captured ONCE into a CUDA graph and replayed per query batch.
 
@@ -1122,7 +1276,9 @@ def search_shards(stores, queries, k, weights=None, exclude=None, eps=None, smal
        number is the only thing the host reads back, asynchronously: with ``defer=True`` the function returns a
        :class:`PendingSearch` right after enqueueing steps 1-5 and ``.result()`` does step 6.
 
-    Corpora of at most ``small_nv`` rows skip 2-4: every shard forms its fp64 score matrix directly.
+    Corpora of at most ``small_nv`` rows replace 2-4 (:class:`_SmallSearch`): every shard forms its fp64 score matrix
+    with the DMMA kernel in batches of queries, and its best rows by that score are rescored by the rescore kernel;
+    steps 5-6 certify them with the bound :func:`small_delta` on the difference of the two fp64 scores.
     With one shard and one rank no gather happens and the certificate comes from the local selection kernel.
 
     ``head_stream`` (a ``torch.cuda.Stream``; use with ``defer=True``): steps 1-2 are enqueued on that stream and the
@@ -1200,20 +1356,11 @@ def _search_shards(stores, queries, k, weights, exclude, eps, small_nv, stats, c
     out_i = torch.full((nq, k), -1, dtype=torch.int64, device=dev)
 
     if n_total <= small_nv:
-        kw = {} if masks is None else {"label_mask": masks}
-        parts = [s._exact_small(q_raw, q_norm, nq, k_eff, wts, excl, **kw) for s in stores if s.n]
-        if not parts:
-            parts = [(torch.full((nq, k_eff), float("-inf"), dtype=torch.float64, device=dev),
-                      torch.full((nq, k_eff), -1, dtype=torch.int64, device=dev))]
-        if solo:
-            s_, i_ = parts[0]
-        else:
-            s_, i_ = _merge(_union([p[0] for p in parts], comm), _union([p[1] for p in parts], comm), k_eff)
-        out_s[:, :k_eff] = s_
-        out_i[:, :k_eff] = i_
-        return PendingSearch.ready(out_s, out_i)
+        eps_t = torch.full((1,), small_delta(wts, ref.dims), dtype=torch.float32, device=dev)
+        return _first_pass(_SmallSearch(stores, comm, k, k_eff, wts, excl, eps_t, q_raw, q_norm, nq, out_s, out_i,
+                                        stats, ph, masks), in_graph, flag_host)
 
-    kk = k_eff + (1 if excl is not None else 0)               # one extra in case the excluded row is among them
+    kk = k_eff + (1 if excl is not None else 0)              # one extra in case the excluded row is among them
     pl = plan(kk, n_total)
     with _head_on(head_stream):
         eps_t, thr = _threshold(stores, comm, solo, wts, eps, pl, a_op, q_res, nq, ph, masks)
@@ -1225,12 +1372,16 @@ def _search_shards(stores, queries, k, weights, exclude, eps, small_nv, stats, c
         for t in (a_op, q_raw, q_norm, q_res, eps_t, thr, excl, masks, n_elig):
             if t is not None:
                 t.record_stream(main)
-    search = _Search(stores, comm, k, k_eff, kk, wts, excl, eps_t, pl, a_op, q_raw, q_norm, nq, thr, out_s, out_i,
-                     stats, ph, masks, n_elig)
+    return _first_pass(_Search(stores, comm, k, k_eff, kk, wts, excl, eps_t, pl, a_op, q_raw, q_norm, nq, thr, out_s,
+                               out_i, stats, ph, masks, n_elig), in_graph, flag_host)
+
+
+def _first_pass(search, in_graph, flag_host):
+    """Enqueue the first pass of ``search`` -> its :class:`PendingSearch`."""
     search.first_pass(in_graph, flag_host)
     pending = PendingSearch(search)
     pending._ctx_template = search
-    pending.scores, pending.idx = out_s, out_i
+    pending.scores, pending.idx = search.out_s, search.out_i
     return pending
 
 

@@ -344,7 +344,7 @@ def test_two_stores_equal_one(X):
 @pytest.mark.parametrize("k", [10, 1000])
 def test_range_search_holds_the_top_k(X, k):
     """r[q] = the k-th score search returns: range_search(q, r) starts with exactly the top-k list; any further entry
-    scores exactly r[q].  Larger than SMALL_NV, so that both score with the rescore kernel."""
+    scores exactly r[q].  (test_gpu_small_path.py checks the same at most SMALL_NV rows.)"""
     dims, w = (128, 64), (0.6, 0.4)
     V = X.synth.clustered(111, 50000, sum(dims))
     Q = X.synth.clustered(112, 256, sum(dims))
