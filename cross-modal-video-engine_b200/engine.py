@@ -20,6 +20,7 @@ import ctypes as C
 import math
 import os
 import struct
+from typing import NamedTuple
 
 import torch
 
@@ -66,6 +67,58 @@ N_LABELS = 64
 
 def _round_up(x, m):
     return (x + m - 1) // m * m
+
+
+class QueryBatch(NamedTuple):
+    """K1 on a query batch (:meth:`CorpusStore.prepare_queries`): the bf16 operand ``a_op [nq_pad, K]`` (rows padded to
+    ``_BM`` with zeros), ``q_raw`` fp32 ``[nq, raw_ld]``, ``q_norm`` fp64 ``[S, nq]``, ``q_res`` fp32 ``[S, nq]``
+    (squared bf16 residuals) and ``nq``.  A shard's ``prepare_queries`` may return these as a plain 5-tuple: the
+    search paths take it through ``QueryBatch._make``."""
+    a_op: torch.Tensor
+    q_raw: torch.Tensor
+    q_norm: torch.Tensor
+    q_res: torch.Tensor
+    nq: int
+
+    def take(self, rows):
+        """The queries ``rows`` (int64 tensor) as a batch of their own; ``None``: this batch."""
+        if rows is None:
+            return self
+        n = rows.numel()
+        a_op = torch.zeros((_round_up(n, _BM), self.a_op.shape[1]), dtype=self.a_op.dtype, device=self.a_op.device)
+        a_op[:n] = self.a_op[rows]
+        return QueryBatch(a_op, self.q_raw[rows].contiguous(), _take(self.q_norm, rows, 1), _take(self.q_res, rows, 1),
+                          n)
+
+
+def _take(t, rows, dim=0):
+    """The entries ``rows`` of a per-query tensor along ``dim``, contiguous (``t`` or ``rows`` None: ``t``)."""
+    if t is None or rows is None:
+        return t
+    return t.index_select(dim, rows).contiguous()
+
+
+def _mask_kw(label_mask):
+    """``label_mask=`` for a shard method, passed only when set: an unfiltered call needs nothing of a shard beyond
+    the unlabelled interface."""
+    return {} if label_mask is None else {"label_mask": label_mask}
+
+
+def _excludes(exclude, nq, device):
+    """``exclude`` (one global row or -1 per query, or None) -> int64 device tensor ``[nq]``; ValueError on a wrong
+    length (the kernels read ``excl[q]`` for every query)."""
+    if exclude is None:
+        return None
+    excl = torch.as_tensor(exclude, dtype=torch.int64).reshape(-1).to(device).contiguous()
+    if excl.numel() != nq:
+        raise ValueError("exclude: expected one row (or -1) per query (%d), got %d" % (nq, excl.numel()))
+    return excl
+
+
+def _device_ctx(dev):
+    """Launch on ``dev`` whatever device is current (no-op off CUDA)."""
+    import contextlib
+    return torch.cuda.device(dev) if dev.type == "cuda" else contextlib.nullcontext()
 
 
 def _as_spaces(x, dims):
@@ -295,8 +348,7 @@ class CorpusStore:
 
     # -- query side ------------------------------------------------------------------------------
     def prepare_queries(self, queries, weights=None):
-        """K1 on the query batch: returns (a_op bf16 [nq_pad, K], q_raw fp32 [nq, raw_ld], q_norm fp64 [S, nq],
-        q_resid fp32 [S, nq] squared bf16 residuals, nq)."""
+        """K1 on the query batch -> :class:`QueryBatch` ``(a_op, q_raw, q_norm, q_res, nq)``."""
         weights = _weights(weights, len(self.dims))
         spaces = [_to_device(s, self.device) for s in _as_spaces(queries, self.dims)]
         nq = spaces[0].shape[0]
@@ -309,7 +361,7 @@ class CorpusStore:
             _prepare(src, d, q_raw, raw_off, q_norm[s], q_res[s], a_op, op_off, N.OP_X1, weights[s], self.norm_mode)
             op_off += dp
             raw_off += d
-        return a_op, q_raw, q_norm, q_res, nq
+        return QueryBatch(a_op, q_raw, q_norm, q_res, nq)
 
     # -- search ----------------------------------------------------------------------------------
     def search(self, queries, k, weights=None, exclude=None, eps=None, small_nv=SMALL_NV, stats=None, defer=False,
@@ -394,13 +446,7 @@ class CorpusStore:
         16 384 rows, with a ``small_nv`` above the default, could still be cut by more float ties than that)."""
         dev, st = self.device, N.stream_ptr()
         kk = min(k, self.n)
-        vn, o = [], 0
-        for d in self.dims:
-            v = torch.empty((self.n, d), dtype=torch.float64, device=dev)
-            N.call("xmve_normalize_f64", N.ptr(self.raw[:, o:o + d]), N.F32, self.n, d, self.raw.stride(0), N.ptr(v), d,
-                   self.norm_mode, st)
-            vn.append(v)
-            o += d
+        vn = [_normalize_f64(self.raw[:self.n, o:o + d], self.norm_mode) for o, d in zip(self.space_off, self.dims)]
         out_s = torch.full((nq, k), float("-inf"), dtype=torch.float64, device=dev)
         out_i = torch.full((nq, k), -1, dtype=torch.int64, device=dev)
         s_ = torch.empty((nq, kk), dtype=torch.float64, device=dev)
@@ -410,19 +456,9 @@ class CorpusStore:
         cut_free = self.n <= max(2048, _pow2(4 * kk))                       # no row can hold more than the sort
         for q0 in range(0, nq, batch):
             q1 = min(nq, q0 + batch)
-            acc, o = None, 0
-            for s, d in enumerate(self.dims):
-                qn = torch.empty((q1 - q0, d), dtype=torch.float64, device=dev)
-                N.call("xmve_normalize_f64", N.ptr(q_raw[q0:q1, o:o + d]), N.F32, q1 - q0, d, q_raw.stride(0), N.ptr(qn),
-                       d, self.norm_mode, st)
-                sc = torch.empty((q1 - q0, self.n), dtype=torch.float64, device=dev)
-                N.call("xmve_score_f64", N.ptr(qn), q1 - q0, d, N.ptr(vn[s]), self.n, d, d, float(wts[s]), N.ptr(sc),
-                       self.n, st)
-                acc = sc if acc is None else acc.add_(sc)
-                o += d
-            if label_mask is not None:
-                N.call("xmve_mask_scores", N.ptr(acc), N.F64, q1 - q0, self.n, acc.stride(0),
-                       N.ptr(self._ensure_labels()), 1, N.ptr(label_mask[q0:q1]), st)
+            acc = _fused_f64(((_normalize_f64(q_raw[q0:q1, o:o + d], self.norm_mode), v)
+                              for o, d, v in zip(self.space_off, self.dims, vn)), wts,
+                             None if label_mask is None else (self._ensure_labels(), label_mask[q0:q1]))
             ex = N.ptr(excl[q0:q1]) if excl is not None else None
             N.call("xmve_select_topk_i32", N.ptr(acc), None, q1 - q0, self.n, None, self.index_offset, ex, kk, None,
                    0.0, None, None, N.ptr(s_[q0:]), N.ptr(i_[q0:]), None, None if cut_free else N.ptr(exact[q0:q1]),
@@ -440,7 +476,7 @@ class CorpusStore:
                 redo = (exact[q0:q1] == 0).unsqueeze(1)
                 s_[q0:q1] = torch.where(redo, s2, s_[q0:q1])
                 i_[q0:q1] = torch.where(redo, i2, i_[q0:q1])
-            del acc, sc
+            del acc
         out_s[:, :kk] = s_
         out_i[:, :kk] = i_
         return out_s, out_i
@@ -458,58 +494,23 @@ class CorpusStore:
                    step, N.ptr(label_mask), N.stream_ptr())
         return sample
 
-    def _filter(self, a_op, nq, thr, cap, step=1, label_mask=None):
+    def _filter(self, a_op, nq, lo, cap, step=1, hi=None, label_mask=None):
         """K2 FILTER over the shard (or over every ``step``-th row): candidates (approximate score, local row --
-        sampled-row number when ``step > 1``) above ``thr`` per query; ``label_mask``: eligible rows only."""
+        sampled-row number when ``step > 1``) above ``lo`` per query -> (count int32 [nq], scores fp32 [nq, cap],
+        local rows int32 [nq, cap]).  ``hi``: a two-sided window -- rows scoring above ``hi`` are counted, rows in
+        ``(lo, hi]`` are listed -> (above int32 [nq], count, scores, rows).  ``label_mask``: eligible rows only."""
         dev = self.device
         rows = (self.n + step - 1) // step
-        cand_count = torch.zeros((nq,), dtype=torch.int32, device=dev)
-        cand_score = torch.empty((nq, cap), dtype=torch.float32, device=dev)
-        cand_idx = torch.empty((nq, cap), dtype=torch.int32, device=dev)
-        if label_mask is not None:
-            N.call("xmve_score_filter_labeled", N.ptr(a_op), nq, a_op.stride(0), N.ptr(self.op), rows,
-                   self.op.stride(0), step, self.k, N.ptr(thr), None, None, N.ptr(cand_count), N.ptr(cand_score),
-                   N.ptr(cand_idx), cap, N.ptr(self._ensure_labels()), N.ptr(label_mask), N.stream_ptr())
-            return cand_count, cand_score, cand_idx
-        N.call("xmve_score_filter", N.ptr(a_op), nq, a_op.stride(0), N.ptr(self.op), rows, self.op.stride(0), step,
-               self.k, N.ptr(thr), None, None, N.ptr(cand_count), N.ptr(cand_score), N.ptr(cand_idx), cap,
-               N.stream_ptr())
-        return cand_count, cand_score, cand_idx
-
-    def _filter_band(self, a_op, nq, lo, hi, cap, label_mask=None):
-        """K2 FILTER with a two-sided window per row: rows scoring above ``hi`` are counted, rows in ``(lo, hi]``
-        are listed -> (above int32 [nq], count int32 [nq], scores fp32 [nq, cap], local rows int32 [nq, cap]).
-        ``label_mask``: eligible rows only, counted and listed."""
-        dev = self.device
-        above = torch.zeros((nq,), dtype=torch.int32, device=dev)
+        above = None if hi is None else torch.zeros((nq,), dtype=torch.int32, device=dev)
         count = torch.zeros((nq,), dtype=torch.int32, device=dev)
         c_s = torch.empty((nq, cap), dtype=torch.float32, device=dev)
         c_i = torch.empty((nq, cap), dtype=torch.int32, device=dev)
+        name, labels = "xmve_score_filter", ()
         if label_mask is not None:
-            N.call("xmve_score_filter_labeled", N.ptr(a_op), nq, a_op.stride(0), N.ptr(self.op), self.n,
-                   self.op.stride(0), 1, self.k, N.ptr(lo), N.ptr(hi), N.ptr(above), N.ptr(count), N.ptr(c_s),
-                   N.ptr(c_i), cap, N.ptr(self._ensure_labels()), N.ptr(label_mask), N.stream_ptr())
-            return above, count, c_s, c_i
-        N.call("xmve_score_filter", N.ptr(a_op), nq, a_op.stride(0), N.ptr(self.op), self.n, self.op.stride(0), 1,
-               self.k, N.ptr(lo), N.ptr(hi), N.ptr(above), N.ptr(count), N.ptr(c_s), N.ptr(c_i), cap, N.stream_ptr())
-        return above, count, c_s, c_i
-
-    def _sample_top(self, a_op, nq, step, big_j, label_mask=None):
-        """The largest scores of the ``step``-strided sample of this shard WITHOUT writing the sample matrix:
-        a coarse STORE pass (every ``r * step``-th row, a few thousand columns) gives a per-query floor ``thr0``
-        that about ``4 * big_j`` of the fine sample's scores exceed; a FILTER pass over the fine sample keeps those.
-        Returns ``(scores fp32 [nq, cap_s], counts int32 [nq], thr0 fp32 [nq])``; rows whose count is below
-        ``big_j`` (the floor came out too high -- vanishingly rare) are handled by the caller through ``thr0``.
-        ``label_mask``: both passes see the eligible rows only."""
-        n_s = (self.n + step - 1) // step
-        r = max(2, min(16, n_s // 2048))
-        kw = {} if label_mask is None else {"label_mask": label_mask}
-        coarse = self._sample(a_op, nq, step * r, **kw)
-        j0 = min(coarse.shape[1], int(math.ceil(4.0 * big_j / r)))
-        thr0 = _row_kth(coarse, None, j0, 0.0, 0)
-        cap_s = 1 << max(10, int(math.ceil(math.log2(16 * big_j))))
-        count, score, _ = self._filter(a_op, nq, thr0, cap_s, step=step, **kw)
-        return score, count, thr0
+            name, labels = "xmve_score_filter_labeled", (N.ptr(self._ensure_labels()), N.ptr(label_mask))
+        N.call(name, N.ptr(a_op), nq, a_op.stride(0), N.ptr(self.op), rows, self.op.stride(0), step, self.k, N.ptr(lo),
+               N.ptr(hi), N.ptr(above), N.ptr(count), N.ptr(c_s), N.ptr(c_i), cap, *labels, N.stream_ptr())
+        return (count, c_s, c_i) if hi is None else (above, count, c_s, c_i)
 
     def _rescore(self, q_raw, q_norm, nq, wts, cand, bound, bound_hi=None, exact=None):
         """Exact fp64 scores of the candidates whose approximate score reaches ``bound`` (second round: of those in
@@ -695,6 +696,33 @@ def _row_kth(vals, counts, j1, sub, j2, sub_dev=None):
     return out
 
 
+def _normalize_f64(x, norm_mode):
+    """fp32 rows ``x [n, d]`` (unit column stride) -> fp64 ``[n, d]``, each row divided by its norm."""
+    n, d = x.shape
+    out = torch.empty((n, d), dtype=torch.float64, device=x.device)
+    N.call("xmve_normalize_f64", N.ptr(x), N.F32, n, d, x.stride(0), N.ptr(out), d, norm_mode, N.stream_ptr())
+    return out
+
+
+def _fused_f64(spaces, wts, mask=None):
+    """The fused fp64 DMMA score matrix ``sum_s w_s * q_s @ v_s^T`` -> fp64 ``[m, n]``, added in space order.
+    ``spaces`` yields, space by space, operands already normalised row by row: ``(q_s fp64 [m, d_s], v_s fp64 [n,
+    d_s])``.  It is consumed one space at a time, so a generator that normalises one side as it goes launches each
+    normalisation right before its product.  ``mask = (labels uint8 [n], masks int64 [m])``: entries whose label the
+    query's mask does not allow are set to -inf."""
+    st = N.stream_ptr()
+    acc = None
+    for w, (q, v) in zip(wts, spaces):
+        (m, d), n = q.shape, v.shape[0]
+        sc = torch.empty((m, n), dtype=torch.float64, device=q.device)
+        N.call("xmve_score_f64", N.ptr(q), m, d, N.ptr(v), n, d, d, float(w), N.ptr(sc), n, st)
+        acc = sc if acc is None else acc.add_(sc)
+    if mask is not None:
+        N.call("xmve_mask_scores", N.ptr(acc), N.F64, acc.shape[0], acc.shape[1], acc.stride(0), N.ptr(mask[0]), 1,
+               N.ptr(mask[1]), st)
+    return acc
+
+
 def _eps_device(q_res, dv2, wts, n_space, k_len):
     """:func:`measured_eps` on the device: fp32 ``[1]`` tensor (no host round trip)."""
     out = torch.empty((1,), dtype=torch.float32, device=q_res.device)
@@ -795,10 +823,7 @@ class PendingSearch:
 
     def result(self):
         if not self._done:
-            if self._ctx.dev.type == "cuda":
-                with torch.cuda.device(self._ctx.dev):
-                    self.reran = self._ctx.resolve()
-            else:
+            with _device_ctx(self._ctx.dev):
                 self.reran = self._ctx.resolve()
             self._done = True
             self._ctx = None
@@ -806,69 +831,103 @@ class PendingSearch:
 
 
 class _Search:
-    """State of one filtered search (every rank holds the same queries, thresholds and outputs)."""
+    """State of one top-k search (every rank holds the same queries, thresholds and outputs) and its passes: a
+    candidate step, the selection with its certificate, and the re-run of the rows that missed it.  The candidate
+    step and the re-run policy here are the filtered pipeline's (steps 3-4 and 6 of :func:`search_shards`);
+    :class:`_SmallSearch` brings its own."""
 
-    def __init__(self, stores, comm, k, k_eff, kk, wts, excl, eps_t, pl, a_op, q_raw, q_norm, nq, thr, out_s, out_i,
-                 stats, ph, masks=None, n_elig=None):
+    #: rows reach the selection with thr = -inf without label masks (see run_pass)
+    open_thr = False
+
+    def __init__(self, stores, comm, k, k_eff, kk, wts, excl, eps_t, qb, thr, cap, out_s, out_i, stats, ph, masks=None,
+                 n_elig=None):
         self.stores, self.comm, self.k, self.k_eff, self.kk, self.wts = stores, comm, k, k_eff, kk, wts
-        self.excl, self.eps_t, self.pl = excl, eps_t, pl
-        self.a_op, self.q_raw, self.q_norm, self.nq, self.thr = a_op, q_raw, q_norm, nq, thr
+        self.excl, self.eps_t, self.qb, self.thr, self.cap = excl, eps_t, qb, thr, cap
         self.out_s, self.out_i, self.stats, self.ph = out_s, out_i, stats, ph
-        self.ref = stores[0]
-        self.dev = self.ref.device
+        self.dev = stores[0].device
         self.live = [s for s in stores if s.n]
         self.n_shards = len(stores) * comm.world
         self.solo = self.n_shards == 1
-        cap = pl["cap"]
-        if not self.solo:
-            cap = max(2048, min(cap, 1 << int(math.ceil(math.log2(4.0 * cap / self.n_shards)))))
-        self.cap = cap
         self.n_shard_max = max(s.n for s in self.live) if self.live else 1
-        self.pending = None
+        self.pilot_m = None                                   # set by the filtered path's candidate step
         # filtered search: a row with at most `cap` eligible rows in the whole corpus gets thr = -inf -- every shard's
         # list then holds all its eligible rows, and the list is complete even when it is shorter than k
         self.masks, self.n_elig = masks, n_elig
         # (a row with no eligible row at all gets thr = +inf: nothing enters its window, and its answer is empty)
-        if masks is not None:
+        if n_elig is not None:
             self.thr = torch.where(n_elig == 0, torch.full_like(thr, float("inf")),
                                    torch.where(n_elig <= cap, torch.full_like(thr, float("-inf")), thr))
 
     # one pass over all rows (rows None) or over the rows that are re-run --------------------------------
     def run_pass(self, rows):
-        ref, dev, comm, ph, k_eff, kk, eps_t = self.ref, self.dev, self.comm, self.ph, self.k_eff, self.kk, self.eps_t
-        if rows is None:
-            a_sub, q_sub, qn_sub, thr_sub, ex_sub, n_sub = self.a_op, self.q_raw, self.q_norm, self.thr, self.excl, self.nq
+        q, ex, mk = self.qb.take(rows), _take(self.excl, rows), _take(self.masks, rows)
+        thr = _take(self.thr, rows)
+        self.ph.mark("alloc")
+        cands, exacts, thr, bound = self._candidates(q, thr, ex, mk)
+        # 5: selection.  One shard: the local kernel certifies.  Several: packed local lists, ONE gather, K3.
+        # With 512 rows or more the selection kernels sort at most max(2048, 4k) entries per row; a re-run selects in
+        # smaller batches, so that the rows whose lists did not fit (heavy float ties) get the full 16 384 entries.
+        n_bad = torch.zeros((1,), dtype=torch.int32, device=self.dev)
+        batch = q.nq if rows is None else SELECT_RERUN_ROWS
+        parts = [self._select_rows(r0, min(q.nq, r0 + batch), cands, exacts, ex, thr, bound, n_bad)
+                 for r0 in range(0, q.nq, batch)]
+        if len(parts) == 1:
+            s_, i_, cert, thr_next, over = parts[0]
         else:
-            n_sub = rows.numel()
-            a_sub = torch.zeros((_round_up(n_sub, _BM), ref.k), dtype=torch.bfloat16, device=dev)
-            a_sub[:n_sub] = self.a_op[rows]
-            q_sub = self.q_raw[rows].contiguous()
-            qn_sub = self.q_norm[:, rows].contiguous()
-            thr_sub = self.thr[rows].contiguous()
-            ex_sub = self.excl[rows].contiguous() if self.excl is not None else None
-        cap = self.cap
-        kw = {}
-        if self.masks is not None:
-            kw["label_mask"] = self.masks if rows is None else self.masks[rows].contiguous()
+            s_, i_, cert, thr_next = (torch.cat([p[j] for p in parts]) for j in range(4))
+            over = ("parts", [p[4] for p in parts])
+        if self.masks is not None or self.open_thr:
+            # a row with thr = -inf whose lists did not overflow holds every valid row of every shard.  When it holds
+            # fewer than k (its last entry is padding: fewer than k eligible rows, or k >= n with an exclusion) the
+            # selection cannot certify it, yet it is exact; a row with k entries or more keeps the selection's verdict
+            # (which also covers float ties cut by the sort).  A row without any eligible row is empty.
+            short = (thr == float("-inf")) & ~self._overflowed(over) & (i_[:, -1] == -1)
+            if self.n_elig is not None:
+                short |= _take(self.n_elig, rows) == 0
+            cert = torch.where(short, torch.ones_like(cert), cert)
+            n_bad.copy_((cert == 0).sum().reshape(1))
+        self.ph.mark("select_merge")
+        if self.stats is not None and rows is None:
+            st = self.stats
+            st["eps"] = float(self.eps_t)
+            st["cap"] = self.cap
+            if self.pilot_m is not None:                      # the filtered path's candidate lists
+                st["pilot_m"] = self.pilot_m
+                st["cand_count"] = [c[0] for c in cands]
+                ar = torch.arange(self.cap, device=self.dev)
+                st["rescored_per_query"] = sum(
+                    float(((ar[None, :] < c[0][:, None]) & (e[:, :self.cap] > float("-inf"))).sum())
+                    for c, e in zip(cands, exacts)) / max(q.nq, 1)
+                if self.masks is not None:
+                    st["eligible_min"], st["eligible_max"] = int(self.n_elig.min()), int(self.n_elig.max())
+                    st["thr_inf_rows"] = int((thr == float("-inf")).sum())
+                self.ph.mark("stats_bookkeeping")
+        return s_, i_, cert, thr_next, over, n_bad, thr
+
+    def _candidates(self, q, thr, ex, mk):
+        """Steps 3-4 of :func:`search_shards` for the queries ``q`` (thresholds ``thr``, exclusions ``ex``, label masks
+        ``mk``) -> (per-shard candidate lists, their exact scores, the threshold, the rescore bound)."""
+        dev, comm, ph, k_eff, kk, eps_t = self.dev, self.comm, self.ph, self.k_eff, self.kk, self.eps_t
         # 3: fused score + threshold filter on every local shard
-        ph.mark("alloc")
-        cands = [s._filter(a_sub, n_sub, thr_sub, cap, **kw) for s in self.live]
+        cands = [s._filter(q.a_op, q.nq, thr, self.cap, **_mask_kw(mk)) for s in self.live]
         ph.mark("filter")
         # 4: what needs an exact score
         m = kk if self.solo else min(kk, int(math.ceil(1.5 * kk / self.n_shards)) + 10)
+        self.pilot_m = m
         if kk <= PILOT_MAX and (self.solo or self.n_shards * m <= PILOT_UNION_MAX):
             # two rounds.  One: every shard rescores its m best approximate candidates; the k-th largest exact score
             # of the union of these pilots (kth1) is a lower bound on the true k-th best.  Two: only candidates whose
             # approximate score reaches kth1 - eps can still belong to the top-k.
             firsts = [_row_kth(c[1], c[0], m, 0.0, 0) for c in cands]
-            exacts = [s._rescore(q_sub, qn_sub, n_sub, self.wts, c, b1) for s, c, b1 in zip(self.live, cands, firsts)]
-            pilots = [s._pilot_top(e, c, n_sub, ex_sub, m) for s, c, e in zip(self.live, cands, exacts)]
+            exacts = [s._rescore(q.q_raw, q.q_norm, q.nq, self.wts, c, b1)
+                      for s, c, b1 in zip(self.live, cands, firsts)]
+            pilots = [s._pilot_top(e, c, q.nq, ex, m) for s, c, e in zip(self.live, cands, exacts)]
             if not pilots:
-                pilots = [torch.full((n_sub, m), float("-inf"), dtype=torch.float64, device=dev)]
+                pilots = [torch.full((q.nq, m), float("-inf"), dtype=torch.float64, device=dev)]
             bound = _pilot_bound(_segments(pilots, comm), k_eff, eps_t)
             ph.mark("pilot")
             for s, c, b1, e in zip(self.live, cands, firsts, exacts):
-                s._rescore(q_sub, qn_sub, n_sub, self.wts, c, bound, b1, e)
+                s._rescore(q.q_raw, q.q_norm, q.nq, self.wts, c, bound, b1, e)
         else:
             # very deep lists (k > 1000): one round against (kk-th largest approximate score over all shards) - 2 eps
             if self.solo:
@@ -876,55 +935,19 @@ class _Search:
             elif kk <= ROW_TOPJ_MAX:
                 tops = [_row_topj(c[1], c[0], kk) for c in cands]
                 if not tops:
-                    tops = [torch.full((n_sub, kk), float("-inf"), dtype=torch.float32, device=dev)]
+                    tops = [torch.full((q.nq, kk), float("-inf"), dtype=torch.float32, device=dev)]
                 bound = _row_kth(_union(tops, comm), None, kk, 2.0, 0, eps_t)
             else:
                 # deeper than xmve_row_topj extracts: the best shard's own kk-th largest approximate score is a lower
                 # bound on the kk-th largest of the union (looser, so a few more rows are rescored)
-                bound = torch.full((n_sub,), float("-inf"), dtype=torch.float32, device=dev)
+                bound = torch.full((q.nq,), float("-inf"), dtype=torch.float32, device=dev)
                 for c in cands:
                     bound = torch.maximum(bound, _row_kth(c[1], c[0], kk, 2.0, 0, eps_t))
                 bound = comm.max_(bound)
             ph.mark("bound")
-            exacts = [s._rescore(q_sub, qn_sub, n_sub, self.wts, c, bound) for s, c in zip(self.live, cands)]
+            exacts = [s._rescore(q.q_raw, q.q_norm, q.nq, self.wts, c, bound) for s, c in zip(self.live, cands)]
         ph.mark("rescore")
-        # 5: selection.  One shard: the local kernel certifies.  Several: packed local lists, ONE gather, K3.
-        # With 512 rows or more the selection kernels sort at most max(2048, 4k) entries per row; a re-run selects in
-        # smaller batches, so that the rows whose lists did not fit (heavy float ties) get the full 16 384 entries.
-        n_bad = torch.zeros((1,), dtype=torch.int32, device=dev)
-        batch = n_sub if rows is None else SELECT_RERUN_ROWS
-        parts = [self._select_rows(r0, min(n_sub, r0 + batch), cands, exacts, ex_sub, thr_sub, bound, n_bad)
-                 for r0 in range(0, n_sub, batch)]
-        if len(parts) == 1:
-            s_, i_, cert, thr_next, over = parts[0]
-        else:
-            s_, i_, cert, thr_next = (torch.cat([p[j] for p in parts]) for j in range(4))
-            over = ("parts", [p[4] for p in parts])
-        if self.masks is not None:
-            # a row with thr = -inf whose lists did not overflow holds every eligible row.  When it holds fewer than k
-            # (its last entry is padding) the selection cannot certify it, yet it is exact; a row with k entries or
-            # more keeps the selection's verdict (which also covers float ties cut by the sort).  A row without any
-            # eligible row is empty.
-            n_elig = self.n_elig if rows is None else self.n_elig[rows]
-            short = (thr_sub == float("-inf")) & ~self._overflowed(over) & (i_[:, -1] == -1)
-            cert = torch.where(short | (n_elig == 0), torch.ones_like(cert), cert)
-            n_bad.copy_((cert == 0).sum().reshape(1))
-        ph.mark("select_merge")
-        if self.stats is not None and rows is None:
-            st = self.stats
-            st["eps"] = float(eps_t)
-            st["cap"] = cap
-            st["pilot_m"] = m
-            st["cand_count"] = [c[0] for c in cands]
-            ar = torch.arange(cap, device=dev)
-            st["rescored_per_query"] = sum(
-                float(((ar[None, :] < c[0][:, None]) & (e[:, :cap] > float("-inf"))).sum())
-                for c, e in zip(cands, exacts)) / max(n_sub, 1)
-            if self.masks is not None:
-                st["eligible_min"], st["eligible_max"] = int(self.n_elig.min()), int(self.n_elig.max())
-                st["thr_inf_rows"] = int((thr_sub == float("-inf")).sum())
-            ph.mark("stats_bookkeeping")
-        return s_, i_, cert, thr_next, over, n_bad, thr_sub
+        return cands, exacts, thr, bound
 
     def _select_rows(self, r0, r1, cands, exacts, ex_sub, thr_sub, bound, n_bad):
         """Step 5 for rows ``r0:r1`` of a pass -> (scores, idx, cert, thr_next, overflow descriptor)."""
@@ -1004,41 +1027,42 @@ class _Search:
         return flags.max(dim=0).values != 0
 
     def _rerun(self):
-        cert, thr_next, over, thr_sub = self._last
+        cert, thr_next, over, thr = self._last
         rows = None
         for attempt in range(12):
             bad = torch.nonzero(cert == 0).flatten()            # device -> host sync (identical on every rank)
             if bad.numel() == 0:
                 return
-            over = self._overflowed(over)
-            # an overflowed row needs a HIGHER threshold; if the kernel cannot propose one, grow the lists
-            stuck = over[bad] & (thr_next[bad] <= thr_sub[bad])
-            if rows is None:
-                self.thr = self.thr.clone()
-                self.thr[bad] = thr_next[bad]
-                rows = bad
-            else:
-                self.thr[rows[bad]] = thr_next[bad]
-                rows = rows[bad]
+            rows = bad if rows is None else rows[bad]
             if self.stats is not None:
                 self.stats["reruns"] = self.stats.get("reruns", 0) + 1
                 self.stats["rerun_rows"] = self.stats.get("rerun_rows", 0) + int(rows.numel())
-            if bool(stuck.any()):
-                # overflow that a tighter threshold cannot fix (dense neighbourhoods within eps of the k-th best):
-                # grow the lists -- for the few rows left they may grow until they hold a whole shard
-                room = max(32768, min(1 << int(math.ceil(math.log2(self.n_shard_max))),
-                                      (1 << 27) // max(int(rows.numel()), 1)))
-                self.cap = min(room, self.cap * 4)
-            if self.masks is not None:                        # rows whose eligible rows now fit the lists
-                self.thr[rows] = torch.where(self.n_elig[rows] <= self.cap,
-                                             torch.full_like(self.thr[rows], float("-inf")), self.thr[rows])
-            s_, i_, cert, thr_next, over, _, thr_sub = self.run_pass(rows)
+            self._retune(rows, bad, thr_next, over, thr)
+            s_, i_, cert, thr_next, over, _, thr = self.run_pass(rows)
             self.out_s[rows, :self.k_eff] = s_
             self.out_i[rows, :self.k_eff] = i_
         bad = torch.nonzero(cert == 0).flatten()
         if bad.numel():
             raise N.XmveError("search: %d row(s) could not be certified after 12 passes (increase eps headroom "
                               "or candidate capacity; heavy score ties?)" % int(bad.numel()))
+
+    def _retune(self, rows, bad, thr_next, over, thr):
+        """Re-run policy: ``thr`` and ``cap`` for the query rows ``rows`` about to re-run, from the pass that missed
+        their certificate (``bad``: their positions in it; its ``thr_next``, overflow descriptor and thresholds)."""
+        # an overflowed row needs a HIGHER threshold; if the kernel cannot propose one, grow the lists
+        stuck = self._overflowed(over)[bad] & (thr_next[bad] <= thr[bad])
+        if self.thr is self._thr0:                            # (a captured graph keeps reading the first pass's)
+            self.thr = self.thr.clone()
+        self.thr[rows] = thr_next[bad]
+        if bool(stuck.any()):
+            # overflow that a tighter threshold cannot fix (dense neighbourhoods within eps of the k-th best):
+            # grow the lists -- for the few rows left they may grow until they hold a whole shard
+            room = max(32768, min(1 << int(math.ceil(math.log2(self.n_shard_max))),
+                                  (1 << 27) // max(int(rows.numel()), 1)))
+            self.cap = min(room, self.cap * 4)
+        if self.masks is not None:                            # rows whose eligible rows now fit the lists
+            self.thr[rows] = torch.where(self.n_elig[rows] <= self.cap,
+                                         torch.full_like(self.thr[rows], float("-inf")), self.thr[rows])
 
 
 class _SmallSearch(_Search):
@@ -1050,86 +1074,34 @@ class _SmallSearch(_Search):
     ``thr + eps <= kth``.  Step 6 re-runs the rows without a certificate with four times the lists, selecting in
     batches of ``SELECT_RERUN_ROWS`` rows; lists that hold a whole store are complete."""
 
-    def __init__(self, stores, comm, k, k_eff, wts, excl, eps_t, q_raw, q_norm, nq, out_s, out_i, stats, ph, masks):
-        self.stores, self.comm, self.k, self.k_eff, self.wts = stores, comm, k, k_eff, wts
-        self.excl, self.eps_t, self.masks = excl, eps_t, masks
-        self.q_raw, self.q_norm, self.nq, self.thr = q_raw, q_norm, nq, None
-        self.out_s, self.out_i, self.stats, self.ph = out_s, out_i, stats, ph
-        self.ref = stores[0]
-        self.dev = self.ref.device
-        self.live = [s for s in stores if s.n]
-        self.n_shards = len(stores) * comm.world
-        self.solo = self.n_shards == 1
-        self.n_shard_max = max(s.n for s in self.live) if self.live else 1
-        self.cap = 2 * k_eff + 32                             # candidates per row and store: the k best and slack
-        self.pending = None
+    open_thr = True                                           # a store whose list holds all its valid rows
 
-    def run_pass(self, rows):
+    def _candidates(self, q, thr, ex, mk):
         dev, k_eff = self.dev, self.k_eff
-        if rows is None:
-            q_sub, qn_sub, ex_sub, mk, n_sub = self.q_raw, self.q_norm, self.excl, self.masks, self.nq
-        else:
-            n_sub = rows.numel()
-            q_sub = self.q_raw[rows].contiguous()
-            qn_sub = self.q_norm[:, rows].contiguous()
-            ex_sub = self.excl[rows].contiguous() if self.excl is not None else None
-            mk = self.masks[rows].contiguous() if self.masks is not None else None
         width = max(min(self.cap, self.n_shard_max), k_eff)
-        kw = {} if mk is None else {"label_mask": mk}
-        ninf = torch.full((n_sub,), float("-inf"), dtype=torch.float32, device=dev)
-        self.ph.mark("alloc")
+        ninf = torch.full((q.nq,), float("-inf"), dtype=torch.float32, device=dev)
         cands, thr = [], ninf
         for s in self.live:
             m = min(self.cap, s.n)
-            top_s, top_i = s._exact_small(q_sub, qn_sub, n_sub, m, self.wts, ex_sub, **kw)
+            top_s, top_i = s._exact_small(q.q_raw, q.q_norm, q.nq, m, self.wts, ex, **_mask_kw(mk))
             # every row left out scores at most the m-th DMMA score: thr lies strictly above it (-inf when the list
             # holds every valid row of the store)
             t = torch.where(top_i[:, -1] >= 0, _float_above(top_s[:, -1]), ninf) if m < s.n else ninf
             thr = torch.maximum(thr, t)
-            c_s = torch.full((n_sub, width), float("-inf"), dtype=torch.float32, device=dev)
-            c_i = torch.zeros((n_sub, width), dtype=torch.int32, device=dev)
+            c_s = torch.full((q.nq, width), float("-inf"), dtype=torch.float32, device=dev)
+            c_i = torch.zeros((q.nq, width), dtype=torch.int32, device=dev)
             c_s[:, :m] = top_s.float()
             c_i[:, :m] = torch.where(top_i < 0, torch.zeros_like(top_i), top_i - s.index_offset).to(torch.int32)
             cands.append(((top_i >= 0).sum(1).to(torch.int32), c_s, c_i))
         if self.comm.world > 1:
             thr = self.comm.max_(thr)
         self.ph.mark("score_f64")
-        exacts = [s._rescore(q_sub, qn_sub, n_sub, self.wts, c, None) for s, c in zip(self.live, cands)]
+        exacts = [s._rescore(q.q_raw, q.q_norm, q.nq, self.wts, c, None) for s, c in zip(self.live, cands)]
         self.ph.mark("rescore")
-        n_bad = torch.zeros((1,), dtype=torch.int32, device=dev)
-        batch = n_sub if rows is None else SELECT_RERUN_ROWS
-        parts = [self._select_rows(r0, min(n_sub, r0 + batch), cands, exacts, ex_sub, thr, thr, n_bad)
-                 for r0 in range(0, n_sub, batch)]
-        s_, i_, cert, thr_next = (torch.cat([p[j] for p in parts]) for j in range(4))
-        # a row whose lists hold every valid row of every store is exact however short (fewer than k eligible rows,
-        # or k >= n with an exclusion); the selection cannot certify it, as its k-th entry is padding
-        short = (thr == float("-inf")) & (i_[:, -1] == -1)
-        cert = torch.where(short, torch.ones_like(cert), cert)
-        n_bad.copy_((cert == 0).sum().reshape(1))
-        self.ph.mark("select_merge")
-        if self.stats is not None and rows is None:
-            self.stats["eps"] = float(self.eps_t)
-            self.stats["cap"] = self.cap
-        return s_, i_, cert, thr_next, None, n_bad, thr
+        return cands, exacts, thr, thr
 
-    def _rerun(self):
-        cert = self._last[0]
-        rows = None
-        for attempt in range(12):
-            bad = torch.nonzero(cert == 0).flatten()            # device -> host sync (identical on every rank)
-            if bad.numel() == 0:
-                return
-            rows = bad if rows is None else rows[bad]
-            self.cap = min(4 * self.cap, self.n_shard_max, 16384)   # (the selection sorts at most 16 384 entries)
-            if self.stats is not None:
-                self.stats["reruns"] = self.stats.get("reruns", 0) + 1
-                self.stats["rerun_rows"] = self.stats.get("rerun_rows", 0) + int(rows.numel())
-            s_, i_, cert = self.run_pass(rows)[:3]
-            self.out_s[rows, :self.k_eff] = s_
-            self.out_i[rows, :self.k_eff] = i_
-        if bool((cert == 0).any()):
-            raise N.XmveError("search: %d row(s) could not be certified after 12 passes (heavy score ties?)"
-                              % int((cert == 0).sum()))
+    def _retune(self, rows, bad, thr_next, over, thr):
+        self.cap = min(4 * self.cap, self.n_shard_max, 16384)   # (the selection sorts at most 16 384 entries)
 
 
 class GraphSearch:
@@ -1295,20 +1267,10 @@ def search_shards(stores, queries, k, weights=None, exclude=None, eps=None, smal
     lists are complete and certified however short.  ``None`` runs the unfiltered pipeline unchanged.
     """
     comm = comm or SoloComm()
-    ref = stores[0]
-    if ref.device.type == "cuda":
-        with torch.cuda.device(ref.device):                     # kernels, streams and allocations follow the store
-            pending = _search_shards(stores, queries, k, weights, exclude, eps, small_nv, stats, comm, n_total,
-                                     head_stream=head_stream, label_mask=label_mask)
-            return pending if defer else pending.result()
-    pending = _search_shards(stores, queries, k, weights, exclude, eps, small_nv, stats, comm, n_total,
-                             label_mask=label_mask)
-    return pending if defer else pending.result()
-
-
-def _head_on(stream):
-    import contextlib
-    return torch.cuda.stream(stream) if stream is not None else contextlib.nullcontext()
+    with _device_ctx(stores[0].device):                        # kernels, streams and allocations follow the store
+        pending = _search_shards(stores, queries, k, weights, exclude, eps, small_nv, stats, comm, n_total,
+                                 head_stream=head_stream, label_mask=label_mask)
+        return pending if defer else pending.result()
 
 
 def _search_shards(stores, queries, k, weights, exclude, eps, small_nv, stats, comm, n_total, in_graph=False,
@@ -1338,11 +1300,10 @@ def _search_shards(stores, queries, k, weights, exclude, eps, small_nv, stats, c
         for s in stores:                                      # the head reads the stores' rows and residuals: only
             if getattr(s, "added", None) is not None:         # their last add, not the whole current stream, must
                 head_stream.wait_event(s.added)               # be complete
-    with _head_on(head_stream):
-        a_op, q_raw, q_norm, q_res, nq = ref.prepare_queries(queries, wts)
-        excl = None
-        if exclude is not None:
-            excl = torch.as_tensor(exclude, dtype=torch.int64).to(dev).contiguous()   # the kernels read excl[q]
+    with torch.cuda.stream(head_stream):                      # (no-op without a head stream)
+        qb = QueryBatch._make(ref.prepare_queries(queries, wts))
+        nq = qb.nq
+        excl = _excludes(exclude, nq, dev)
         masks = n_elig = None
         if label_mask is not None:
             masks = _label_masks(label_mask, nq, dev)
@@ -1357,23 +1318,27 @@ def _search_shards(stores, queries, k, weights, exclude, eps, small_nv, stats, c
 
     if n_total <= small_nv:
         eps_t = torch.full((1,), small_delta(wts, ref.dims), dtype=torch.float32, device=dev)
-        return _first_pass(_SmallSearch(stores, comm, k, k_eff, wts, excl, eps_t, q_raw, q_norm, nq, out_s, out_i,
-                                        stats, ph, masks), in_graph, flag_host)
+        # candidates per row and store: the k best and slack
+        return _first_pass(_SmallSearch(stores, comm, k, k_eff, k_eff, wts, excl, eps_t, qb, None, 2 * k_eff + 32,
+                                        out_s, out_i, stats, ph, masks), in_graph, flag_host)
 
     kk = k_eff + (1 if excl is not None else 0)              # one extra in case the excluded row is among them
     pl = plan(kk, n_total)
-    with _head_on(head_stream):
-        eps_t, thr = _threshold(stores, comm, solo, wts, eps, pl, a_op, q_res, nq, ph, masks)
+    with torch.cuda.stream(head_stream):
+        eps_t, thr = _threshold(stores, comm, solo, wts, eps, pl, qb, ph, masks)
     if head_stream is not None:
         # step 3 onwards runs on the caller's stream: it waits for the head, and the caching allocator must not hand
         # the head's tensors back to the head stream while this stream still reads them
         main = torch.cuda.current_stream()
         main.wait_stream(head_stream)
-        for t in (a_op, q_raw, q_norm, q_res, eps_t, thr, excl, masks, n_elig):
+        for t in (*qb[:4], eps_t, thr, excl, masks, n_elig):
             if t is not None:
                 t.record_stream(main)
-    return _first_pass(_Search(stores, comm, k, k_eff, kk, wts, excl, eps_t, pl, a_op, q_raw, q_norm, nq, thr, out_s,
-                               out_i, stats, ph, masks, n_elig), in_graph, flag_host)
+    cap = pl["cap"]
+    if not solo:                                              # each shard lists about its share of the candidates
+        cap = max(2048, min(cap, 1 << int(math.ceil(math.log2(4.0 * cap / n_shards)))))
+    return _first_pass(_Search(stores, comm, k, k_eff, kk, wts, excl, eps_t, qb, thr, cap, out_s, out_i, stats, ph,
+                               masks, n_elig), in_graph, flag_host)
 
 
 def _first_pass(search, in_graph, flag_host):
@@ -1385,27 +1350,43 @@ def _first_pass(search, in_graph, flag_host):
     return pending
 
 
-def _threshold(stores, comm, solo, wts, eps, pl, a_op, q_res, nq, ph, masks=None):
+def _sample_top(store, a_op, nq, step, big_j, label_mask=None):
+    """The largest scores of the ``step``-strided sample of one shard WITHOUT writing the sample matrix: a coarse STORE
+    pass (every ``r * step``-th row, a few thousand columns) gives a per-query floor ``thr0`` that about ``4 * big_j``
+    of the fine sample's scores exceed; a FILTER pass over the fine sample keeps those.  Returns ``(scores fp32 [nq,
+    cap_s], counts int32 [nq], thr0 fp32 [nq])``; rows whose count is below ``big_j`` (the floor came out too high --
+    vanishingly rare) are handled by the caller through ``thr0``.  ``label_mask``: both passes see the eligible rows
+    only."""
+    n_s = (store.n + step - 1) // step
+    r = max(2, min(16, n_s // 2048))
+    coarse = store._sample(a_op, nq, step * r, **_mask_kw(label_mask))
+    j0 = min(coarse.shape[1], int(math.ceil(4.0 * big_j / r)))
+    thr0 = _row_kth(coarse, None, j0, 0.0, 0)
+    cap_s = 1 << max(10, int(math.ceil(math.log2(16 * big_j))))
+    count, score, _ = store._filter(a_op, nq, thr0, cap_s, step=step, **_mask_kw(label_mask))
+    return score, count, thr0
+
+
+def _threshold(stores, comm, solo, wts, eps, pl, qb, ph, masks=None):
     """Steps 1b-2 of :func:`search_shards`: the error bound and the per-query threshold -> (eps_t, thr).  With
     ``masks`` the samples hold eligible rows only: the strided sample keeps its meaning among them (about k / step
     of a query's top-k eligible rows are sampled), so :func:`plan` applies unchanged."""
-    dev = stores[0].device
-    eps_t = _eps_for(stores, comm, wts, eps, q_res)
+    dev, a_op, nq = stores[0].device, qb.a_op, qb.nq
+    eps_t = _eps_for(stores, comm, wts, eps, qb.q_res)
     ph.mark("eps")
     live = [s for s in stores if s.n]
     # 2: one global threshold from the shards' samples
     j_cap = pl["j_cap"] if solo else min(pl["j_cap"], ROW_TOPJ_MAX)      # xmve_row_topj holds 4096 values per row
     big_j = max(pl["j"], j_cap)
-    kw = {} if masks is None else {"label_mask": masks}
     lists, floor = [], torch.full((nq,), float("-inf"), dtype=torch.float32, device=dev)
     for s in live:
         if (s.n + pl["step"] - 1) // pl["step"] >= 16384:
             # two-level: the sample matrix (2.1 GB at 10 M rows) is never written or radix-selected
-            sc, cnt, thr0 = s._sample_top(a_op, nq, pl["step"], big_j, **kw)
+            sc, cnt, thr0 = _sample_top(s, a_op, nq, pl["step"], big_j, masks)
             lists.append((sc, cnt))
             floor = thr0 if len(lists) == 1 else torch.minimum(floor, thr0)
         else:                                                 # small shard: the few launches of the plain way win
-            lists.append((s._sample(a_op, nq, pl["step"], **kw), None))
+            lists.append((s._sample(a_op, nq, pl["step"], **_mask_kw(masks)), None))
             floor = torch.full_like(floor, float("-inf"))     # a complete list needs no floor
     if solo:
         thr = _row_kth(lists[0][0], lists[0][1], pl["j"], pl["margin"], j_cap, eps_t)
@@ -1465,9 +1446,9 @@ def rank_of_gt(stores, queries, gt_off, gt_rows, weights=None, comm=None, n_tota
     wts = _weights(weights, n_space)
     if n_total is None:
         n_total = comm.sum_int(sum(s.n for s in stores))
-    import contextlib
-    with (torch.cuda.device(dev) if dev.type == "cuda" else contextlib.nullcontext()):
-        a_op, q_raw, q_norm, q_res, nq = ref.prepare_queries(queries, wts)
+    with _device_ctx(dev):
+        qb = QueryBatch._make(ref.prepare_queries(queries, wts))
+        nq = qb.nq
         off = torch.as_tensor(gt_off, dtype=torch.int64)
         g = torch.as_tensor(gt_rows, dtype=torch.int64).to(dev)
         n_ent = int(g.numel())
@@ -1475,36 +1456,32 @@ def rank_of_gt(stores, queries, gt_off, gt_rows, weights=None, comm=None, n_tota
         if n_ent == 0:
             return torch.zeros((0,), dtype=torch.int32, device=dev)
         owner = torch.repeat_interleave(torch.arange(nq), off[1:] - off[:-1]).to(dev)        # entry -> query row
-        eps_t = _eps_for(stores, comm, wts, eps, q_res)
-        # one operand / raw row per entry
-        a_ent = torch.zeros((_round_up(n_ent, _BM), ref.k), dtype=torch.bfloat16, device=dev)
-        a_ent[:n_ent] = a_op[owner]
-        q_ent = q_raw[owner].contiguous()
-        qn_ent = q_norm[:, owner].contiguous()
+        eps_t = _eps_for(stores, comm, wts, eps, qb.q_res)
+        ent = qb.take(owner)                                  # one query row per entry
         live = [s for s in stores if s.n]
         # 1: exact score of every ground-truth item, from the shard that owns it
-        s_gt = comm.max_(_row_scores(live, q_ent, qn_ent, n_ent, wts, g))
+        s_gt = comm.max_(_row_scores(live, ent, wts, g))
         if bool((s_gt == float("-inf")).any()):
             raise IndexError("rank_of_gt: a ground-truth row is outside the corpus (or its score is not finite)")
         # 2-3: rows before g
-        before, n_deep = _count_before_all(live, comm, a_ent, q_ent, qn_ent, n_ent, wts, s_gt, g, eps_t, cap)
+        before, n_deep = _count_before_all(live, comm, ent, wts, s_gt, g, eps_t, cap)
         if stats is not None:
             stats["eps"] = float(eps_t)
             stats["deep_entries"] = n_deep
         return (before + 1).to(torch.int32)
 
 
-def _row_scores(live, q_ent, qn_ent, n_ent, wts, g, masks=None):
-    """Exact fp64 score of global row ``g[e]`` for entry ``e``, from the local shard that owns it; -inf where no local
-    shard owns ``g[e]`` (or, with ``masks``, where its label is not allowed).  The caller all-reduces (max) over
-    ranks."""
-    dev = q_ent.device
+def _row_scores(live, ent, wts, g, masks=None):
+    """Exact fp64 score of global row ``g[e]`` for the query ``e`` of the batch ``ent``, from the local shard that owns
+    it; -inf where no local shard owns ``g[e]`` (or, with ``masks``, where its label is not allowed).  The caller
+    all-reduces (max) over ranks."""
+    dev, n_ent = ent.q_raw.device, ent.nq
     s_gt = torch.full((n_ent,), float("-inf"), dtype=torch.float64, device=dev)
     for s in live:
         mine = (g >= s.index_offset) & (g < s.index_offset + s.n)
         loc = torch.where(mine, g - s.index_offset, torch.zeros_like(g)).to(torch.int32).unsqueeze(1).contiguous()
         cnt = mine.to(torch.int32)
-        ex = s._rescore(q_ent, qn_ent, n_ent, wts, (cnt, torch.zeros((n_ent, 1), device=dev), loc), None)
+        ex = s._rescore(ent.q_raw, ent.q_norm, n_ent, wts, (cnt, torch.zeros((n_ent, 1), device=dev), loc), None)
         if masks is not None:
             lab = s._ensure_labels()[loc[:, 0].long()].long()
             mine = mine & (torch.bitwise_and(torch.bitwise_right_shift(masks, lab), 1) != 0)
@@ -1512,20 +1489,19 @@ def _row_scores(live, q_ent, qn_ent, n_ent, wts, g, masks=None):
     return s_gt
 
 
-def _count_before_all(live, comm, a_ent, q_ent, qn_ent, n_ent, wts, s_gt, g, eps_t, cap, masks=None):
+def _count_before_all(live, comm, ent, wts, s_gt, g, eps_t, cap, masks=None):
     """Steps 2-3 of :func:`rank_of_gt`: int64 ``[n_ent]`` = #{corpus rows v of every shard of every rank (eligible
-    under ``masks``) : s(v) > s_gt[e], or s(v) == s_gt[e] and v < g[e]} -> (counts, entries settled by the fp64
-    fallback).  With ``g = INT64_MAX`` that is #{v : s(v) >= s_gt[e]}."""
-    dev = q_ent.device
+    under ``masks``) : s(v) > s_gt[e], or s(v) == s_gt[e] and v < g[e]}, ``e`` a query of the batch ``ent`` -> (counts,
+    entries settled by the fp64 fallback).  With ``g = INT64_MAX`` that is #{v : s(v) >= s_gt[e]}."""
+    dev, n_ent = ent.q_raw.device, ent.nq
     # 2: window around s(g), widened by the float roundings of its ends
     e64 = eps_t.double()
     lo = (s_gt - 1.001 * e64 - 1e-7).float()
     hi = (s_gt + 1.001 * e64 + 1e-7).float()
-    kw = {} if masks is None else {"label_mask": masks}
     tally = torch.zeros((2, n_ent), dtype=torch.int64, device=dev)                            # [before, overflowed]
     for s in live:
-        above, count, c_s, c_i = s._filter_band(a_ent, n_ent, lo, hi, cap, **kw)
-        ex = s._rescore(q_ent, qn_ent, n_ent, wts, (count, c_s, c_i), None)
+        above, count, c_s, c_i = s._filter(ent.a_op, n_ent, lo, cap, hi=hi, **_mask_kw(masks))
+        ex = s._rescore(ent.q_raw, ent.q_norm, n_ent, wts, (count, c_s, c_i), None)
         tally[0] += above
         _count_before(ex, c_i, count, s.index_offset, s_gt, g, tally[0])
         tally[1] += (count > cap)
@@ -1534,56 +1510,38 @@ def _count_before_all(live, comm, a_ent, q_ent, qn_ent, n_ent, wts, s_gt, g, eps
     deep = torch.nonzero(tally[1] != 0).flatten()                                             # host sync
     # 3: exact fp64 pass for the entries whose window overflowed
     if deep.numel():
-        kw = {} if masks is None else {"masks": masks[deep].contiguous()}
-        fix = _rank_deep(live, q_ent[deep].contiguous(), qn_ent[:, deep].contiguous(), s_gt[deep].contiguous(),
-                         g[deep].contiguous(), wts, **kw)
-        tally[0, deep] = comm.sum_(fix)
+        tally[0, deep] = comm.sum_(_rank_deep(live, ent, deep, s_gt, g, wts, masks=masks))
     return tally[0], int(deep.numel())
 
 
-def _rank_deep(live, q_ent, qn_ent, s_gt, g, wts, chunk=1 << 17, band_cap=64, delta=1e-13, masks=None):
-    """#{rows before the ground truth} over this rank's shards from an exact fp64 score matrix, chunk by chunk.
-    Scores more than ``delta`` above ``s_gt`` are counted; the handful within ``delta`` (the fp64 matrix and the
-    rescore kernel sum in different orders, ~1e-15 apart) are settled by the rescore kernel itself.  ``masks``
-    (int64 ``[n_ent]``): ineligible rows are set to -inf first."""
-    dev = q_ent.device
-    n_ent = q_ent.shape[0]
-    before = torch.zeros((n_ent,), dtype=torch.int64, device=dev)
+def _rank_deep(live, ent, deep, s_gt, g, wts, chunk=1 << 17, band_cap=64, delta=1e-13, masks=None):
+    """#{rows before the ground truth} of the queries ``deep`` of the batch ``ent`` over this rank's shards, from an
+    exact fp64 score matrix, chunk by chunk.  Scores more than ``delta`` above ``s_gt`` are counted; the handful within
+    ``delta`` (the fp64 matrix and the rescore kernel sum in different orders, ~1e-15 apart) are settled by the rescore
+    kernel itself.  ``masks`` (int64 ``[ent.nq]``): ineligible rows are set to -inf first."""
+    dev = ent.q_raw.device
+    n_deep = deep.numel()
+    before = torch.zeros((n_deep,), dtype=torch.int64, device=dev)
     st = N.stream_ptr()
     for s in live:
-        for e0 in range(0, n_ent, 4096):
-            e1 = min(n_ent, e0 + 4096)
-            ne = e1 - e0
-            qs_n, o = [], 0
-            for d in s.dims:
-                qn = torch.empty((ne, d), dtype=torch.float64, device=dev)
-                src = q_ent[e0:e1, o:o + d]
-                N.call("xmve_normalize_f64", N.ptr(src), N.F32, ne, d, q_ent.stride(0), N.ptr(qn), d, s.norm_mode, st)
-                qs_n.append(qn)
-                o += d
+        for e0 in range(0, n_deep, 4096):
+            e1 = min(n_deep, e0 + 4096)
+            rows = deep[e0:e1]
+            q, sg, gg, mk = ent.take(rows), _take(s_gt, rows), _take(g, rows), _take(masks, rows)
+            ne = q.nq
+            qs_n = [_normalize_f64(q.q_raw[:, o:o + d], s.norm_mode) for o, d in zip(s.space_off, s.dims)]
             for r0 in range(0, s.n, chunk):
                 r1 = min(s.n, r0 + chunk)
-                acc, o = None, 0
-                for si, d in enumerate(s.dims):
-                    vn = torch.empty((r1 - r0, d), dtype=torch.float64, device=dev)
-                    vs = s.raw[r0:r1, o:o + d]
-                    N.call("xmve_normalize_f64", N.ptr(vs), N.F32, r1 - r0, d, s.raw.stride(0), N.ptr(vn), d,
-                           s.norm_mode, st)
-                    sc = torch.empty((ne, r1 - r0), dtype=torch.float64, device=dev)
-                    N.call("xmve_score_f64", N.ptr(qs_n[si]), ne, d, N.ptr(vn), r1 - r0, d, d, float(wts[si]),
-                           N.ptr(sc), r1 - r0, st)
-                    acc = sc if acc is None else acc.add_(sc)
-                    o += d
-                if masks is not None:
-                    N.call("xmve_mask_scores", N.ptr(acc), N.F64, ne, r1 - r0, acc.stride(0),
-                           N.ptr(s._ensure_labels()[r0:]), 1, N.ptr(masks[e0:e1]), st)
+                acc = _fused_f64(((qn, _normalize_f64(s.raw[r0:r1, o:o + d], s.norm_mode))
+                                  for qn, o, d in zip(qs_n, s.space_off, s.dims)), wts,
+                                 None if mk is None else (s._ensure_labels()[r0:], mk))
                 # band_count keeps counting past the capacity: a band that did not fit (many rows tied to 1e-13, e.g.
                 # exact duplicates) is listed again with room for all of it
                 cap_b, above = band_cap, torch.zeros((ne,), dtype=torch.int64, device=dev)
                 while True:
                     bcount = torch.zeros((ne,), dtype=torch.int32, device=dev)
                     bidx = torch.zeros((ne, cap_b), dtype=torch.int32, device=dev)
-                    N.call("xmve_count_band_f64", N.ptr(acc), ne, r1 - r0, r1 - r0, r0, N.ptr(s_gt[e0:]),
+                    N.call("xmve_count_band_f64", N.ptr(acc), ne, r1 - r0, r1 - r0, r0, N.ptr(sg),
                            float(delta), N.ptr(above), N.ptr(bcount), N.ptr(bidx), cap_b, st)
                     longest = int(bcount.max())
                     if longest <= cap_b:
@@ -1592,9 +1550,8 @@ def _rank_deep(live, q_ent, qn_ent, s_gt, g, wts, chunk=1 << 17, band_cap=64, de
                     above.zero_()
                 before[e0:e1] += above
                 bidx += r0                                                                    # shard-local rows
-                ex = s._rescore(q_ent[e0:e1], qn_ent[:, e0:e1].contiguous(), ne, wts,
-                                (bcount, torch.zeros((ne, cap_b), device=dev), bidx), None)
-                _count_before(ex, bidx, bcount, s.index_offset, s_gt[e0:e1], g[e0:e1], before[e0:e1])
+                ex = s._rescore(q.q_raw, q.q_norm, ne, wts, (bcount, torch.zeros((ne, cap_b), device=dev), bidx), None)
+                _count_before(ex, bidx, bcount, s.index_offset, sg, gg, before[e0:e1])
                 del acc, ex
     return before
 
@@ -1664,21 +1621,12 @@ def _range_setup(stores, queries, min_score, weights, exclude, label_mask, eps, 
     ref = stores[0]
     dev = ref.device
     wts = _weights(weights, len(ref.dims))
-    a_op, q_raw, q_norm, q_res, nq = ref.prepare_queries(queries, wts)
-    ms = _min_scores(min_score, nq, dev)
-    excl = None
-    if exclude is not None:
-        excl = torch.as_tensor(exclude, dtype=torch.int64).reshape(-1).to(dev).contiguous()
-        if excl.numel() != nq:
-            raise ValueError("exclude: expected one row (or -1) per query (%d), got %d" % (nq, excl.numel()))
-    masks = None if label_mask is None else _label_masks(label_mask, nq, dev)
-    eps_t = _eps_for(stores, comm, wts, eps, q_res)
-    return wts, a_op, q_raw, q_norm, nq, ms, excl, masks, eps_t
-
-
-def _device_ctx(dev):
-    import contextlib
-    return torch.cuda.device(dev) if dev.type == "cuda" else contextlib.nullcontext()
+    qb = QueryBatch._make(ref.prepare_queries(queries, wts))
+    ms = _min_scores(min_score, qb.nq, dev)
+    excl = _excludes(exclude, qb.nq, dev)
+    masks = None if label_mask is None else _label_masks(label_mask, qb.nq, dev)
+    eps_t = _eps_for(stores, comm, wts, eps, qb.q_res)
+    return wts, qb, ms, excl, masks, eps_t
 
 
 def _range_select(exact, cand, idx_offset, excl, ms, counts=None, off=None, max_len=0, out_s=None, out_i=None,
@@ -1751,8 +1699,8 @@ def _range_search(stores, queries, min_score, weights, exclude, label_mask, eps,
     dev = ref.device
     ph = _Phases(stats is not None and dev.type == "cuda")
     ph.mark("start")
-    wts, a_op, q_raw, q_norm, nq, ms, excl, masks, eps_t = _range_setup(stores, queries, min_score, weights, exclude,
-                                                                        label_mask, eps, comm)
+    wts, qb, ms, excl, masks, eps_t = _range_setup(stores, queries, min_score, weights, exclude, label_mask, eps, comm)
+    nq = qb.nq
     if nq == 0:
         return RangeResult(torch.zeros((1,), dtype=torch.int64, device=dev),
                            torch.empty((0,), dtype=torch.float64, device=dev),
@@ -1765,22 +1713,12 @@ def _range_search(stores, queries, min_score, weights, exclude, label_mask, eps,
     n_st = len(stores)
     solo = n_st * comm.world == 1
 
-    def sub(t, rows, dim=0):
-        if t is None or rows is None:
-            return t
-        return t.index_select(dim, rows).contiguous()
-
     def filter_pass(rows, cap):
         """FILTER over every local store for ``rows`` (None: all) -> (per-store lists, all-shard max count, host)."""
-        if rows is None:
-            a_sub, n_sub = a_op, nq
-        else:
-            n_sub = rows.numel()
-            a_sub = torch.zeros((_round_up(n_sub, _BM), ref.k), dtype=a_op.dtype, device=dev)
-            a_sub[:n_sub] = a_op[rows]
-        kw = {} if masks is None else {"label_mask": sub(masks, rows)}
-        cands = [s._filter(a_sub, n_sub, sub(lo, rows), cap, **kw) if s.n else None for s in stores]
-        cnt = torch.stack([c[0] if c is not None else torch.zeros((n_sub,), dtype=torch.int32, device=dev)
+        q = qb.take(rows)
+        cands = [s._filter(q.a_op, q.nq, _take(lo, rows), cap, **_mask_kw(_take(masks, rows))) if s.n else None
+                 for s in stores]
+        cnt = torch.stack([c[0] if c is not None else torch.zeros((q.nq,), dtype=torch.int32, device=dev)
                            for c in cands])
         allc = _segments(list(cnt.unbind(0)), comm).to("cpu", torch.int64)        # one collective; host sync
         return cands, allc
@@ -1856,15 +1794,15 @@ def _range_search(stores, queries, min_score, weights, exclude, label_mask, eps,
     for p, (rows, cs, cap) in enumerate(pieces):
         own = (owner == p) if rows is None else (owner[rows.cpu()] == p)
         own = own.to(dev)
-        q_sub, qn_sub, n_sub = sub(q_raw, rows), sub(q_norm, rows, 1), nq if rows is None else rows.numel()
-        ex_sub, ms_sub = sub(excl, rows), sub(ms, rows)
-        fl = {} if after is None else {"after": sub(after, rows)}
+        q = qb.take(rows)
+        ex_sub, ms_sub = _take(excl, rows), _take(ms, rows)
+        fl = {} if after is None else {"after": _take(after, rows)}
         ex_p = []
         for li, (s, c) in enumerate(zip(stores, cs)):
             if c is None:
                 ex_p.append(None)
                 continue
-            e = s._rescore(q_sub, qn_sub, n_sub, wts, c, None)
+            e = s._rescore(q.q_raw, q.q_norm, q.nq, wts, c, None)
             cp = torch.where(own, _range_select(e, c, s.index_offset, ex_sub, ms_sub, **fl),
                              torch.zeros((), dtype=torch.int64, device=dev))
             if rows is None:
@@ -1882,7 +1820,7 @@ def _range_search(stores, queries, min_score, weights, exclude, label_mask, eps,
                 continue
             e, cp = ex_p[li]
             max_len = min(cap, int(counts_h[li].max())) if rows is None else min(cap, int(counts_h[li][rows.cpu()].max()))
-            _range_select(e, cs[li], s.index_offset, ex_sub, ms_sub, counts=cp, off=sub(starts, rows), max_len=max_len,
+            _range_select(e, cs[li], s.index_offset, ex_sub, ms_sub, counts=cp, off=_take(starts, rows), max_len=max_len,
                           out_s=out_s, out_i=out_i, **fl)
 
     # 6: lay the lists out
@@ -1947,16 +1885,16 @@ def range_count_shards(stores, queries, min_score, weights=None, exclude=None, l
     comm = comm or SoloComm()
     stores = list(stores) if isinstance(stores, (list, tuple)) else [stores]
     with _device_ctx(stores[0].device):
-        wts, a_op, q_raw, q_norm, nq, ms, excl, masks, eps_t = _range_setup(stores, queries, min_score, weights,
-                                                                            exclude, label_mask, eps, comm)
+        wts, qb, ms, excl, masks, eps_t = _range_setup(stores, queries, min_score, weights, exclude, label_mask, eps,
+                                                       comm)
         dev = stores[0].device
-        if nq == 0:
+        if qb.nq == 0:
             return torch.zeros((0,), dtype=torch.int64, device=dev)
         live = [s for s in stores if s.n]
-        g = torch.full((nq,), torch.iinfo(torch.int64).max, dtype=torch.int64, device=dev)
-        count, n_deep = _count_before_all(live, comm, a_op, q_raw, q_norm, nq, wts, ms, g, eps_t, cap, masks)
+        g = torch.full((qb.nq,), torch.iinfo(torch.int64).max, dtype=torch.int64, device=dev)
+        count, n_deep = _count_before_all(live, comm, qb, wts, ms, g, eps_t, cap, masks)
         if excl is not None:
-            s_ex = comm.max_(_row_scores(live, q_raw, q_norm, nq, wts, excl, masks))
+            s_ex = comm.max_(_row_scores(live, qb, wts, excl, masks))
             count = count - ((s_ex > float("-inf")) & (s_ex >= ms)).to(torch.int64)
         if stats is not None:
             stats["eps"] = float(eps_t)

@@ -91,52 +91,48 @@ class ModelShard:
             o += d
         return acc
 
-    def _exact_small(self, q_raw, q_norm, nq, k, wts, excl):
+    def _eligible(self, label_mask, step=1):
+        """bool [nq, rows]: which of every ``step``-th row each query's label mask allows (None: every row).  The model
+        has no labels (the filtered protocol test adds them)."""
+        assert label_mask is None, "ModelShard has no row labels"
+        return None
+
+    def _exact_small(self, q_raw, q_norm, nq, k, wts, excl, label_mask=None):
         sc = self._exact(q_raw, q_norm, wts)
+        ok = self._eligible(label_mask)
+        if ok is not None:
+            sc[~ok] = float("-inf")
         ids = torch.arange(self.n)
-        rows = [_sorted_topk(sc[r], ids, k, None if excl is None else int(excl[r]), self.index_offset) for r in range(nq)]
+        rows = [_sorted_topk(sc[r], ids, k, None if excl is None else int(excl[r]), self.index_offset)
+                for r in range(nq)]
         return torch.stack([r[0] for r in rows]), torch.stack([r[1] for r in rows])
 
-    def _sample(self, a_op, nq, step):
-        return (a_op[:nq].float() @ self.op[::step].T).float()
+    def _sample(self, a_op, nq, step, label_mask=None):
+        sc = (a_op[:nq].float() @ self.op[::step].T).float()
+        ok = self._eligible(label_mask, step)
+        if ok is not None:
+            sc[~ok] = float("-inf")
+        return sc
 
-    def _filter(self, a_op, nq, thr, cap, step=1):
+    def _filter(self, a_op, nq, lo, cap, step=1, hi=None, label_mask=None):
         sc = (a_op[:nq].float() @ self.op[::step].T).float()       # re-run passes hand over a bf16 operand
+        hit = sc > lo[:, None]
+        ok = self._eligible(label_mask, step)
+        if ok is not None:
+            hit &= ok
+        if hi is not None:                                          # two-sided window: count above hi, list the rest
+            above = (hit & (sc > hi[:, None])).sum(1).int()
+            hit &= sc <= hi[:, None]
         count = torch.zeros(nq, dtype=torch.int32)
         c_s = torch.full((nq, cap), float("nan"), dtype=torch.float32)
         c_i = torch.zeros((nq, cap), dtype=torch.int32)
         for r in range(nq):
-            hit = torch.nonzero(sc[r] > thr[r]).flatten()
-            hit = hit[torch.randperm(len(hit), generator=torch.Generator().manual_seed(r))]   # arrival order is arbitrary
-            count[r] = len(hit)
-            m = min(len(hit), cap)
-            c_s[r, :m], c_i[r, :m] = sc[r, hit[:m]], hit[:m].int()
-        return count, c_s, c_i
-
-    def _filter_band(self, a_op, nq, lo, hi, cap):
-        sc = (a_op[:nq].float() @ self.op.T).float()
-        above = (sc > hi[:, None]).sum(1).int()
-        count = torch.zeros(nq, dtype=torch.int32)
-        c_s = torch.full((nq, cap), float("nan"), dtype=torch.float32)
-        c_i = torch.zeros((nq, cap), dtype=torch.int32)
-        for r in range(nq):
-            hit = torch.nonzero((sc[r] > lo[r]) & (sc[r] <= hi[r])).flatten()
-            hit = hit[torch.randperm(len(hit), generator=torch.Generator().manual_seed(r))]
-            count[r] = len(hit)
-            m = min(len(hit), cap)
-            c_s[r, :m], c_i[r, :m] = sc[r, hit[:m]], hit[:m].int()
-        return above, count, c_s, c_i
-
-    def _sample_top(self, a_op, nq, step, big_j):
-        from cross_modal_video_engine_b200 import engine
-        n_s = (self.n + step - 1) // step
-        r = max(2, min(16, n_s // 2048))
-        coarse = self._sample(a_op, nq, step * r)
-        j0 = min(coarse.shape[1], int(math.ceil(4.0 * big_j / r)))
-        thr0 = engine._row_kth(coarse, None, j0, 0.0, 0)
-        cap_s = 1 << max(10, int(math.ceil(math.log2(16 * big_j))))
-        count, score, _ = self._filter(a_op, nq, thr0, cap_s, step=step)
-        return score, count, thr0
+            h = torch.nonzero(hit[r]).flatten()
+            h = h[torch.randperm(len(h), generator=torch.Generator().manual_seed(r))]   # arrival order is arbitrary
+            count[r] = len(h)
+            m = min(len(h), cap)
+            c_s[r, :m], c_i[r, :m] = sc[r, h[:m]], h[:m].int()
+        return (count, c_s, c_i) if hi is None else (above, count, c_s, c_i)
 
     def _rescore(self, q_raw, q_norm, nq, wts, cand, bound, bound_hi=None, exact=None):
         count, c_s, c_i = cand

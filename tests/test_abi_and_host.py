@@ -186,3 +186,18 @@ def test_search_pipeline_two_level_sampling_on_cpu_model(monkeypatch):
     shards = [cpu_model.ModelShard(V[:cut], (d,), 0), cpu_model.ModelShard(V[cut:], (d,), cut)]
     s2, i2 = engine.search_shards(shards, Q, k)
     assert all(torch.equal(i2[r], ref[r][1]) for r in range(nq))
+
+
+@pytest.mark.parametrize("small_nv", [1000, 10 ** 9])
+def test_search_rejects_exclude_shorter_than_the_batch(monkeypatch, small_nv):
+    """``exclude`` holds one row per query: the selection, pilot and rescore kernels read ``excl[q]`` for every query,
+    so a shorter one raises ValueError (as range_search does) instead of reaching them -- filtered and small path."""
+    import sys
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    import cpu_model
+    from cross_modal_video_engine_b200 import engine
+    cpu_model.patch_engine(monkeypatch.setattr)
+    g = torch.Generator().manual_seed(3)
+    V, Q = torch.randn((20000, 16), generator=g), torch.randn((4, 16), generator=g)
+    with pytest.raises(ValueError, match="exclude: expected one row"):
+        engine.search_shards([cpu_model.ModelShard(V, (16,))], Q, 5, exclude=torch.tensor([3, -1]), small_nv=small_nv)

@@ -1,10 +1,9 @@
 """Filtered search (``label_mask``) through the multi-rank pipeline on CPU: two gloo ranks, each with a CPU model shard
-that applies row labels in the shard-local methods the engine calls (``_filter``, ``_sample``, ``_sample_top``,
-``_exact_small``, ``_label_counts``).  Covers the globally reduced label histogram and eligible counts, the sharded
+with row labels (its ``_label_counts``, and ``_eligible``, through which the model's ``_filter``, ``_sample`` and
+``_exact_small`` apply them).  Covers the globally reduced label histogram and eligible counts, the sharded
 threshold over masked samples, the routing of rows with few eligible rows to thr = -inf and the certificate of their
 short lists, the re-run loop, and the small-corpus branch -- each against the full-corpus fp64 model restricted to the
 eligible rows.  The labelled kernels themselves are tested on the B200 (test_gpu_filtered_search.py)."""
-import math
 import os
 import socket
 
@@ -45,47 +44,8 @@ def _labelled_shard_class():
             self.labels[loc[mine]] = torch.as_tensor(labels)[mine]
             self.label_version += 1
 
-        def _exact_small(self, q_raw, q_norm, nq, k, wts, excl, label_mask=None):
-            sc = self._exact(q_raw, q_norm, wts)
-            if label_mask is not None:
-                sc[~_allowed(label_mask[:nq], self.labels)] = float("-inf")
-            ids = torch.arange(self.n)
-            rows = [cpu_model._sorted_topk(sc[r], ids, k, None if excl is None else int(excl[r]), self.index_offset)
-                    for r in range(nq)]
-            return torch.stack([r[0] for r in rows]), torch.stack([r[1] for r in rows])
-
-        def _sample(self, a_op, nq, step, label_mask=None):
-            sc = super()._sample(a_op, nq, step)
-            if label_mask is not None:
-                sc[~_allowed(label_mask[:nq], self.labels[::step])] = float("-inf")
-            return sc
-
-        def _filter(self, a_op, nq, thr, cap, step=1, label_mask=None):
-            if label_mask is None:
-                return super()._filter(a_op, nq, thr, cap, step)
-            sc = (a_op[:nq].float() @ self.op[::step].T).float()
-            ok = _allowed(label_mask[:nq], self.labels[::step])
-            count = torch.zeros(nq, dtype=torch.int32)
-            c_s = torch.full((nq, cap), float("nan"), dtype=torch.float32)
-            c_i = torch.zeros((nq, cap), dtype=torch.int32)
-            for r in range(nq):
-                hit = torch.nonzero((sc[r] > thr[r]) & ok[r]).flatten()
-                hit = hit[torch.randperm(len(hit), generator=torch.Generator().manual_seed(r))]
-                count[r] = len(hit)
-                m = min(len(hit), cap)
-                c_s[r, :m], c_i[r, :m] = sc[r, hit[:m]], hit[:m].int()
-            return count, c_s, c_i
-
-        def _sample_top(self, a_op, nq, step, big_j, label_mask=None):
-            from cross_modal_video_engine_b200 import engine
-            n_s = (self.n + step - 1) // step
-            r = max(2, min(16, n_s // 2048))
-            coarse = self._sample(a_op, nq, step * r, label_mask=label_mask)
-            j0 = min(coarse.shape[1], int(math.ceil(4.0 * big_j / r)))
-            thr0 = engine._row_kth(coarse, None, j0, 0.0, 0)
-            cap_s = 1 << max(10, int(math.ceil(math.log2(16 * big_j))))
-            count, score, _ = self._filter(a_op, nq, thr0, cap_s, step=step, label_mask=label_mask)
-            return score, count, thr0
+        def _eligible(self, label_mask, step=1):
+            return None if label_mask is None else _allowed(label_mask, self.labels[::step])
 
     return LabelledShard
 
